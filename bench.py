@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """Headline benchmark: QPs solved per second at batch 2^16 per GPU (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's shard) as DIR/<name>.npy, float64:
+the inputs depend on the arguments only, so two builds can be compared output for output.
 
 One "step" = one cold batched Solve of 65 536 QPs per GPU: the 2019 logged Cassie walking QPs
 (tests/golden/walking_log_compact.npz) tiled to 2^16 (SURVEY.md 8d config 2), solver settings of
@@ -49,6 +52,18 @@ def algorithmic_flops_per_qp(n, m, iters_executed, cold=True):
     """SURVEY.md 8d: (1/3)N^3 per factorization (x2 cold) + 2N^2 per executed iteration."""
     N = n + m
     return (2 if cold else 1) * N ** 3 / 3.0 + 2.0 * N * N * iters_executed
+
+
+def dump_outputs(path, sol):
+    """The arrays FCCQPBatch.GetSolution() returned, one float64 .npy each (n_iter and solve_status are exact
+    in float64): about 35 MB at 2^16 QPs of the walking log."""
+    os.makedirs(path, exist_ok=True)
+    d = sol.details
+    arrays = {"z": sol.z, "n_iter": d.n_iter, "solve_status": d.solve_status, "eps_bounds": d.eps_bounds,
+              "eps_friction_cone": d.eps_friction_cone, "bounds_viol": d.bounds_viol,
+              "friction_cone_viol": d.friction_cone_viol}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy().astype(np.float64))
 
 
 def measured_peaks():
@@ -410,6 +425,7 @@ def run_ours(args):
         solver.Solve(*dev_args)          # asynchronous launch on the current torch stream
         ev[k + 1].record(stream)
     torch.cuda.synchronize(dev)
+    sol = solver.GetSolution()           # of the last timed step (the untimed launches below replace it)
     sharding.barrier()
     launches = nat.lib().fccqp_kernel_launch_count() - launches0
     step_ms = [ev[k].elapsed_time(ev[k + 1]) for k in range(args.steps)]
@@ -424,7 +440,8 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     sharding.barrier()
     value = world * B * args.steps / total_s
-    sol = solver.GetSolution()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sol)
     n_iter = sol.details.n_iter.cpu().numpy()
     status = sol.details.solve_status.cpu().numpy()
     iters_executed = float(np.where(n_iter == OPTS["max_iter"], OPTS["max_iter"], n_iter + 1).mean())
@@ -639,7 +656,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the extra keys (other shapes, CPU baseline variants)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's solution arrays to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU solver (--impl ours)")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_ours(args)
