@@ -43,7 +43,7 @@ def build_cuda(force=False, verbose=False, extra=()):
            [os.path.join(ROOT, "include", "fccqp.h")]
     if force or _stale(LIB, srcs):
         nvcc = os.environ.get("NVCC", "nvcc")
-        # FCCQP_DEV=1 compiles the developer instrumentation in (FCCQP_PROFILE / FCCQP_TRACE); the
+        # FCCQP_DEV=1 compiles the developer instrumentation in (FCCQP_PROFILE phase counters); the
         # production build leaves it out: the hot loops have to fit the instruction cache.
         dev = ["-DFCCQP_DEV"] if os.environ.get("FCCQP_DEV") else []
         _run([nvcc, *NVCC_ARCH, "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-shared",

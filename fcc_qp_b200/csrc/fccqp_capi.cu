@@ -128,43 +128,63 @@ int get_ctx(int device, DeviceCtx** out) {
 
 using KernelFn = void (*)(const fccqp::SolveParams);
 
+// Developer switches, read from the environment once per process: tests and tools/ compare kernel paths with them.
+struct DevSwitches {
+  bool no_warp = false;     // FCCQP_NO_WARP: FP64 problems with n + m <= 32 take the CTA-per-QP kernels
+  bool no_shared = false;   // FCCQP_NO_SHARED: shared-structure batches take the structure-exploiting / general kernels
+  int full_inverse_at = 0;  // FCCQP_FULL_INVERSE_AT (>= 1): ADMM iteration from which long-running QPs use the completed
+                            // inverse of L; 0 = unset: 8 for n + m <= 32 (tuned on the warp kernel), 6 above
+                            // (8 until the compact operator loop; sweep: profiles/r02_full_inverse_at_sweep.log)
+  int cta_cap = 0;          // FCCQP_CTAS_PER_SM: at most this many CTAs per SM (0: as many as fit)
+#ifdef FCCQP_DEV
+  bool profile = false;     // FCCQP_PROFILE: phase cycle counters of the structure-exploiting and general kernels
+#endif
+};
 
-// Chooses the template instance (threads >= n + m; CTAs/SM hint from the packed-matrix footprint).
-int pick_kernel(const DeviceCtx& ctx, int n, int m, int nc, KernelFn* fn, int* threads, size_t* smem,
-                KernelFn* fn_shared = nullptr, KernelFn* fn_f32 = nullptr, bool adapt = false) {
+const DevSwitches& dev_switches() {
+  static const DevSwitches s = [] {
+    DevSwitches d;
+    d.no_warp = getenv("FCCQP_NO_WARP") != nullptr;
+    d.no_shared = getenv("FCCQP_NO_SHARED") != nullptr;
+    if (const char* v = getenv("FCCQP_FULL_INVERSE_AT")) d.full_inverse_at = atoi(v) < 1 ? 1 : atoi(v);
+    if (const char* v = getenv("FCCQP_CTAS_PER_SM")) d.cta_cap = atoi(v);
+#ifdef FCCQP_DEV
+    d.profile = getenv("FCCQP_PROFILE") != nullptr;
+#endif
+    return d;
+  }();
+  return s;
+}
+
+// Whether the CTA-per-QP kernels take the shape: one thread per padded KKT row, at most 256 rows, the packed matrix in
+// shared memory.
+int check_shape(const DeviceCtx& ctx, int n, int m, int nc) {
   const int N = n + m;
   if (N < 1) return fail(FCCQP_E_INVALID, "n + m must be >= 1");
-  fccqp::Layout l(n, m, nc);
-  *smem = l.bytes();
-  if (l.N8 > 256 || *smem > (size_t)ctx.max_smem_optin)
+  const fccqp::Layout l(n, m, nc);
+  if (l.N8 > 256 || l.bytes() > (size_t)ctx.max_smem_optin)
     return fail(FCCQP_E_UNSUPPORTED,
                 "n + m = %d (padded %d) needs %zu B of shared memory per QP (limit %d B, 256 rows): too large "
-                "for the shared-memory-resident kernels", N, l.N8, *smem, ctx.max_smem_optin);
-  // one thread per padded KKT row; 4 CTAs/SM for the <= 128-row shapes (Cassie, quadruped)
-  if (l.N8 <= 128) {
-    *threads = 128;
-    *fn = adapt ? (KernelFn)fccqp::fccqp_solve_kernel<128, 4, false, false, true> : (KernelFn)fccqp::fccqp_solve_kernel<128, 4, false, false>;
-    if (fn_shared) *fn_shared = (KernelFn)fccqp::fccqp_solve_kernel<128, 4, true, false>;
-    if (fn_f32) *fn_f32 = adapt ? (KernelFn)fccqp::fccqp_solve_kernel<128, 4, false, true, true> : (KernelFn)fccqp::fccqp_solve_kernel<128, 4, false, true>;
-  } else {
-    *threads = 256;
-    *fn = adapt ? (KernelFn)fccqp::fccqp_solve_kernel<256, 2, false, false, true> : (KernelFn)fccqp::fccqp_solve_kernel<256, 2, false, false>;
-    if (fn_shared) *fn_shared = (KernelFn)fccqp::fccqp_solve_kernel<256, 2, true, false>;
-    if (fn_f32) *fn_f32 = adapt ? (KernelFn)fccqp::fccqp_solve_kernel<256, 2, false, true, true> : (KernelFn)fccqp::fccqp_solve_kernel<256, 2, false, true>;
-  }
+                "for the shared-memory-resident kernels", N, l.N8, l.bytes(), ctx.max_smem_optin);
   return FCCQP_OK;
 }
 
-// Structure-exploiting kernel instances (fccqp_struct.cuh): threads >= max(n, padded reduced KKT size).
-int pick_struct_kernel(const fccqp::StructLayout& sl, int n, KernelFn* fn, int* threads, bool adapt) {
-  const int need = n > sl.N8c ? n : sl.N8c;
-  using namespace fccqp;
-  if (need <= 64) { *threads = 64; *fn = adapt ? (KernelFn)fccqp_struct_kernel<64, 8, true> : (KernelFn)fccqp_struct_kernel<64, 8, false>; }
-  else if (need <= 96) { *threads = 96; *fn = adapt ? (KernelFn)fccqp_struct_kernel<96, 5, true> : (KernelFn)fccqp_struct_kernel<96, 5, false>; }
-  else if (need <= 128) { *threads = 128; *fn = adapt ? (KernelFn)fccqp_struct_kernel<128, 4, true> : (KernelFn)fccqp_struct_kernel<128, 4, false>; }
-  else if (need <= 256) { *threads = 256; *fn = adapt ? (KernelFn)fccqp_struct_kernel<256, 2, true> : (KernelFn)fccqp_struct_kernel<256, 2, false>; }
-  else return 1;
-  return 0;
+// CTA-per-QP kernel instances (fccqp_kernel.cuh): 4 CTAs/SM for the <= 128-row shapes (Cassie, quadruped), 2 above.
+// Shared-structure batches have no adaptive-rho instance: they run with a fixed rho.
+template <int kThreads, int kMinBlocks>
+KernelFn solve_instance(bool shared, bool f32, bool adapt) {
+  using fccqp::fccqp_solve_kernel;
+  if (shared) return fccqp_solve_kernel<kThreads, kMinBlocks, true, false>;
+  if (f32) return adapt ? fccqp_solve_kernel<kThreads, kMinBlocks, false, true, true> : fccqp_solve_kernel<kThreads, kMinBlocks, false, true>;
+  return adapt ? fccqp_solve_kernel<kThreads, kMinBlocks, false, false, true> : fccqp_solve_kernel<kThreads, kMinBlocks, false, false>;
+}
+KernelFn pick_kernel(int threads, bool shared, bool f32, bool adapt) {
+  return threads == 128 ? solve_instance<128, 4>(shared, f32, adapt) : solve_instance<256, 2>(shared, f32, adapt);
+}
+
+template <int kThreads, int kMinBlocks>
+KernelFn struct_instance(bool adapt) {
+  return adapt ? fccqp::fccqp_struct_kernel<kThreads, kMinBlocks, true> : fccqp::fccqp_struct_kernel<kThreads, kMinBlocks, false>;
 }
 
 // Host-side twin of fccqp::struct_classify for callers whose data is in host memory (no probe launch,
@@ -194,330 +214,283 @@ bool host_classify(int n, int m, const double* Q, long long q_rs, long long q_cs
   return ok;
 }
 
+// Launch geometry of fn: as many CTAs per SM as fit (occupancy calculator, cached per device; at most
+// FCCQP_CTAS_PER_SM), and no more CTAs than the batch fills at qps_per_cta QPs each.
+int geometry(DeviceCtx& ctx, KernelFn fn, int threads, size_t smem, int B, int qps_per_cta, LaunchInfo* li) {
+  int c = 0;
+  {
+    std::lock_guard<std::mutex> lk(ctx.mu);
+    const auto key = std::make_pair((const void*)fn, smem);
+    auto it = ctx.occupancy.find(key);
+    if (it != ctx.occupancy.end()) c = it->second;
+    else {
+      // the attribute is per kernel, the smem size per problem shape: raise it to the device maximum once
+      CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx.max_smem_optin));
+      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c, fn, threads, smem));
+      if (c < 1) return fail(FCCQP_E_UNSUPPORTED, "kernel does not fit on an SM (smem %zu B)", smem);
+      ctx.occupancy[key] = c;
+    }
+  }
+  const int cap = dev_switches().cta_cap;
+  if (cap > 0 && cap < c) c = cap;
+  const int need = (B + qps_per_cta - 1) / qps_per_cta;
+  *li = {c * ctx.num_sms < need ? c * ctx.num_sms : need, threads, (int)smem, c};
+  return FCCQP_OK;
+}
+
+// Stream-ordered scratch of one launch_solve call: one allocation and one memset of its header, so that any number of
+// calls may be in flight on any number of streams.  Offsets in 32-bit words.
+struct Scratch {
+  static constexpr size_t kWork = 0;       // work counter of the first launch
+  static constexpr size_t kWork2 = 1;      // work counter of the second launch
+  static constexpr size_t kListCount = 2;  // length of the hand-over list
+  static constexpr size_t kProbe = 4;      // [4, 8): structure probe (atomicMax)
+  static constexpr size_t kLpt = 8;        // [8, 10): counters of lpt_order_kernel
+  static constexpr size_t kHeader = 16;    // then [B] the hand-over list, then [B] the LPT order
+  unsigned int* w = nullptr;
+  size_t B = 0;
+  int* list() const { return reinterpret_cast<int*>(w + kHeader); }
+  int* order() const { return reinterpret_cast<int*>(w + kHeader + B); }
+};
+
+// Allocates the scratch of a call.  FCCQP_SCHEDULE_LPT, when the batch holds at least two QPs for each of the `slots`
+// that run at once: QPs whose previous solve ran long go to the front of the processing order (p.index_list).
+int begin_call(fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long long slots, Scratch* s) {
+  const bool lpt = lpt_hint && p.n_iter != nullptr && p.B >= 2 * slots;
+  s->B = (size_t)p.B;
+  CUDA_TRY(cudaMallocAsync(&s->w, (Scratch::kHeader + (lpt ? 2 : 1) * s->B) * sizeof(unsigned int), stream));
+  CUDA_TRY(cudaMemsetAsync(s->w, 0, Scratch::kHeader * sizeof(unsigned int), stream));
+  p.work_counter = s->w + Scratch::kWork;
+  if (lpt) {
+    fccqp::lpt_order_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.n_iter, p.B, p.full_inverse_at, s->order(),
+                                                                   s->w + Scratch::kLpt, s->w + Scratch::kLpt + 1);
+    CUDA_TRY(cudaGetLastError());
+    p.index_list = s->order();
+  }
+  return FCCQP_OK;
+}
+
+// Frees the scratch (stream-ordered) and records the call for fccqp_kernel_launch_count, fccqp_last_launch_info and
+// fccqp_last_struct_info.
+int end_call(const Scratch& s, cudaStream_t stream, int launches, const LaunchInfo& li, const StructInfo& si) {
+  CUDA_TRY(cudaFreeAsync(s.w, stream));
+  g_launches.fetch_add(launches);
+  std::lock_guard<std::mutex> lk(g_info_mu);
+  g_last_launch = li;
+  g_last_struct = si;
+  return FCCQP_OK;
+}
+
+StructInfo dense_info(const DeviceCtx& ctx, int rows) {
+  StructInfo si;
+  si.rows = si.rows_dense = rows;
+  si.device = ctx.device;
+  return si;
+}
+
+#ifdef FCCQP_DEV
+// FCCQP_PROFILE: per-phase cycle counters of one launch (SolveParams::prof), summed over its CTAs and printed per QP
+// to stderr.  Slot 14 counts the QPs; slot 15, when it has no name, the ADMM iterations.
+struct PhaseProfile {
+  unsigned long long* d = nullptr;
+  int start(cudaStream_t stream, fccqp::SolveParams* p) {
+    if (!dev_switches().profile) return FCCQP_OK;
+    CUDA_TRY(cudaMalloc(&d, 16 * sizeof(unsigned long long)));
+    CUDA_TRY(cudaMemsetAsync(d, 0, 16 * sizeof(unsigned long long), stream));
+    p->prof = d;
+    return FCCQP_OK;
+  }
+  int report(cudaStream_t stream, const char* kernel, const char* const (&names)[16], int B, int grid) {
+    if (!d) return FCCQP_OK;
+    unsigned long long h[16];
+    CUDA_TRY(cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    CUDA_TRY(cudaFree(d));
+    const double qps = (double)h[14];
+    double tot = 0;
+    for (int i = 0; i < 16; ++i) if (names[i]) tot += (double)h[i];
+    fprintf(stderr, "[fccqp %s profile] B=%d grid=%d qps=%llu", kernel, B, grid, h[14]);
+    if (!names[15]) fprintf(stderr, " iters=%llu", h[15]);
+    fprintf(stderr, " cycles/QP=%.0f\n", qps > 0 ? tot / qps : 0.0);
+    for (int i = 0; i < 16; ++i)
+      if (names[i])
+        fprintf(stderr, "   %-14s %10.0f cyc/QP  %5.1f%%\n", names[i], qps > 0 ? (double)h[i] / qps : 0.0,
+                tot > 0 ? 100.0 * (double)h[i] / tot : 0.0);
+    return FCCQP_OK;
+  }
+};
+const char* const kStructPhases[16] = {"fetch+vectors", "classify", "zero+scatter", "wait-copies", "C+diag", "factor",
+                                       "x: rhs", "x: solve", "project/exit", "epilogue", "x: refine | op: F", "x: recover",
+                                       "x: rest", "op: inv(L)", nullptr, "op: G"};
+const char* const kGeneralPhases[16] = {"stage-in", "assemble", "sigma/rhs0", "ldlt-acc+diag", "full-inverse", "-",
+                                        "xinv32", "kkt-solve", "presolve-tail", "admm-project", "epilogue",
+                                        "B-work-w0w2", "B-work-w1w3", "B-barrier-w0", nullptr, nullptr};
+#endif
+
 // Small problems (n + m <= 32): one QP per warp (fccqp_warp.cuh), four warps per CTA, each pulling QPs from the work
 // counter on its own; shared memory per CTA = 4 private (n + m) x ((n + m) | 1) slabs.
 // f32: the FP32 arithmetic instance (FCCQP_PRECISION_FP32: float32 problem data, float slabs).
-int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool f32 = false, bool lpt_hint = false) {
+int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool f32, bool lpt_hint) {
   constexpr int kW = 4;
   const int N = p.n + p.m;
   const size_t smem = (size_t)kW * N * (N | 1) * (f32 ? sizeof(float) : sizeof(double));
   KernelFn fn = f32 ? (KernelFn)fccqp::fccqp_warp_kernel<kW, 6, float> : (KernelFn)fccqp::fccqp_warp_kernel<kW, 6, double>;
   // (measured, tools/bench_small.py: 6 CTAs x 4 warps at 80 registers beats 8 x 4 at 64 and 4 x 4 at 128 on every shape but n = 6;
   //  float instance, tools/fp32_occ.py: 6 / 8 / 10 / 12 CTAs -> 82.7 / 78.5 / 71.4 / 70.5 M QP/s at n = 6, 22.4 / 23.1 / 21.1 / 21.7 at n = 24)
-  int ctas_per_sm = 0;
-  {
-    std::lock_guard<std::mutex> lk(ctx.mu);
-    const auto key = std::make_pair((const void*)fn, smem);
-    auto it = ctx.occupancy.find(key);
-    if (it != ctx.occupancy.end()) ctas_per_sm = it->second;
-    else {
-      CUDA_TRY(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx.max_smem_optin));
-      CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas_per_sm, fn, 32 * kW, smem));
-      if (ctas_per_sm < 1) return fail(FCCQP_E_UNSUPPORTED, "warp kernel does not fit on an SM (smem %zu B)", smem);
-      ctx.occupancy[key] = ctas_per_sm;
-    }
-  }
-  static const int cta_cap = getenv("FCCQP_CTAS_PER_SM") ? atoi(getenv("FCCQP_CTAS_PER_SM")) : 0;  // developer aid
-  if (cta_cap > 0 && cta_cap < ctas_per_sm) ctas_per_sm = cta_cap;
-  int grid = ctas_per_sm * ctx.num_sms;
-  if (grid > (p.B + kW - 1) / kW) grid = (p.B + kW - 1) / kW;
-  unsigned int* scr = nullptr;   // the work counter of this call (stream-ordered: any number of calls may be in flight)
-  const bool lpt = lpt_hint && p.n_iter != nullptr && p.B >= 2 * kW * ctas_per_sm * ctx.num_sms;
-  CUDA_TRY(cudaMallocAsync(&scr, (8 + (lpt ? (size_t)p.B : 0)) * sizeof(unsigned int), stream));
-  CUDA_TRY(cudaMemsetAsync(scr, 0, 8 * sizeof(unsigned int), stream));
-  p.work_counter = scr;
-  if (lpt) {   // FCCQP_SCHEDULE_LPT: [8, 8 + B) the processing order, its two counters in [4], [5]
-    int* const order = reinterpret_cast<int*>(scr + 8);
-    fccqp::lpt_order_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.n_iter, p.B, p.full_inverse_at, order, scr + 4, scr + 5);
-    CUDA_TRY(cudaGetLastError());
-    p.index_list = order;
-  }
-  fn<<<grid, 32 * kW, smem, stream>>>(p);
+  LaunchInfo li;
+  Scratch s;
+  int rc = geometry(ctx, fn, 32 * kW, smem, p.B, kW, &li);
+  if (!rc) rc = begin_call(p, stream, lpt_hint, (long long)kW * li.ctas_per_sm * ctx.num_sms, &s);
+  if (rc) return rc;
+  fn<<<li.grid, li.block, smem, stream>>>(p);
   CUDA_TRY(cudaGetLastError());
-  CUDA_TRY(cudaFreeAsync(scr, stream));
-  g_launches.fetch_add(1);
-  StructInfo si;
-  si.rows = si.rows_dense = N;
-  si.device = ctx.device;
-  std::lock_guard<std::mutex> lk(g_info_mu);
-  g_last_launch = {grid, 32 * kW, (int)smem, ctas_per_sm};
-  g_last_struct = si;
-  return FCCQP_OK;
+  return end_call(s, stream, 1, li, dense_info(ctx, N));
 }
 
-// Launches the fused solve on `stream` for device-resident data described by p
-// (work counters / device-side lists are allocated here, stream-ordered).
-// precision: fccqp_precision of the call (FP32_DATA and FP32: float32 problem data behind the pointers of p; FP32: FP32
-// arithmetic too where a kernel for it exists -- the warp kernel -- and FP32_DATA's FP64 arithmetic otherwise)
-int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int precision = FCCQP_PRECISION_FP64,
-                 const StructHint* hint_in = nullptr) {
-  if (p.B == 0) return FCCQP_OK;
-  KernelFn fn, fn_shared, fn_f32; int threads; size_t smem;
-  int rc = pick_kernel(ctx, p.n, p.m, p.nc, &fn, &threads, &smem, &fn_shared, &fn_f32, p.adapt_k > 0);
+// Shared-structure batch (one Q and one A_eq for the whole batch): every CTA caches its KKT factorization
+// (SolveParams::shared_mode).  Cold: a pre-solve launch hands the QPs that need ADMM iterations to an ADMM launch.
+// Warm (an MPC loop re-solving around one linearisation with carried duals): no pre-solve, the ADMM launch alone.
+int launch_shared(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s) {
+  const int threads = p.lay.N8 <= 128 ? 128 : 256;
+  KernelFn fn = pick_kernel(threads, true, false, false);
+  LaunchInfo li;
+  int rc = geometry(ctx, fn, threads, p.lay.bytes(), p.B, 1, &li);
   if (rc) return rc;
-  const bool f32 = precision != FCCQP_PRECISION_FP64;
-  if (f32) fn = fn_f32;   // float32 problem data: same launch geometry, widening stage-in
-  p.lay = fccqp::Layout(p.n, p.m, p.nc);
-  // developer switch: FCCQP_FIRST_UPDATE_IDENTITY=0 solves the (mathematically redundant) first x-update of cold QPs
-  static const int fui = getenv("FCCQP_FIRST_UPDATE_IDENTITY") ? atoi(getenv("FCCQP_FIRST_UPDATE_IDENTITY")) : 1;
-  p.first_update_identity = fui != 0;
-  // developer switch: ADMM iteration at which long-running QPs complete inv(L) (huge value = never)
-  static const int fia = getenv("FCCQP_FULL_INVERSE_AT") ? atoi(getenv("FCCQP_FULL_INVERSE_AT")) : 6;   // (8 until the compact operator loop; sweep: profiles/r02_full_inverse_at_sweep.log)
-  p.full_inverse_at = fia < 1 ? 1 : fia;
-  // iterative refinement of the reduced cold pre-solve: FCCQP_STRUCTURE_REFINE of the caller (developer override
-  // FCCQP_STRUCT_REFINE=0/1, read per call)
-  p.struct_refine = getenv("FCCQP_STRUCT_REFINE") ? atoi(getenv("FCCQP_STRUCT_REFINE")) : (hint_in ? hint_in->refine : 0);
-  p.struct_prefetch = getenv("FCCQP_STRUCT_PREFETCH") ? atoi(getenv("FCCQP_STRUCT_PREFETCH")) : 1;
-  p.struct_bulk = getenv("FCCQP_STRUCT_BULK") ? atoi(getenv("FCCQP_STRUCT_BULK")) : 1;
-  // problem-size-specialised mapping: a QP whose KKT matrix fits one row per lane goes to the warp-per-QP kernel
-  // (FCCQP_NO_WARP=1: the CTA-per-QP kernels, for A/B tests)
-  const bool lpt_hint = hint_in && hint_in->lpt;
-  if (p.n + p.m <= 32 && !getenv("FCCQP_FULL_INVERSE_AT")) p.full_inverse_at = 8;   // the warp kernel keeps its own (tuned) switch point
-  if (!f32 && p.n + p.m <= 32 && !getenv("FCCQP_NO_WARP")) return launch_warp(ctx, p, stream, false, lpt_hint);
-  if (precision == FCCQP_PRECISION_FP32 && p.n + p.m <= 32) return launch_warp(ctx, p, stream, true, lpt_hint);
-  auto occupancy_of = [&](KernelFn f, int thr, size_t sm, int* out) -> int {
-    std::lock_guard<std::mutex> lk(ctx.mu);
-    const auto key = std::make_pair((const void*)f, sm);
-    auto it = ctx.occupancy.find(key);
-    if (it != ctx.occupancy.end()) { *out = it->second; return FCCQP_OK; }
-    // the attribute is per kernel, the smem size per problem shape: raise it to the device maximum once
-    CUDA_TRY(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx.max_smem_optin));
-    int c = 0;
-    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c, f, thr, sm));
-    if (c < 1) return fail(FCCQP_E_UNSUPPORTED, "kernel does not fit on an SM (smem %zu B)", sm);
-    ctx.occupancy[key] = c;
-    *out = c;
-    return FCCQP_OK;
-  };
-  int ctas_per_sm = 0;
-  if ((rc = occupancy_of(fn, threads, smem, &ctas_per_sm))) return rc;
-  static const int cta_cap = getenv("FCCQP_CTAS_PER_SM") ? atoi(getenv("FCCQP_CTAS_PER_SM")) : 0;  // developer aid
-  if (cta_cap > 0 && cta_cap < ctas_per_sm) ctas_per_sm = cta_cap;
-  int grid = ctas_per_sm * ctx.num_sms;
-  if (grid > p.B) grid = p.B;
-
-  // Stream-ordered scratch of this call: [0] work counter, [1] second work counter, [2] length of the
-  // device-side QP list, [3] spare, [4..7] structure probe, [8..8+B) the list.  One allocation per call, so
-  // any number of calls may be in flight on any number of streams.
-  unsigned int* scr = nullptr;
-  const bool lpt = hint_in && hint_in->lpt && p.n_iter != nullptr && p.B >= 2 * ctas_per_sm * ctx.num_sms;
-  CUDA_TRY(cudaMallocAsync(&scr, ((size_t)p.B * (lpt ? 2 : 1) + 8 + (lpt ? 2 : 0)) * sizeof(unsigned int), stream));
-  CUDA_TRY(cudaMemsetAsync(scr, 0, 8 * sizeof(unsigned int), stream));
-  p.work_counter = scr;
-  if (lpt) {
-    // FCCQP_SCHEDULE_LPT: lanes whose previous solve ran long go to the front of the processing order
-    // ([8 + B, 8 + 2B) the order, then its two counters)
-    int* const order = reinterpret_cast<int*>(scr + 8 + p.B);
-    unsigned int* const cnt = scr + 8 + 2 * (size_t)p.B;
-    CUDA_TRY(cudaMemsetAsync(cnt, 0, 2 * sizeof(unsigned int), stream));
-    fccqp::lpt_order_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.n_iter, p.B, p.full_inverse_at, order, cnt, cnt + 1);
-    CUDA_TRY(cudaGetLastError());
-    p.index_list = order;
-  }
-  unsigned int* const counter2 = scr + 1;
-  unsigned int* const list_count = scr + 2;
-  int* const list = reinterpret_cast<int*>(scr + 8);
-  auto finish = [&](int launches, const LaunchInfo& li, const StructInfo& si) -> int {
-    CUDA_TRY(cudaFreeAsync(scr, stream));
-    g_launches.fetch_add(launches);
-    std::lock_guard<std::mutex> lk(g_info_mu);
-    g_last_launch = li;
-    g_last_struct = si;
-    return FCCQP_OK;
-  };
-  StructInfo no_struct;
-  no_struct.rows = no_struct.rows_dense = p.lay.N8;
-  no_struct.device = ctx.device;
-
-  // Shared-structure batches (one Q and one A_eq for the whole batch, cold): two launches, each with
-  // its KKT factorization cached per CTA (SolveParams::shared_mode).  Worth it once every CTA sees
-  // several QPs; FCCQP_NO_SHARED=1 forces the general path (tests compare the two).
-  static const bool no_shared = getenv("FCCQP_NO_SHARED") != nullptr;
-  const bool shared_structure = !no_shared && !f32 && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) && p.B >= 4 * ctas_per_sm * ctx.num_sms;
-  if (shared_structure) {
-    int c2 = 0;
-    if ((rc = occupancy_of(fn_shared, threads, smem, &c2))) return rc;
-  }
-  if (shared_structure && p.warm) {
-    // warm shared-structure batch (an MPC loop re-solving around one linearisation with carried duals):
-    // no pre-solve, so ONE launch of the ADMM mode over all QPs with the rho-KKT operator cached per CTA
-    fccqp::SolveParams b = p;
-    b.shared_mode = 2;
-    fn_shared<<<grid, threads, smem, stream>>>(b);
-    CUDA_TRY(cudaGetLastError());
-    return finish(1, {grid, threads, (int)smem, ctas_per_sm}, no_struct);
-  }
-  if (shared_structure) {
+  p.shared_mode = 2;
+  if (!p.warm) {
     fccqp::SolveParams a = p;
     a.shared_mode = 1;
-    a.pending_count = list_count;
-    a.pending_list = list;
-    static const bool timing = getenv("FCCQP_SHARED_TIMING") != nullptr;   // developer aid: per-launch times
-    cudaEvent_t te[3] = {nullptr, nullptr, nullptr};
-    if (timing) { for (auto& e : te) CUDA_TRY(cudaEventCreate(&e)); CUDA_TRY(cudaEventRecord(te[0], stream)); }
-    fn_shared<<<grid, threads, smem, stream>>>(a);
+    a.pending_count = s.w + Scratch::kListCount;
+    a.pending_list = s.list();
+    fn<<<li.grid, li.block, li.smem, stream>>>(a);
     CUDA_TRY(cudaGetLastError());
-    if (timing) CUDA_TRY(cudaEventRecord(te[1], stream));
-    fccqp::SolveParams b = p;
-    b.shared_mode = 2;
-    b.count_dev = list_count;
-    b.index_list = list;
-    b.work_counter = counter2;
-    fn_shared<<<grid, threads, smem, stream>>>(b);
-    CUDA_TRY(cudaGetLastError());
-    if (timing) {
-      unsigned int pending = 0;
-      CUDA_TRY(cudaEventRecord(te[2], stream));
-      CUDA_TRY(cudaMemcpyAsync(&pending, list_count, sizeof(pending), cudaMemcpyDeviceToHost, stream));
-      CUDA_TRY(cudaEventSynchronize(te[2]));
-      CUDA_TRY(cudaStreamSynchronize(stream));
-      float m1 = 0.f, m2 = 0.f;
-      cudaEventElapsedTime(&m1, te[0], te[1]); cudaEventElapsedTime(&m2, te[1], te[2]);
-      fprintf(stderr, "[fccqp shared] B=%d pre-solve launch %.3f ms, ADMM launch %.3f ms over %u QPs\n", p.B, m1, m2, pending);
-      for (auto& e : te) cudaEventDestroy(e);
-    }
-    return finish(2, {grid, threads, (int)smem, ctas_per_sm}, no_struct);
+    p.count_dev = a.pending_count;
+    p.index_list = s.list();
+    p.work_counter = s.w + Scratch::kWork2;
   }
-
-  // ---- structure-exploiting kernel (fccqp_struct.cuh): QPs whose separable variables can be eliminated
-  // analytically run on a reduced KKT system; the others (if any) are appended to a device-side list and
-  // taken by the general kernel in a second launch.
-  const bool no_struct_env = getenv("FCCQP_NO_STRUCT") != nullptr;   // developer switch, read per call
-  StructHint hint;
-  if (hint_in) hint = *hint_in;
-  static const bool dev_instr = getenv("FCCQP_TRACE") != nullptr;
-  if (!no_struct_env && !dev_instr && !f32 && hint.mode != FCCQP_STRUCTURE_DENSE && p.n <= 256 && p.m <= 256 && p.m > 0) {
-    int caps[3] = {hint.caps[0], hint.caps[1], hint.caps[2]};
-    bool ok = true;
-    if (hint.mode != FCCQP_STRUCTURE_CAPS) {
-      // probe: classify up to 128 QPs spread over the batch, take the largest structure seen
-      const int ns = p.B < 128 ? p.B : 128;
-      int* d_probe = reinterpret_cast<int*>(scr + 4);
-      if (p.n <= 128 && p.m <= 128) fccqp::fccqp_struct_probe_kernel<128><<<ns, 128, 0, stream>>>(p, ns, d_probe);
-      else fccqp::fccqp_struct_probe_kernel<256><<<ns, 256, 0, stream>>>(p, ns, d_probe);
-      CUDA_TRY(cudaGetLastError());
-      int h[4] = {0, 0, 0, 0};
-      {
-        std::lock_guard<std::mutex> lk(ctx.mu);   // the pinned landing pad is per device
-        CUDA_TRY(cudaMemcpyAsync(ctx.h_probe, d_probe, sizeof(h), cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaStreamSynchronize(stream));
-        memcpy(h, ctx.h_probe, sizeof(h));
-      }
-      g_launches.fetch_add(1);
-      caps[0] = h[0]; caps[1] = h[1]; caps[2] = h[2];
-      ok = h[3] == 0;
-    }
-    if (ok && caps[0] >= 0 && caps[0] <= p.n && caps[1] >= 0 && caps[2] >= 0 && caps[0] + caps[1] + caps[2] <= p.n) {
-      fccqp::StructLayout sl(p.n, p.m, p.nc, caps[0], caps[1] + caps[2], caps[2]);   // D+ store: pass 1 eliminates D0 too
-      KernelFn sfn = nullptr; int sthreads = 0;
-      // worth it when at least one tile row of the KKT matrix goes away
-      if (sl.N8c + 8 <= p.lay.N8 && sl.bytes() <= (size_t)ctx.max_smem_optin && pick_struct_kernel(sl, p.n, &sfn, &sthreads, p.adapt_k > 0) == 0) {
-        int sctas = 0;
-        if ((rc = occupancy_of(sfn, sthreads, sl.bytes(), &sctas))) return rc;
-        if (cta_cap > 0 && cta_cap < sctas) sctas = cta_cap;
-        int sgrid = sctas * ctx.num_sms;
-        if (sgrid > p.B) sgrid = p.B;
-        fccqp::SolveParams a = p;
-        a.slay = sl;
-        a.pending_count = list_count;
-        a.pending_list = list;
-        static const bool sprofile = getenv("FCCQP_PROFILE") != nullptr;  // developer aid: phase cycle counters
-        unsigned long long* d_sprof = nullptr;
-        if (sprofile) {
-          CUDA_TRY(cudaMalloc(&d_sprof, 16 * sizeof(unsigned long long)));
-          CUDA_TRY(cudaMemsetAsync(d_sprof, 0, 16 * sizeof(unsigned long long), stream));
-          a.prof = d_sprof;
-        }
-        // per-CTA global scratch of the full-space operator of long-running QPs (build_full_op): B, Z, X, Y tiles and 1/h
-        // sized for every variable eliminated; FCCQP_STRUCT_FULLOP=0 keeps the operator in the reduced space (ablation)
-        double* d_opscr = nullptr;
-        {
-          const char* fo = getenv("FCCQP_STRUCT_FULLOP");
-          if (!(fo && atoi(fo) == 0)) {
-            const long long neT = sl.n8 >> 3, NBr = sl.nr8c >> 3, mt = sl.mt;
-            const long long per = (2 * mt * neT + neT * NBr + neT * (neT + 1) / 2) * 64 + 8 * neT;
-            CUDA_TRY(cudaMallocAsync(&d_opscr, (size_t)sgrid * per * sizeof(double), stream));
-            a.op_scratch = d_opscr;
-            a.op_stride = per;
-          }
-        }
-        sfn<<<sgrid, sthreads, sl.bytes(), stream>>>(a);
-        CUDA_TRY(cudaGetLastError());
-        if (d_opscr) CUDA_TRY(cudaFreeAsync(d_opscr, stream));
-        if (sprofile) {
-          unsigned long long h[16];
-          CUDA_TRY(cudaMemcpyAsync(h, d_sprof, sizeof(h), cudaMemcpyDeviceToHost, stream));
-          CUDA_TRY(cudaStreamSynchronize(stream));
-          CUDA_TRY(cudaFree(d_sprof));
-          static const char* names[16] = {"fetch+vectors", "classify", "zero+scatter", "wait-copies", "C+diag", "factor", "x: rhs",
-                                          "x: solve", "project/exit", "epilogue", "x: refine | op: F", "x: recover", "x: rest",
-                                          "op: inv(L)", "(count)", "op: G"};
-          double tot = 0;
-          for (int i = 0; i < 16; ++i) if (i != 14) tot += (double)h[i];
-          fprintf(stderr, "[fccqp struct profile] B=%d grid=%d qps=%llu cycles/QP=%.0f\n", p.B, sgrid, h[14], h[14] ? tot / (double)h[14] : 0.0);
-          for (int i = 0; i < 16; ++i)
-            if (i != 14) fprintf(stderr, "   %-14s %10.0f cyc/QP  %5.1f%%\n", names[i], h[14] ? (double)h[i] / (double)h[14] : 0.0,
-                    tot > 0 ? 100.0 * (double)h[i] / tot : 0.0);
-        }
-        fccqp::SolveParams b = p;
-        b.count_dev = list_count;
-        b.index_list = list;
-        b.work_counter = counter2;
-        fn<<<grid, threads, smem, stream>>>(b);
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, list_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, stream));
-        StructInfo si;
-        si.used = 1; si.nr = caps[0]; si.ndp = caps[1]; si.nd0 = caps[2]; si.rows = sl.N8c; si.rows_dense = p.lay.N8; si.device = ctx.device;
-        return finish(2, {sgrid, sthreads, (int)sl.bytes(), sctas}, si);
-      }
-    }
-  }
-
-  static const bool profile = getenv("FCCQP_PROFILE") != nullptr;  // developer aid: phase cycle counters
-  unsigned long long* d_prof = nullptr;
-  if (profile) {
-    CUDA_TRY(cudaMalloc(&d_prof, 16 * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemsetAsync(d_prof, 0, 16 * sizeof(unsigned long long), stream));
-    p.prof = d_prof;
-  }
-  static const char* trace_path = getenv("FCCQP_TRACE");  // developer aid: per-warp event trace of CTA 0
-  unsigned long long* d_trace = nullptr;
-  if (trace_path) {
-    CUDA_TRY(cudaMalloc(&d_trace, 8 * 4096 * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemsetAsync(d_trace, 0, 8 * 4096 * sizeof(unsigned long long), stream));
-    p.trace = d_trace;
-  }
-  fn<<<grid, threads, smem, stream>>>(p);
+  fn<<<li.grid, li.block, li.smem, stream>>>(p);
   CUDA_TRY(cudaGetLastError());
-  if (trace_path) {
-    std::vector<unsigned long long> h(8 * 4096);
-    CUDA_TRY(cudaMemcpyAsync(h.data(), d_trace, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    CUDA_TRY(cudaFree(d_trace));
-    if (FILE* f = fopen(trace_path, "w")) {
-      for (int w = 0; w < 8; ++w)
-        for (int e = 0; e < 4096 && h[w * 4096 + e]; ++e)
-          fprintf(f, "%d %llu %llu\n", w, h[w * 4096 + e] >> 8, h[w * 4096 + e] & 255ull);
-      fclose(f);
+  return end_call(s, stream, p.warm ? 1 : 2, li, dense_info(ctx, p.lay.N8));
+}
+
+constexpr int kNotApplicable = 1;
+
+// Structure-exploiting kernel (fccqp_struct.cuh): QPs whose separable variables can be eliminated analytically run on
+// a reduced KKT system; the others (if any) are appended to a device-side list that the general kernel (geometry gli)
+// takes in a second launch.  Returns kNotApplicable, with nothing launched but the probe, when the reduction does not pay.
+int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stream, const Scratch& s, const StructHint& hint,
+                  KernelFn general, const LaunchInfo& gli) {
+  int caps[3] = {hint.caps[0], hint.caps[1], hint.caps[2]};
+  if (hint.mode != FCCQP_STRUCTURE_CAPS) {
+    // probe: classify up to 128 QPs spread over the batch, take the largest structure seen
+    const int ns = p.B < 128 ? p.B : 128;
+    int* d_probe = reinterpret_cast<int*>(s.w + Scratch::kProbe);
+    if (p.n <= 128 && p.m <= 128) fccqp::fccqp_struct_probe_kernel<128><<<ns, 128, 0, stream>>>(p, ns, d_probe);
+    else fccqp::fccqp_struct_probe_kernel<256><<<ns, 256, 0, stream>>>(p, ns, d_probe);
+    CUDA_TRY(cudaGetLastError());
+    int h[4];
+    {
+      std::lock_guard<std::mutex> lk(ctx.mu);   // the pinned landing pad is per device
+      CUDA_TRY(cudaMemcpyAsync(ctx.h_probe, d_probe, sizeof(h), cudaMemcpyDeviceToHost, stream));
+      CUDA_TRY(cudaStreamSynchronize(stream));
+      memcpy(h, ctx.h_probe, sizeof(h));
     }
+    g_launches.fetch_add(1);
+    if (h[3] != 0) return kNotApplicable;   // a structurally singular QP in the sample
+    caps[0] = h[0]; caps[1] = h[1]; caps[2] = h[2];
   }
-  if (profile) {
-    unsigned long long h[16];
-    CUDA_TRY(cudaMemcpyAsync(h, d_prof, sizeof(h), cudaMemcpyDeviceToHost, stream));
-    CUDA_TRY(cudaStreamSynchronize(stream));
-    CUDA_TRY(cudaFree(d_prof));
-    static const char* names[14] = {"stage-in", "assemble", "sigma/rhs0", "ldlt-acc+diag", "full-inverse",
-                                    "-", "xinv32", "kkt-solve", "presolve-tail", "admm-project",
-                                    "epilogue", "B-work-w0w2", "B-work-w1w3", "B-barrier-w0"};
-    double tot = 0;
-    for (int i = 0; i < 14; ++i) tot += (double)h[i];
-    fprintf(stderr, "[fccqp profile] B=%d grid=%d qps=%llu iters=%llu cycles/QP=%.0f\n", p.B, grid, h[14], h[15],
-            h[14] ? tot / (double)h[14] : 0.0);
-    for (int i = 0; i < 14; ++i)
-      fprintf(stderr, "   %-14s %10.0f cyc/QP  %5.1f%%\n", names[i], h[14] ? (double)h[i] / (double)h[14] : 0.0,
-              tot > 0 ? 100.0 * (double)h[i] / tot : 0.0);
-  }
-  return finish(1, {grid, threads, (int)smem, ctas_per_sm}, no_struct);
+  if (caps[0] < 0 || caps[0] > p.n || caps[1] < 0 || caps[2] < 0 || caps[0] + caps[1] + caps[2] > p.n) return kNotApplicable;
+  const fccqp::StructLayout sl(p.n, p.m, p.nc, caps[0], caps[1] + caps[2], caps[2]);   // D+ store: pass 1 eliminates D0 too
+  // worth it when at least one tile row of the KKT matrix goes away
+  if (sl.N8c + 8 > p.lay.N8 || sl.bytes() > (size_t)ctx.max_smem_optin) return kNotApplicable;
+  // threads >= max(n, padded reduced KKT size), at most 256 since the reduced size is below p.lay.N8
+  const int need = p.n > sl.N8c ? p.n : sl.N8c;
+  const bool adapt = p.adapt_k > 0;
+  KernelFn fn;
+  int threads;
+  if (need <= 64) { threads = 64; fn = struct_instance<64, 8>(adapt); }
+  else if (need <= 96) { threads = 96; fn = struct_instance<96, 5>(adapt); }
+  else if (need <= 128) { threads = 128; fn = struct_instance<128, 4>(adapt); }
+  else { threads = 256; fn = struct_instance<256, 2>(adapt); }
+  LaunchInfo li;
+  int rc = geometry(ctx, fn, threads, sl.bytes(), p.B, 1, &li);
+  if (rc) return rc;
+  fccqp::SolveParams a = p;
+  a.slay = sl;
+  a.pending_count = s.w + Scratch::kListCount;
+  a.pending_list = s.list();
+  // per-CTA global scratch of the full-space operator of long-running QPs (build_full_op): B, Z, X, Y tiles and 1/h
+  // sized for every variable eliminated
+  const long long neT = sl.n8 >> 3, NBr = sl.nr8c >> 3, mt = sl.mt;
+  a.op_stride = (2 * mt * neT + neT * NBr + neT * (neT + 1) / 2) * 64 + 8 * neT;
+  CUDA_TRY(cudaMallocAsync(&a.op_scratch, (size_t)li.grid * a.op_stride * sizeof(double), stream));
+#ifdef FCCQP_DEV
+  PhaseProfile prof;
+  if ((rc = prof.start(stream, &a))) return rc;
+#endif
+  fn<<<li.grid, li.block, li.smem, stream>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaFreeAsync(a.op_scratch, stream));
+#ifdef FCCQP_DEV
+  if ((rc = prof.report(stream, "struct", kStructPhases, p.B, li.grid))) return rc;
+#endif
+  fccqp::SolveParams b = p;
+  b.count_dev = a.pending_count;
+  b.index_list = s.list();
+  b.work_counter = s.w + Scratch::kWork2;
+  general<<<gli.grid, gli.block, gli.smem, stream>>>(b);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, a.pending_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, stream));
+  StructInfo si;
+  si.used = 1; si.nr = caps[0]; si.ndp = caps[1]; si.nd0 = caps[2]; si.rows = sl.N8c; si.rows_dense = p.lay.N8; si.device = ctx.device;
+  return end_call(s, stream, 2, li, si);
+}
+
+int launch_general(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s, KernelFn fn, const LaunchInfo& li) {
+#ifdef FCCQP_DEV
+  PhaseProfile prof;
+  int rc = prof.start(stream, &p);
+  if (rc) return rc;
+#endif
+  fn<<<li.grid, li.block, li.smem, stream>>>(p);
+  CUDA_TRY(cudaGetLastError());
+#ifdef FCCQP_DEV
+  if ((rc = prof.report(stream, "general", kGeneralPhases, p.B, li.grid))) return rc;
+#endif
+  return end_call(s, stream, 1, li, dense_info(ctx, p.lay.N8));
+}
+
+// Launches the solve on `stream` for device-resident data described by p (scratch allocated here, stream-ordered).
+// precision: fccqp_precision of the call (FP32_DATA and FP32: float32 problem data behind the pointers of p; FP32: FP32
+// arithmetic too where a kernel for it exists -- the warp kernel -- and FP32_DATA's FP64 arithmetic otherwise)
+int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int precision, const StructHint& hint) {
+  if (p.B == 0) return FCCQP_OK;
+  int rc = check_shape(ctx, p.n, p.m, p.nc);
+  if (rc) return rc;
+  const DevSwitches& sw = dev_switches();
+  const bool f32 = precision != FCCQP_PRECISION_FP64;
+  const bool small = p.n + p.m <= 32;   // the KKT matrix fits one row per lane
+  p.lay = fccqp::Layout(p.n, p.m, p.nc);
+  p.full_inverse_at = sw.full_inverse_at ? sw.full_inverse_at : (small ? 8 : 6);
+  p.struct_refine = hint.refine;
+  if (small && (precision == FCCQP_PRECISION_FP32 || (!f32 && !sw.no_warp)))
+    return launch_warp(ctx, p, stream, precision == FCCQP_PRECISION_FP32, hint.lpt);
+
+  // one CTA per QP; float32 problem data take the general kernel's widening instance, same geometry
+  const int threads = p.lay.N8 <= 128 ? 128 : 256;
+  KernelFn general = pick_kernel(threads, false, f32, p.adapt_k > 0);
+  LaunchInfo li;
+  Scratch s;
+  if ((rc = geometry(ctx, general, threads, p.lay.bytes(), p.B, 1, &li)) ||
+      (rc = begin_call(p, stream, hint.lpt, (long long)li.ctas_per_sm * ctx.num_sms, &s)))
+    return rc;
+  // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs
+  if (!sw.no_shared && !f32 && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) && p.B >= 4 * li.ctas_per_sm * ctx.num_sms)
+    return launch_shared(ctx, p, stream, s);
+  if (!f32 && hint.mode != FCCQP_STRUCTURE_DENSE && p.m > 0 &&
+      (rc = launch_struct(ctx, p, stream, s, hint, general, li)) != kNotApplicable)
+    return rc;
+  return launch_general(ctx, p, stream, s, general, li);
 }
 
 int check_dims(int n, int m, int nc, int lcs) {
@@ -539,6 +512,17 @@ int check_options(const fccqp_options& o) {
 }
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// The solve parameters every path needs; the data pointers are left to the caller.
+fccqp::SolveParams solve_params(int B, int n, int m, int nc, int lcs, const fccqp_options& o, bool warm) {
+  fccqp::SolveParams p{};
+  p.B = B; p.n = n; p.m = m; p.nc = nc; p.lcs = lcs;
+  p.max_iter = o.max_iter; p.rho = o.rho; p.eps_fcone = o.eps_fcone; p.eps_bound = o.eps_bound;
+  p.alpha = o.relaxation > 0.0 ? o.relaxation : 1.0;
+  p.adapt_k = o.adapt_rho_interval;
+  p.warm = warm;
+  return p;
+}
 
 }  // namespace
 
@@ -650,8 +634,7 @@ int fccqp_create(int n, int m, int nc, int lcs, int device, fccqp_handle* out) {
   DeviceCtx* ctx = nullptr;
   rc = get_ctx(device, &ctx);
   if (rc) return rc;
-  KernelFn fn; int threads; size_t smem;
-  rc = pick_kernel(*ctx, n, m, nc, &fn, &threads, &smem);
+  rc = check_shape(*ctx, n, m, nc);
   if (rc) return rc;
   CUDA_TRY(cudaSetDevice(device));
   auto* h = new fccqp_solver();
@@ -727,8 +710,9 @@ int fccqp_set_warm_start(fccqp_handle h, int warm) {
 }
 int fccqp_set_structure(fccqp_handle h, int structure) {
   if (!h) return fail(FCCQP_E_INVALID, "null handle");
-  const int mode = structure & ~(FCCQP_STRUCTURE_REFINE | FCCQP_SCHEDULE_LPT);
-  if (mode != FCCQP_STRUCTURE_AUTO && mode != FCCQP_STRUCTURE_DENSE)
+  StructHint hint;
+  hint.set(structure);
+  if (hint.mode != FCCQP_STRUCTURE_AUTO && hint.mode != FCCQP_STRUCTURE_DENSE)
     return fail(FCCQP_E_INVALID, "structure must be FCCQP_STRUCTURE_AUTO or FCCQP_STRUCTURE_DENSE (optionally | FCCQP_STRUCTURE_REFINE)");
   h->structure = structure;
   return FCCQP_OK;
@@ -771,12 +755,8 @@ int fccqp_solve(fccqp_handle h, const double* Q, ptrdiff_t q_rs, ptrdiff_t q_cs,
   memcpy(sub, ub, sizeof(double) * n);
   CUDA_TRY(cudaMemcpyAsync(h->d_in, h->h_in, h->in_doubles * sizeof(double), cudaMemcpyHostToDevice, h->stream));
 
-  fccqp::SolveParams p{};
-  p.B = 1; p.n = n; p.m = m; p.nc = nc; p.lcs = h->lcs;
-  p.max_iter = h->opt.max_iter; p.rho = h->opt.rho; p.eps_fcone = h->opt.eps_fcone; p.eps_bound = h->opt.eps_bound;
-  p.alpha = h->opt.relaxation > 0.0 ? h->opt.relaxation : 1.0;
-  p.adapt_k = h->opt.adapt_rho_interval;
-  p.warm = h->warm;  // warm with no earlier Solve starts from the zero state, like the reference object
+  // warm with no earlier Solve starts from the zero state, like the reference object
+  fccqp::SolveParams p = solve_params(1, n, m, nc, h->lcs, h->opt, h->warm != 0);
   double* d = h->d_in;
   p.Q = d; p.q_bs = 0; p.q_rs = n; p.q_cs = 1; d += (size_t)n * n;
   p.A = d; p.a_bs = 0; p.a_rs = k_a_rs; p.a_cs = k_a_cs; d += (size_t)m * n;
@@ -797,7 +777,7 @@ int fccqp_solve(fccqp_handle h, const double* Q, ptrdiff_t q_rs, ptrdiff_t q_cs,
   if (want_struct && m > 0 &&
       host_classify(n, m, sQ, n, 1, sA, k_a_rs, k_a_cs, &hint.caps[0], &hint.caps[1], &hint.caps[2]))
     hint.mode = FCCQP_STRUCTURE_CAPS;
-  int rc = launch_solve(*h->ctx, p, h->stream, FCCQP_PRECISION_FP64, &hint);
+  int rc = launch_solve(*h->ctx, p, h->stream, FCCQP_PRECISION_FP64, hint);
   if (rc) return rc;
   CUDA_TRY(cudaMemcpyAsync(h->h_out, h->d_x, sizeof(double) * (n + 8), cudaMemcpyDeviceToHost, h->stream));   // packed outputs
   CUDA_TRY(cudaStreamSynchronize(h->stream));
@@ -868,16 +848,6 @@ static void host_struct_hint(const fccqp_batch_desc& d, StructHint* out) {
 // ---------------------------------------------------------------------------
 // batched entry point
 // ---------------------------------------------------------------------------
-static int fill_params(const fccqp_batch_desc& d, fccqp::SolveParams& p) {
-  p.B = d.batch; p.n = d.n; p.m = d.m; p.nc = d.nc; p.lcs = d.lambda_c_start;
-  p.max_iter = d.options.max_iter; p.rho = d.options.rho;
-  p.eps_fcone = d.options.eps_fcone; p.eps_bound = d.options.eps_bound;
-  p.alpha = d.options.relaxation > 0.0 ? d.options.relaxation : 1.0;
-  p.adapt_k = d.options.adapt_rho_interval;
-  p.warm = d.warm_start != 0;
-  return FCCQP_OK;
-}
-
 static int validate_desc(const fccqp_batch_desc* d) {
   if (!d) return fail(FCCQP_E_INVALID, "desc is null");
   if (d->abi_version != FCCQP_ABI_VERSION)
@@ -912,8 +882,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
   const int n = d.n, m = d.m, nc = d.nc, B = d.batch;
 
   if (d.memory_space == FCCQP_MEM_DEVICE) {
-    fccqp::SolveParams p{};
-    fill_params(d, p);
+    fccqp::SolveParams p = solve_params(B, n, m, nc, d.lambda_c_start, d.options, d.warm_start != 0);
     p.Q = d.Q; p.q_bs = d.q_batch_stride; p.q_rs = d.q_row_stride; p.q_cs = d.q_col_stride;
     p.b = d.b; p.b_bs = d.b_batch_stride;
     p.A = d.A_eq; p.a_bs = d.a_batch_stride; p.a_rs = d.a_row_stride; p.a_cs = d.a_col_stride;
@@ -935,7 +904,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
       CUDA_TRY(cudaEventCreate(&ev1));
       CUDA_TRY(cudaEventRecord(ev0, st));
     }
-    rc = launch_solve(*ctx, p, st, d.precision, &hint);
+    rc = launch_solve(*ctx, p, st, d.precision, hint);
     if (rc) { if (ev0) { cudaEventDestroy(ev0); cudaEventDestroy(ev1); } return rc; }
     if (d.device_seconds) {
       float ms = 0.f;
@@ -1057,9 +1026,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
     if (d.warm_start) {
       if ((rc = h2d(sx, d.x, 8)) || (rc = h2d(smx, d.mu_x, 8)) || (rc = h2d(smc, d.mu_lambda_c, 8))) return rc;
     }
-    fccqp::SolveParams p{};
-    fill_params(d, p);
-    p.B = (int)cnt;
+    fccqp::SolveParams p = solve_params((int)cnt, n, m, nc, d.lambda_c_start, d.options, d.warm_start != 0);
     auto off = [&](const Seg& s) { return s.shared ? dp(s) : dp(s) + lo * s.per_qp; };
     auto offi = [&](const Seg& s) {   // problem data: element size es
       return s.shared ? dp(s) : reinterpret_cast<double*>(reinterpret_cast<char*>(dp(s)) + (size_t)lo * s.per_qp * es);
@@ -1075,7 +1042,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
     p.n_iter = d_niter + lo; p.status = d_status + lo;
     double* res = dp(sres);
     p.res_b = res + lo; p.res_f = res + (size_t)B + lo; p.bviol = res + 2 * (size_t)B + lo; p.fviol = res + 3 * (size_t)B + lo;
-    rc = launch_solve(*ctx, p, st, d.precision, &hint);
+    rc = launch_solve(*ctx, p, st, d.precision, hint);
     if (rc) return rc;
     // D2H: straight into the caller's buffer when it is page-locked (a true asynchronous DMA);
     // otherwise into the pinned bounce buffer, copied out below once the chunk's event has fired

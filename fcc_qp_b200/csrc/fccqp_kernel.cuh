@@ -181,8 +181,7 @@ struct SolveParams {
   const unsigned int* count_dev;  // mode 2: how many (device memory, written by the mode-1 launch)
   int* pending_list;              // mode 1: output list
   unsigned int* pending_count;    // mode 1: its length
-  int full_inverse_at;        // ADMM iteration from which x-updates use the completed inverse of L (default 8)
-  int first_update_identity;  // cold solves: take x-update 0 as the identity it is (see kernel), default 1
+  int full_inverse_at;        // ADMM iteration from which x-updates use the completed inverse of L (launch_solve)
   double rho, eps_fcone, eps_bound;
   double alpha;               // over-relaxation (fccqp_options::relaxation); 1.0 = the reference's iteration
   int adapt_k;                // adaptive rho (fccqp_options::adapt_rho_interval): rebalance every adapt_k iterations; 0 = off
@@ -197,17 +196,13 @@ struct SolveParams {
   int* n_iter; int* status;
   double* res_b; double* res_f; double* bviol; double* fviol;
   unsigned int* work_counter;
-  double* dbg_x0;              // optional [B,n]: pre-solve point (debug / tests)
   unsigned long long* cycles;  // optional [2]: summed factorization / total cycles
   unsigned long long* prof;    // optional [16]: per-phase cycle counters (developer profiling)
-  unsigned long long* trace;   // optional [8][4096]: (clock << 8 | tag) events of CTA 0's first QP (developer tracing)
   Layout lay;                  // filled in by launch_solve
   StructLayout slay;           // structure-exploiting kernel (fccqp_struct.cuh); filled in by launch_solve
   int struct_refine;           // that kernel: one step of iterative refinement on the cold pre-solve
-  int struct_prefetch;         // that kernel: bulk L2 prefetch of the next QP's Q and A_eq
-  int struct_bulk;             // that kernel: bulk-async (TMA) staging of dense Q / A_eq blocks (0: per-row cp.async)
   double* op_scratch;          // that kernel: per-CTA global scratch of the full-space operator of long-running QPs
-  long long op_stride;         //   doubles per CTA (0: the operator stays in the reduced space)
+  long long op_stride;         //   doubles per CTA
 };
 
 __device__ __forceinline__ double warp_max(double v) {
@@ -428,17 +423,8 @@ __device__ __forceinline__ void bar_sync(int odd, int count) {
       t_prof = t_now;                                                      \
     }                                                                      \
   } while (0)
-#define TR(tag)                                                                                      \
-  do {                                                                                               \
-    if (trbuf && lane == 0 && trn < 4096) trbuf[trn++] = ((unsigned long long)clock64() << 8) | (unsigned)(tag); \
-  } while (0)
-#define FCCQP_TRACE_PARAMS , unsigned long long* trbuf, int& trn
-#define FCCQP_TRACE_ARGS , trbuf, trn
 #else
 #define FCCQP_PROF(slot) do { } while (0)
-#define TR(tag) do { } while (0)
-#define FCCQP_TRACE_PARAMS
-#define FCCQP_TRACE_ARGS
 #endif
 
 // One helper step of the left-looking LDL^T for up to T tile rows i_t = i0 + t*stride owned by
@@ -453,10 +439,7 @@ __device__ __forceinline__ void bar_sync(int odd, int count) {
 template <int T>
 __device__ __forceinline__ void helper_step(double* __restrict__ M, const double* __restrict__ dneg, int i0,
                                             int stride, int j, const double2 li, const double2 di,
-                                            int fragC, int fq, const int cnt FCCQP_TRACE_PARAMS) {
-#ifdef FCCQP_DEV
-  const int lane = threadIdx.x & 31;
-#endif
+                                            int fragC, int fq, const int cnt) {
   int rowoff[T];
   double2 l[T], ca[T], cb[T];
 #pragma unroll
@@ -480,7 +463,6 @@ __device__ __forceinline__ void helper_step(double* __restrict__ M, const double
     l[t] = make_double2((wa.x + wb.x) * di.x, (wa.y + wb.y) * di.y);
     if (t < cnt) st2(M + rowoff[t] + 64 * j, l[t]);
   }
-  TR(16);
   // (A), terms k < j from shared memory
   const double* bp = M + tile_off(j + 1, 0) + fragC;
   const double* dp = dneg + 2 * fq;
@@ -502,7 +484,6 @@ __device__ __forceinline__ void helper_step(double* __restrict__ M, const double
       dmma(db.x, db.y, a[0].y, a[0].y * d.y);
     }
   }
-  TR(17);
   // term k = j from registers
   {
     const double2 b = ld2(bp), d = ld2(dp);
@@ -593,7 +574,7 @@ __device__ __forceinline__ double col_dot8(const double* __restrict__ tcol, int 
 // ---------------------------------------------------------------------------
 template <int kThreads>
 __device__ __noinline__ void factor_tiles(double* __restrict__ M, double* __restrict__ dinv, double* __restrict__ dneg,
-                                          const int NB, const int NB32 FCCQP_TRACE_PARAMS) {
+                                          const int NB, const int NB32) {
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   constexpr int kWarps = kThreads / 32;
   constexpr int kHelpers = kWarps - 1;
@@ -611,7 +592,6 @@ __device__ __noinline__ void factor_tiles(double* __restrict__ M, double* __rest
       double* dt = M + tile_off(j, j);
       if (lane == 0) factor_diag_tile(dt, dinv + 8 * j, dneg + 8 * j);
       __syncwarp();
-      TR(12);
       if (j > 0) bar_sync<3>((j - 1) & 1, kThreads);   // helpers finished step j-1
       if (j + 1 < NB) {
         const double2 li = ld2(dt + fragC), di = ld2(dinv + 8 * j + 2 * fq);
@@ -630,14 +610,12 @@ __device__ __noinline__ void factor_tiles(double* __restrict__ M, double* __rest
         st2(lp + 64, make_double2(t1.x + t2.x, t1.y + t2.y));
       }
       bar_arrive<1>(j & 1, kThreads);                     // column j: inv(L_jj), D_j, L_{j+1,j} ready
-      TR(13);
     }
     bar_sync<3>((NB - 1) & 1, kThreads);
   } else {
 #pragma unroll 1
     for (int j = 0; j < NB; ++j) {
       bar_sync<1>(j & 1, kThreads);
-      TR(10);
       const double2 li = ld2(M + tile_off(j, j) + fragC), di = ld2(dinv + 8 * j + 2 * fq);
       // own tile rows i >= j+2, i = warp-1 (mod kHelpers), four at a time
       int i0 = j + 2;
@@ -645,15 +623,13 @@ __device__ __noinline__ void factor_tiles(double* __restrict__ M, double* __rest
 #pragma unroll 1
       for (; i0 < NB; i0 += 4 * kHelpers) {
         const int cnt = (NB - i0 + kHelpers - 1) / kHelpers;
-        if (cnt > 2) helper_step<4>(M, dneg, i0, kHelpers, j, li, di, fragC, fq, cnt FCCQP_TRACE_ARGS);
-        else helper_step<2>(M, dneg, i0, kHelpers, j, li, di, fragC, fq, cnt FCCQP_TRACE_ARGS);
+        if (cnt > 2) helper_step<4>(M, dneg, i0, kHelpers, j, li, di, fragC, fq, cnt);
+        else helper_step<2>(M, dneg, i0, kHelpers, j, li, di, fragC, fq, cnt);
       }
-      TR(11);
       bar_arrive<3>(j & 1, kThreads);
     }
   }
   __syncthreads();
-  TR(15);
   // ---------------- explicit inverses of the 32x32 diagonal blocks of L, in place ----------------
   // level 1: 16x16 = [[X1,0],[-X2 L21 X1, X2]] from the 8x8 inverses left by the factorization
 #pragma unroll 1
@@ -724,7 +700,7 @@ __device__ __noinline__ void factor_tiles(double* __restrict__ M, double* __rest
 // ---------------------------------------------------------------------------
 __device__ __noinline__ double kkt_solve(const double* __restrict__ M, const double* __restrict__ dinv,
                                          double* __restrict__ tbuf, double* __restrict__ ybuf, double acc,
-                                         const int NB, const int NB32, const int N8 FCCQP_TRACE_PARAMS) {
+                                         const int NB, const int NB32, const int N8) {
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const bool is_row = t < N8;
   const int tb = t >> 3, tr = t & 7, tf = tr >> 1;
@@ -748,9 +724,7 @@ __device__ __noinline__ double kkt_solve(const double* __restrict__ M, const dou
       val = is_row ? s : 0.0;
       ybuf[t] = val;
     }
-    TR(31);
     __syncthreads();
-    TR(32);
     if (warp > J && is_row) {
       double s = 0.0;
 #pragma unroll 2
@@ -773,9 +747,7 @@ __device__ __noinline__ double kkt_solve(const double* __restrict__ M, const dou
       val = is_row ? s : 0.0;
       ybuf[t] = val;
     }
-    TR(33);
     __syncthreads();
-    TR(34);
     if (warp < J) {
       double s = 0.0;
 #pragma unroll 2
@@ -1050,12 +1022,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
   unsigned long long* const s_prof = reinterpret_cast<unsigned long long*>(ibuf + 2);  // [16]
   long long t_prof = 0;
   if (p.prof && tid == 0) { for (int i = 0; i < 16; ++i) s_prof[i] = 0; t_prof = clock64(); }
-  // developer tracing: lane 0 of every warp of CTA 0 logs (clock, tag) for the first QP it solves
-  // (the THIRD QP of CTA 0 when it gets that many: instruction caches warm, neighbours out of step)
-  unsigned long long* const trbase = (p.trace && blockIdx.x == 0) ? p.trace + warp * 4096 : nullptr;
-  unsigned long long* trbuf = nullptr;
-  int trn = 0, trcount = 0;
-  const int trsel = (p.B >= 3 * (int)gridDim.x) ? 2 : 0;
 #endif
 
   int parity = 0;
@@ -1095,10 +1061,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
     const int qslot = *s_work;
     if (qslot >= Btot) break;
     const int qp = p.index_list ? p.index_list[qslot] : qslot;
-#ifdef FCCQP_DEV
-    trbuf = (trcount++ == trsel) ? trbase : nullptr;
-#endif
-    TR(1);
 
     const double* Qg = p.Q + (size_t)qp * p.q_bs;
     const double* Ag = p.A + (size_t)qp * p.a_bs;
@@ -1141,7 +1103,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
     int n_iter = 0;
     double res_x = 0.0, res_c = 0.0;
     FCCQP_PROF(0);
-    TR(2);
 
     // pass 0: cold pre-solve on [[Q + sigma A'A, A'],[A,0]];  pass 1: ADMM on [[Q + rho I, A'],[A,0]].
     // A KKT matrix is assembled and factored lazily, right before the first solve that needs it.
@@ -1151,7 +1112,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
     // whose minimiser is x0 itself (x0 minimises the first two terms on the same set).  The kernel
     // takes that x-update as the identity: a QP whose pre-solve point already passes the exit test
     // (98 % of the walking log) finishes without the second factorization; the others factor and
-    // carry on from iteration 1.  first_update_identity = 0 runs the solve instead.
+    // carry on from iteration 1.
     bool defer = false;   // shared_mode 1: this QP needs ADMM iterations, hand it to the second launch
     for (int pass = (presolve && !resume) ? 0 : 1; pass < 2 && !defer; ++pass) {
       if (pass == 1 && eqc) break;
@@ -1172,7 +1133,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
 #pragma unroll 1
       for (int iter = 0; iter < iters; ++iter) {
       double val = v_x;    // solution component of row t (t < N8)
-      if (!(pass == 1 && iter == 0 && presolve && p.first_update_identity)) {
+      if (!(pass == 1 && iter == 0 && presolve)) {
       while (!factored) {   // (a second trip only for a rank-deficient A_eq, see reg_delta below)
       factored = true;
       const long long t_f0 = clock64();
@@ -1315,11 +1276,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
           }
         }
       }
-      TR(3);
       cp_async_wait_all();
       __syncthreads();
       FCCQP_PROF(1);
-      TR(4);
 
       // retry after a failed factorization: -delta on the (so far zero) diagonal entry of the dependent constraint rows
       if (reg_mine) M[mat_off(t, t)] = -reg_delta;
@@ -1342,7 +1301,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
           fro = (fro + f1) + (f2 + f3);
         }
         block_reduce2<true>(trq, fro, red, parity);
-        TR(6);
         const double sigma = (trq > 0.0 && fro > 0.0 && isfinite(trq / fro)) ? trq / fro : 1.0;
         sigma_cached = sigma;
         // rhs_x = -b + sigma A' b_eq (needs A before the factorization overwrites it)
@@ -1354,7 +1312,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
         } else if (is_c) {
           rhs0 = v_b;
         }
-        TR(7);
         // H += sigma A'A on the tiles of the variable block, in place: chunks of up to four tiles of
         // one tile row (shared A operand, 2 x cnt independent DMMA chains), round-robin over the warps
         {
@@ -1375,9 +1332,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
       }
       __syncthreads();
       FCCQP_PROF(2);
-      TR(5);
 
-      factor_tiles<kThreads>(M, dinv, dneg, NB, NB32 FCCQP_TRACE_ARGS);
+      factor_tiles<kThreads>(M, dinv, dneg, NB, NB32);
       FCCQP_PROF(3);
       fact_cycles += (unsigned long long)(clock64() - t_f0);
       {
@@ -1428,7 +1384,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
         cached_pass = pass;
       }
       FCCQP_PROF(6);
-      TR(20);
       }
       }  // lazy factorization
       if (factor_flag) status_flag = 2;
@@ -1445,7 +1400,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
         } else if (is_c) {
           acc = v_b;
         }
-        TR(30);
         if (shared_mode != 0) {
           const double gx = g_apply(M, tbuf, is_row ? acc : 0.0, NB, n8);   // x = [K^{-1}]_{x,:} rhs, cached operator
           val = is_x ? gx : 0.0;
@@ -1466,11 +1420,10 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
           const double gw = g_apply(M, tbuf, w, NBx, n8);
           val = is_x ? fma(rho_cur, gw, v_xbase) : 0.0;
         } else {
-          val = kkt_solve(M, dinv, tbuf, ybuf, acc, NB, NB32, N8 FCCQP_TRACE_ARGS);
+          val = kkt_solve(M, dinv, tbuf, ybuf, acc, NB, NB32, N8);
         }
         }
         FCCQP_PROF(7);
-        TR(35);
         // val = solution component of row t (t < N8)
 
         }  // x-update solve
@@ -1478,10 +1431,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
         if (pass == 0) {
           v_x = val;
           if (t < n8) xs[t] = is_x ? val : 0.0;
-          if (p.dbg_x0 && is_x) p.dbg_x0[(size_t)qp * n + t] = val;
           __syncthreads();
           FCCQP_PROF(8);
-          TR(41);
           continue;
         }
 
@@ -1523,7 +1474,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
         // themselves are only needed for the iteration that ends the loop
         const int conv = __syncthreads_and((rc < p.eps_fcone) && (rx < p.eps_bound));
         FCCQP_PROF(9);
-        TR(51);
 #ifdef FCCQP_DEV
         if (p.prof && tid == 0) s_prof[15] += 1;
 #endif
@@ -1566,7 +1516,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
       continue;
     }
     // ---------------- K6: epilogue ----------------
-    TR(60);
     __syncthreads();
     double bv = 0.0, fv = 0.0;
     int bad = 0;
@@ -1611,7 +1560,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
       }
     }
     FCCQP_PROF(10);
-    TR(61);
 #ifdef FCCQP_DEV
     if (p.prof && tid == 0) s_prof[14] += 1;
 #endif
@@ -1621,9 +1569,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
     for (int i = 0; i < 16; ++i) atomicAdd(p.prof + i, s_prof[i]);
 #endif
 #undef FCCQP_PROF
-#undef TR
-#undef FCCQP_TRACE_PARAMS
-#undef FCCQP_TRACE_ARGS
 }
 
 // ---------------------------------------------------------------------------

@@ -40,7 +40,7 @@
 // the compiled reference on the walking log (tools/proto/struct_full_check.py, the numpy model of
 // this kernel) the unpivoted reduced solve alone is within 2e-7 relative with identical iteration
 // counts on all 2019 QPs, and ONE step of iterative refinement of the cold pre-solve against the
-// ORIGINAL Q and A_eq (SolveParams::struct_refine, default on) brings it back to 7e-11 -- the level of
+// ORIGINAL Q and A_eq (SolveParams::struct_refine, on when the caller asks for it) brings it back to 7e-11 -- the level of
 // the general kernel.  The ADMM pass needs none (h_j >= rho).
 #pragma once
 #include "fccqp_kernel.cuh"
@@ -427,14 +427,8 @@ __device__ __forceinline__ double struct_xsolve(const SolveParams& p, const Stru
   } else if (row_0) acc = rf[I.d0list[zrow]];
   XPROF(6);
   double val;
-#ifdef FCCQP_DEV
-  unsigned long long* trbuf = nullptr; int trn = 0;
-  if (use_op) val = g_apply(M, tbuf, acc, S.NB, S.N8);
-  else val = kkt_solve(M, dinv, tbuf, ybuf, acc, S.NB, S.NB32, S.N8, trbuf, trn);
-#else
   if (use_op) val = g_apply(M, tbuf, acc, S.NB, S.N8);
   else val = kkt_solve(M, dinv, tbuf, ybuf, acc, S.NB, S.NB32, S.N8);
-#endif
   XPROF(7);
   if (t < S.N8) sred[t] = val;
   __syncthreads();
@@ -611,11 +605,7 @@ __device__ __forceinline__ double struct_xsolve(const SolveParams& p, const Stru
       else if (row_y) acc2 = d1c[yrow];
       else if (row_0) acc2 = rf[I.d0list[zrow]];
     }
-#ifdef FCCQP_DEV
-    const double dv = kkt_solve(M, dinv, tbuf, ybuf, acc2, S.NB, S.NB32, S.N8, trbuf, trn);
-#else
     const double dv = kkt_solve(M, dinv, tbuf, ybuf, acc2, S.NB, S.NB32, S.N8);
-#endif
     if (t < S.N8) sred[t] = val + dv;
     __syncthreads();
     XPROF(10);
@@ -1037,12 +1027,12 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
     StructQP S;
     const bool q_vec = q_fast == 1 && (n & 1) == 0 && (q_slow & 1) == 0 && (reinterpret_cast<uintptr_t>(Qg) & 15) == 0;
     const bool a_vec = p.a_cs == 1 && (n & 1) == 0 && (p.a_rs & 1) == 0 && (reinterpret_cast<uintptr_t>(Ag) & 15) == 0;
-    sc.q_bulk = q_vec && q_slow == n && p.struct_bulk;
-    sc.a_bulk = a_vec && p.a_rs == n && p.struct_bulk;
+    sc.q_bulk = q_vec && q_slow == n;
+    sc.a_bulk = a_vec && p.a_rs == n;
     bool defer = struct_classify<kThreads>(n, m, n8, m8, Qg, q_slow, q_fast, q_vec, Ag, p.a_rs, p.a_cs, a_vec, M, L.stage_cap, sc,
                                            qd_s, rf, I, L.nr8c, L.ndp8c, L.nd08c, vc, S.nr, S.ndp, S.nd0) != 0;
     SPROF(1);
-    if (tid == 0 && w_next < p.B && p.struct_prefetch) {
+    if (tid == 0 && w_next < p.B) {
       // the next QP of this CTA: start pulling its Q and A_eq into L2 (one bulk-async instruction each); by the
       // time the CTA gets to it, its stage-in reads are L2 hits
       if (q_dense) l2_prefetch(p.Q + (size_t)w_next * p.q_bs, (size_t)n * n * sizeof(double));
@@ -1092,7 +1082,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
 #pragma unroll 1
       for (int iter = 0; iter < iters; ++iter) {
         double val = v_x;
-        if (!(pass == 1 && iter == 0 && presolve && p.first_update_identity)) {
+        if (!(pass == 1 && iter == 0 && presolve)) {
           if (!factored) {
             factored = true;
             const long long t_f0 = clock64();
@@ -1210,11 +1200,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
             if (yrow >= m && yrow < m8) M[mat_off(t, t)] = 1.0;
             __syncthreads();
             SPROF(4);
-#ifdef FCCQP_DEV
-            { unsigned long long* trbuf = nullptr; int trn = 0; factor_tiles<kThreads>(M, dinv, dneg, Se.NB, Se.NB32, trbuf, trn); }
-#else
             factor_tiles<kThreads>(M, dinv, dneg, Se.NB, Se.NB32);
-#endif
             SPROF(5);
             fact_cycles += (unsigned long long)(clock64() - t_f0);
             // inertia (+ on R and D0 rows and all pads, - on the constraint rows): anything else goes to the general kernel
@@ -1265,7 +1251,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
               SPROF(15);
               full_inverse = true;
               // full-space operator (build_full_op) when it fits: rows of F <= threads and vector buffers, tiles of F
-              // within the [M | AP] region (AP is not needed afterwards)
+              // within the [M | AP] region (AP is not needed afterwards).  launch_struct always allocates the operator
+              // scratch, so op_stride > 0 holds; the test stays because without it CUDA 12.9 spills more in the
+              // <64, 8, true> instance.
               if (p.op_stride > 0) {
                 FullOpDims fd;
                 fd.NBr = NBr; fd.mt = mt; fd.dptc = dptc; fd.dpt = Se.dpt;
@@ -1277,7 +1265,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
                   if (lane == 0) I.wtot[warp] = __popc(b1);
                   __syncthreads();
                   int o1 = 0;
-#pragma unroll
+  #pragma unroll
                   for (int w2 = 0; w2 < kWarps; ++w2) if (w2 < warp) o1 += I.wtot[w2];
                   int epos = -1;
                   if (is_x && ve.type == VT_DP) epos = ve.pos;
@@ -1305,7 +1293,6 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
         if (pass == 0) {
           v_x = val;
           if (t < n8) xs[t] = is_x ? val : 0.0;
-          if (p.dbg_x0 && is_x) p.dbg_x0[(size_t)qp * n + t] = val;
           __syncthreads();
           continue;
         }

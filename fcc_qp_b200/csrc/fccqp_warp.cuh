@@ -179,7 +179,7 @@ __global__ void __launch_bounds__(32 * kWarps, kMinBlocks) fccqp_warp_kernel(con
         T val = v_x;
         // x-update 0 of a cold solve is the identity (x_bar = x0, zero duals; fccqp_kernel.cuh): the rho-KKT system is
         // only factored for QPs that go on iterating
-        if (!(pass == 1 && iter == 0 && presolve && p.first_update_identity)) {
+        if (!(pass == 1 && iter == 0 && presolve)) {
           while (!factored) {
             factored = true;
             const long long t_f0 = clock64();
@@ -292,7 +292,6 @@ __global__ void __launch_bounds__(32 * kWarps, kMinBlocks) fccqp_warp_kernel(con
 
         if (pass == 0) {
           v_x = val;
-          if (p.dbg_x0 && is_x) p.dbg_x0[(size_t)qp * n + lane] = (double)val;
           continue;
         }
 

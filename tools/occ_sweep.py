@@ -22,5 +22,5 @@ print(f"{shape} {structure} ctas/SM={li['ctas_per_sm']} threads={li['block']}: {
 '''
 for shape, structure in (("log", "auto"), ("log", "dense"), ("quadruped", "auto")):
     for c in (1, 2, 3, 4, 5, 6, 8):
-        env = dict(os.environ, FCCQP_CTAS_PER_SM=str(c), FCCQP_STRUCT_REFINE=os.environ.get("FCCQP_STRUCT_REFINE", "0"))
+        env = dict(os.environ, FCCQP_CTAS_PER_SM=str(c))
         subprocess.run([sys.executable, "-c", code, ROOT, B, shape, structure], env=env)

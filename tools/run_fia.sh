@@ -1,4 +1,4 @@
-# sweep of the iteration at which long-running QPs switch to the explicit operator (FCCQP_FULL_INVERSE_AT, default 8)
+# sweep of the iteration at which long-running QPs switch to the explicit operator (FCCQP_FULL_INVERSE_AT; default 6, 8 for n + m <= 32)
 for v in 4 6 8; do
   export FCCQP_FULL_INVERSE_AT=$v
   echo "== full_inverse_at $v"

@@ -16,10 +16,11 @@ def rel(z, zr):
     return np.abs(z - zr).max(1) / np.maximum(1.0, np.abs(zr).max(1))
 
 
-def run(qp, structure, warm_state=None):
+def run(qp, structure, refine=False):
     s = FCCQPBatch(qp.n, qp.m, qp.nc, qp.lambda_c_start)
     s.set_options(OPTS)
     s.structure = structure
+    s.refine = refine
     args = [torch.as_tensor(a, device=dev) for a in (qp.Q, qp.b, qp.A_eq, qp.b_eq, qp.friction_coeffs, qp.lb, qp.ub)]
     s.Solve(*args)
     torch.cuda.synchronize()
@@ -29,17 +30,15 @@ def run(qp, structure, warm_state=None):
 
 
 def case(name, qp, gold):
-    for refine in ("1", "0"):
-        os.environ["FCCQP_STRUCT_REFINE"] = refine
-        z, it, st, info, dt = run(qp, "probe")
+    for refine in (True, False):
+        z, it, st, info, dt = run(qp, "probe", refine)
         e = rel(z, gold["z"])
         mis = int((it != gold["n_iter"]).sum())
-        print(f"{name} struct refine={refine}: info={info} max_rel={e.max():.3e} p50={np.median(e):.3e} "
+        print(f"{name} struct refine={int(refine)}: info={info} max_rel={e.max():.3e} p50={np.median(e):.3e} "
               f"n_iter mismatches={mis}/{len(it)} status2={(st == 2).sum()} nan={np.isnan(z).any()}", flush=True)
         if mis:
             idx = np.nonzero(it != gold["n_iter"])[0][:8]
             print("   first mismatches", [(int(i), int(it[i]), int(gold["n_iter"][i])) for i in idx])
-    os.environ.pop("FCCQP_STRUCT_REFINE", None)
     z, it, st, info, dt = run(qp, "dense")
     e = rel(z, gold["z"])
     print(f"{name} dense: info={info} max_rel={e.max():.3e} mismatches={(it != gold['n_iter']).sum()}", flush=True)
@@ -56,13 +55,12 @@ for name, qp in (("log", log.tile(Bt)), ("humanoid", synthetic.make_batch(synthe
                  ("quadruped", synthetic.make_batch(synthetic.QUADRUPED, Bt)),
                  ("multicontact", synthetic.make_batch(synthetic.MULTICONTACT, Bt // 4))):
     args = [torch.as_tensor(a, device=dev) for a in (qp.Q, qp.b, qp.A_eq, qp.b_eq, qp.friction_coeffs, qp.lb, qp.ub)]
-    for structure, refine in (("auto", "1"), ("auto", "0"), ("dense", "1")):
-        os.environ["FCCQP_STRUCT_REFINE"] = refine
-        s = FCCQPBatch(qp.n, qp.m, qp.nc, qp.lambda_c_start); s.set_options(OPTS); s.structure = structure
+    for structure, refine in (("auto", True), ("auto", False), ("dense", True)):
+        s = FCCQPBatch(qp.n, qp.m, qp.nc, qp.lambda_c_start); s.set_options(OPTS); s.structure = structure; s.refine = refine
         ts = []
         for r in range(4):
             s.Solve(*args); torch.cuda.synchronize()
             ts.append(s.GetSolution().details.device_time)
         t = min(ts[1:])
-        print(f"time {name} B={qp.batch} {structure} refine={refine}: {t*1e3:.3f} ms -> {qp.batch/t/1e6:.3f} M QP/s "
+        print(f"time {name} B={qp.batch} {structure} refine={int(refine)}: {t*1e3:.3f} ms -> {qp.batch/t/1e6:.3f} M QP/s "
               f"launch={nat.last_launch_info()} struct={nat.last_struct_info()}", flush=True)
