@@ -186,6 +186,12 @@ template <int kThreads, int kMinBlocks>
 KernelFn struct_instance(bool adapt) {
   return adapt ? fccqp::fccqp_struct_kernel<kThreads, kMinBlocks, true> : fccqp::fccqp_struct_kernel<kThreads, kMinBlocks, false>;
 }
+template <int kThreads, int kMinBlocks>
+KernelFn struct_first_instance(bool refine) {
+  using fccqp::fccqp_struct_kernel;
+  return refine ? fccqp_struct_kernel<kThreads, kMinBlocks, false, fccqp::kStructFirstRefine>
+                : fccqp_struct_kernel<kThreads, kMinBlocks, false, fccqp::kStructFirst>;
+}
 
 // Host-side twin of fccqp::struct_classify for callers whose data is in host memory (no probe launch,
 // no stream sync): counts of one QP.  Returns false for a structurally singular QP.
@@ -246,11 +252,14 @@ struct Scratch {
   static constexpr size_t kListCount = 2;  // length of the hand-over list
   static constexpr size_t kProbe = 4;      // [4, 8): structure probe (atomicMax)
   static constexpr size_t kLpt = 8;        // [8, 10): counters of lpt_order_kernel
-  static constexpr size_t kHeader = 16;    // then [B] the hand-over list, then [B] the LPT order
+  static constexpr size_t kWork3 = 10;     // work counter of the resume launch of a two-stage structure solve
+  static constexpr size_t kResumeCount = 11;  // length of its list
+  static constexpr size_t kHeader = 16;    // then [B] the hand-over list, [B] the resume list, [B] the LPT order
   unsigned int* w = nullptr;
   size_t B = 0;
   int* list() const { return reinterpret_cast<int*>(w + kHeader); }
-  int* order() const { return reinterpret_cast<int*>(w + kHeader + B); }
+  int* resume_list() const { return reinterpret_cast<int*>(w + kHeader + B); }
+  int* order() const { return reinterpret_cast<int*>(w + kHeader + 2 * B); }
 };
 
 // Allocates the scratch of a call.  FCCQP_SCHEDULE_LPT, when the batch holds at least two QPs for each of the `slots`
@@ -258,7 +267,7 @@ struct Scratch {
 int begin_call(fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long long slots, Scratch* s) {
   const bool lpt = lpt_hint && p.n_iter != nullptr && p.B >= 2 * slots;
   s->B = (size_t)p.B;
-  CUDA_TRY(cudaMallocAsync(&s->w, (Scratch::kHeader + (lpt ? 2 : 1) * s->B) * sizeof(unsigned int), stream));
+  CUDA_TRY(cudaMallocAsync(&s->w, (Scratch::kHeader + (lpt ? 3 : 2) * s->B) * sizeof(unsigned int), stream));
   CUDA_TRY(cudaMemsetAsync(s->w, 0, Scratch::kHeader * sizeof(unsigned int), stream));
   p.work_counter = s->w + Scratch::kWork;
   if (lpt) {
@@ -377,7 +386,9 @@ constexpr int kNotApplicable = 1;
 
 // Structure-exploiting kernel (fccqp_struct.cuh): QPs whose separable variables can be eliminated analytically run on
 // a reduced KKT system; the others (if any) are appended to a device-side list that the general kernel (geometry gli)
-// takes in a second launch.  Returns kNotApplicable, with nothing launched but the probe, when the reduction does not pay.
+// takes in a last launch.  Large cold batches run the structure-exploiting solve in two stages (kStructFirst, then
+// the full kernel over the QPs the first stage listed).  Returns kNotApplicable, with nothing launched but the probe, when the
+// reduction does not pay.
 int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stream, const Scratch& s, const StructHint& hint,
                   KernelFn general, const LaunchInfo& gli) {
   int caps[3] = {hint.caps[0], hint.caps[1], hint.caps[2]};
@@ -405,20 +416,47 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   if (sl.N8c + 8 > p.lay.N8 || sl.bytes() > (size_t)ctx.max_smem_optin) return kNotApplicable;
   // threads >= max(n, padded reduced KKT size), at most 256 since the reduced size is below p.lay.N8
   const int need = p.n > sl.N8c ? p.n : sl.N8c;
-  const bool adapt = p.adapt_k > 0;
-  KernelFn fn;
+  const bool adapt = p.adapt_k > 0, refine = p.struct_refine != 0;
   int threads;
-  if (need <= 64) { threads = 64; fn = struct_instance<64, 8>(adapt); }
-  else if (need <= 96) { threads = 96; fn = struct_instance<96, 5>(adapt); }
-  else if (need <= 128) { threads = 128; fn = struct_instance<128, 4>(adapt); }
-  else { threads = 256; fn = struct_instance<256, 2>(adapt); }
-  LaunchInfo li;
-  int rc = geometry(ctx, fn, threads, sl.bytes(), p.B, 1, &li);
+  KernelFn first;
+  if (need <= 64) { threads = 64; first = struct_first_instance<64, 8>(refine); }
+  else if (need <= 96) { threads = 96; first = struct_first_instance<96, 5>(refine); }
+  else if (need <= 128) { threads = 128; first = struct_first_instance<128, 4>(refine); }
+  else { threads = 256; first = struct_first_instance<256, 2>(refine); }
+  LaunchInfo li, fli;
+  int rc = geometry(ctx, first, threads, sl.bytes(), p.B, 1, &fli);
   if (rc) return rc;
+  // Cold batches of at least 8 QPs per resident CTA run in two stages: the first-stage kernel takes every QP through the
+  // exit test of iteration 0 (where nearly all whole-body-control QPs stop) and lists the others, which the full kernel
+  // resumes from there.  Smaller batches and warm solves keep the single launch.
+  const bool split = !p.warm && p.B >= 8LL * fli.ctas_per_sm * ctx.num_sms;
+  KernelFn fn;
+  if (threads == 64) fn = struct_instance<64, 8>(adapt);
+  else if (threads == 96) fn = struct_instance<96, 5>(adapt);
+  else if (threads == 128) fn = struct_instance<128, 4>(adapt);
+  else fn = struct_instance<256, 2>(adapt);
+  if ((rc = geometry(ctx, fn, threads, sl.bytes(), p.B, 1, &li))) return rc;
   fccqp::SolveParams a = p;
   a.slay = sl;
   a.pending_count = s.w + Scratch::kListCount;
   a.pending_list = s.list();
+  if (split) {
+    fccqp::SolveParams f = a;
+    f.resume_list = s.resume_list();
+    f.resume_count = s.w + Scratch::kResumeCount;
+#ifdef FCCQP_DEV
+    PhaseProfile prof;
+    if ((rc = prof.start(stream, &f))) return rc;
+#endif
+    first<<<fli.grid, fli.block, fli.smem, stream>>>(f);
+    CUDA_TRY(cudaGetLastError());
+#ifdef FCCQP_DEV
+    if ((rc = prof.report(stream, "struct first stage", kStructPhases, p.B, fli.grid))) return rc;
+#endif
+    a.count_dev = f.resume_count;
+    a.index_list = f.resume_list;
+    a.work_counter = s.w + Scratch::kWork3;
+  }
   // per-CTA global scratch of the full-space operator of long-running QPs (build_full_op): B, Z, X, Y tiles and 1/h
   // sized for every variable eliminated
   const long long neT = sl.n8 >> 3, NBr = sl.nr8c >> 3, mt = sl.mt;
@@ -432,7 +470,7 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   CUDA_TRY(cudaGetLastError());
   CUDA_TRY(cudaFreeAsync(a.op_scratch, stream));
 #ifdef FCCQP_DEV
-  if ((rc = prof.report(stream, "struct", kStructPhases, p.B, li.grid))) return rc;
+  if ((rc = prof.report(stream, split ? "struct resume" : "struct", kStructPhases, p.B, li.grid))) return rc;
 #endif
   fccqp::SolveParams b = p;
   b.count_dev = a.pending_count;
@@ -443,7 +481,7 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, a.pending_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, stream));
   StructInfo si;
   si.used = 1; si.nr = caps[0]; si.ndp = caps[1]; si.nd0 = caps[2]; si.rows = sl.N8c; si.rows_dense = p.lay.N8; si.device = ctx.device;
-  return end_call(s, stream, 2, li, si);
+  return end_call(s, stream, split ? 3 : 2, split ? fli : li, si);
 }
 
 int launch_general(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s, KernelFn fn, const LaunchInfo& li) {

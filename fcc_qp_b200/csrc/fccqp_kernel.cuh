@@ -203,6 +203,8 @@ struct SolveParams {
   int struct_refine;           // that kernel: one step of iterative refinement on the cold pre-solve
   double* op_scratch;          // that kernel: per-CTA global scratch of the full-space operator of long-running QPs
   long long op_stride;         //   doubles per CTA
+  int* resume_list;            // its first stage (kStructFirst): QPs that keep iterating
+  unsigned int* resume_count;  //   their count
 };
 
 __device__ __forceinline__ double warp_max(double v) {

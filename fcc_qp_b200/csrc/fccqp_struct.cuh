@@ -926,9 +926,25 @@ __device__ __noinline__ int full_op_loop(const OpLoopArgs& a, OpLoopThread& th, 
 #define SPROF(slot) do { } while (0)
 #endif
 
+// Which part of a solve an instance of fccqp_struct_kernel runs.  Cold batches large enough to fill the GPU twice over
+// run in two stages (launch_struct): nearly every QP of a whole-body-control batch passes the exit test at iteration 0,
+// so the first stage stops there and carries none of the code of the QPs that keep iterating (rho-KKT factorization,
+// explicit inverse, full-space operator, adaptive rho); the full kernel then resumes the others.
+//   kStructFull          the whole solve; with p.count_dev set (the resume launch) the QPs of that list, each from ADMM
+//                        iteration 0 at the pre-solve point the first stage left in p.x (mu_x = mu_c = 0, as in any cold
+//                        solve): iteration 0 is redone from the same values.  (One instance for both: a separately
+//                        compiled resume instance rounds differently -- the resumed QPs would no longer be bit-identical
+//                        to a single launch.)
+//   kStructFirst(Refine) cold solves through the exit test of iteration 0, without (with) the refinement step of the
+//                        pre-solve; a QP that needs more iterations leaves its pre-solve point in p.x and its index on
+//                        p.resume_list
+enum : int { kStructFull = 0, kStructFirst = 1, kStructFirstRefine = 2 };
+
 // kAdapt: the adaptive-rho extension compiled in (a separate instance: the default path carries none of it)
-template <int kThreads, int kMinBlocks, bool kAdapt>
+template <int kThreads, int kMinBlocks, bool kAdapt, int kStage = kStructFull>
 __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(const SolveParams p) {
+  constexpr bool kFirst = kStage != kStructFull;
+  static_assert(!(kFirst && kAdapt), "the first stage stops before adaptive rho can act");
   extern __shared__ __align__(16) double smem[];
   const StructLayout& L = p.slay;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -980,10 +996,12 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
 
   // Work indices are fetched one QP ahead (thread 0 keeps the next one in a register): the atomic's round trip
   // hides behind the QP in flight, and the index is known early enough to pull that QP's data into L2.
-  // (p.index_list: a processing order -- FCCQP_SCHEDULE_LPT -- the queue slot is mapped through it, one QP ahead as well)
+  // (p.index_list: a processing order -- FCCQP_SCHEDULE_LPT, or the p.count_dev QPs the first stage left -- the queue
+  // slot is mapped through it, one QP ahead as well; p.B: the queue is drained)
   int w_next = 0;
   if (tid == 0) {
     w_next = (int)atomicAdd(p.work_counter, 1u);
+    if (!kFirst && p.count_dev && w_next >= (int)*p.count_dev) w_next = p.B;
     if (p.index_list && w_next < p.B) w_next = p.index_list[w_next];
   }
   for (;;) {
@@ -992,12 +1010,14 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
       s_work[0] = w_next;
       if (w_next < p.B) {
         w_next = (int)atomicAdd(p.work_counter, 1u);
+        if (!kFirst && p.count_dev && w_next >= (int)*p.count_dev) w_next = p.B;
         if (p.index_list && w_next < p.B) w_next = p.index_list[w_next];
       }
     }
     __syncthreads();
     const int qp = s_work[0];
     if (qp >= p.B) break;
+    const bool resume = !kFirst && p.count_dev != nullptr;
     const double* Qg = p.Q + (size_t)qp * p.q_bs;
     const double* Ag = p.A + (size_t)qp * p.a_bs;
     SPROF(0);
@@ -1009,7 +1029,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
       v_b = p.b[(size_t)qp * p.b_bs + t];
       v_lb = p.lb[(size_t)qp * p.lb_bs + t];
       v_ub = p.ub[(size_t)qp * p.ub_bs + t];
-      if (p.warm) { v_x = p.x[(size_t)qp * n + t]; v_mux = p.mu_x[(size_t)qp * n + t]; }
+      if (p.warm || resume) v_x = p.x[(size_t)qp * n + t];
+      if (p.warm) v_mux = p.mu_x[(size_t)qp * n + t];
     }
     if (t < m) beqs[t] = p.beq[(size_t)qp * p.beq_bs + t];
     if (t < nc / 3) vmu[t] = p.mu[(size_t)qp * p.mu_bs + t];
@@ -1048,7 +1069,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
 
     // pass 0: cold pre-solve (shift 0);  pass 1: ADMM (shift rho).  Same lazy scheme as the general kernel:
     // x-update 0 of a cold solve is the identity, the rho-KKT system is only factored for QPs that iterate.
-    for (int pass = presolve ? 0 : 1; pass < 2 && !defer; ++pass) {
+    bool survive = false;   // first stage: iteration 0 did not end the solve
+    for (int pass = (presolve && !resume) ? 0 : 1; pass < 2 && !defer; ++pass) {
       if (pass == 1 && eqc) break;
       if (pass == 1) {
         v_xbar = v_x;                             // fcc_qp.cpp:74-75
@@ -1082,7 +1104,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
 #pragma unroll 1
       for (int iter = 0; iter < iters; ++iter) {
         double val = v_x;
-        if (!(pass == 1 && iter == 0 && presolve)) {
+        // (the first stage stops at iteration 0 of pass 1, whose x-update is the identity: it solves in pass 0 only)
+        if (kFirst ? pass == 0 : !(pass == 1 && iter == 0 && presolve)) {
           if (!factored) {
             factored = true;
             const long long t_f0 = clock64();
@@ -1223,25 +1246,28 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
           // Long-running QP (iteration full_inverse_at): first x_base = the solve for w = 0 through the factors
           // (rep 0), then the explicit inverse of the reduced matrix; every later x-update is
           // x_base + (one symmetric product with the rho w part).  One call site: the solve is inlined once.
-          const bool make_op = pass == 1 && !full_inverse && iter >= p.full_inverse_at;
+          const bool make_op = !kFirst && pass == 1 && !full_inverse && iter >= p.full_inverse_at;
+          const bool refine = kFirst ? kStage == kStructFirstRefine : (pass == 0 && p.struct_refine != 0);
 #pragma unroll 1
           for (int rep = make_op ? 0 : 1; rep < 2; ++rep) {
             const bool base_solve = rep == 0;
-            if (!base_solve && full_op) {
+            if (!kFirst && !base_solve && full_op) {
               val = full_op_apply(M, smem + L.off_tbuf, smem + L.off_ybuf, smem + L.off_sred, ci, shift * w, NBF, NF);
               break;
             }
-            const bool op = !base_solve && full_inverse;
+            const bool op = !kFirst && !base_solve && full_inverse;
             double r = 0.0;
             if (is_x) r = (base_solve || pass == 0) ? -v_b : (op ? shift * w : -(v_b - shift * w));
 #ifdef FCCQP_DEV
             const double res = struct_xsolve<kThreads>(p, L, smem, I, Se, ve, Qg, Ag, q_slow, q_fast, r, hi, shift, op, op,
-                                                       pass == 0 && p.struct_refine != 0, q_vec && a_vec, s_prof, t_prof);
+                                                       refine, q_vec && a_vec, s_prof, t_prof);
 #else
             const double res = struct_xsolve<kThreads>(p, L, smem, I, Se, ve, Qg, Ag, q_slow, q_fast, r, hi, shift, op, op,
-                                                       pass == 0 && p.struct_refine != 0, q_vec && a_vec);
+                                                       refine, q_vec && a_vec);
 #endif
-            if (base_solve) {
+            if constexpr (kFirst) {
+              val = res;
+            } else if (base_solve) {
               v_xbase = res;
               __syncthreads();
               SPROF(12);
@@ -1334,6 +1360,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
           block_reduce2<false>(rx, rc, red, parity);
           res_x = rx; res_c = rc;
           if (conv) { n_iter = iter; SPROF(8); break; }
+        } else if (kFirst) {
+          survive = true;
+          break;
         } else if (!kAdapt && kThreads > 64 && full_op) {
           // every further iteration of this QP in the compact operator loop (full_op_loop).  Not in the two-warp instance:
           // a barrier between two warps costs little, and the call cost that instance 3.5 % on the quadruped shape
@@ -1383,6 +1412,12 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
     if (defer) {
       // not reducible within the caps / wrong inertia: the general kernel takes this QP (device-side list)
       if (tid == 0) p.pending_list[atomicAdd(p.pending_count, 1u)] = qp;
+      continue;
+    }
+    if (kFirst && survive) {
+      // the full kernel resumes this QP at iteration 0 from its pre-solve point
+      if (is_x) p.x[(size_t)qp * n + t] = v_x;
+      if (tid == 0) p.resume_list[atomicAdd(p.resume_count, 1u)] = qp;
       continue;
     }
     // ---------------- K6: epilogue ----------------
