@@ -170,7 +170,8 @@ int check_shape(const DeviceCtx& ctx, int n, int m, int nc) {
 }
 
 // CTA-per-QP kernel instances (fccqp_kernel.cuh): 4 CTAs/SM for the <= 128-row shapes (Cassie, quadruped), 2 above.
-// Shared-structure batches have no adaptive-rho instance: they run with a fixed rho.
+// The shared-structure instance has no adaptive-rho variant: launch_solve sends stride-0 batches with adaptive rho to the
+// other kernels.
 template <int kThreads, int kMinBlocks>
 KernelFn solve_instance(bool shared, bool f32, bool adapt) {
   using fccqp::fccqp_solve_kernel;
@@ -522,8 +523,11 @@ int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int 
   if ((rc = geometry(ctx, general, threads, p.lay.bytes(), p.B, 1, &li)) ||
       (rc = begin_call(p, stream, hint.lpt, (long long)li.ctas_per_sm * ctx.num_sms, &s)))
     return rc;
-  // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs
-  if (!sw.no_shared && !f32 && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) && p.B >= 4 * li.ctas_per_sm * ctx.num_sms)
+  // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs.  Not with
+  // adaptive rho: a lane that moves its rho needs its own rho-KKT factorization, so those batches take the
+  // structure-exploiting or general kernel (both read Q and A_eq through the batch stride).
+  if (!sw.no_shared && !f32 && p.adapt_k == 0 && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) &&
+      p.B >= 4 * li.ctas_per_sm * ctx.num_sms)
     return launch_shared(ctx, p, stream, s);
   if (!f32 && hint.mode != FCCQP_STRUCTURE_DENSE && p.m > 0 &&
       (rc = launch_struct(ctx, p, stream, s, hint, general, li)) != kNotApplicable)

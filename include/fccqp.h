@@ -72,7 +72,8 @@ typedef struct fccqp_options {
    * (at most 10x per update, kept inside [1e-9, 1e9]), the scaled duals are rescaled so that y = rho mu stays put, and the
    * rho-KKT matrix is factored again.  0 (the default) = off = the reference's fixed rho.  Measured with interval 5 on the
    * walking log: QPs ending at max_iter 1.29 % -> 0, mean iterations of the QPs that iterate 66 -> 18; multi-contact
-   * humanoid set 16.8 % -> 3.1 %.  All three kernels implement it; shared-structure batches ignore it.  (This field was
+   * humanoid set 16.8 % -> 3.1 %.  All three kernels implement it.  A shared-structure batch (Q and A_eq with batch stride 0) that sets
+   * it runs on the per-QP kernels instead of the cached-factorization path.  (This field was
    * `reserved`, always 0, up to ABI version 3.) */
   int32_t adapt_rho_interval; /* 0 */
   double rho;        /* 1e-6 */
