@@ -157,15 +157,16 @@ const DevSwitches& dev_switches() {
 }
 
 // Whether the CTA-per-QP kernels take the shape: one thread per padded KKT row, at most 256 rows, the packed matrix in
-// shared memory.
+// shared memory.  The shared memory binds first: on a B200 (227 KB) padded n + m <= 224 when m <= n.
 int check_shape(const DeviceCtx& ctx, int n, int m, int nc) {
   const int N = n + m;
   if (N < 1) return fail(FCCQP_E_INVALID, "n + m must be >= 1");
   const fccqp::Layout l(n, m, nc);
   if (l.N8 > 256 || l.bytes() > (size_t)ctx.max_smem_optin)
     return fail(FCCQP_E_UNSUPPORTED,
-                "n + m = %d (padded %d) needs %zu B of shared memory per QP (limit %d B, 256 rows): too large "
-                "for the shared-memory-resident kernels", N, l.N8, l.bytes(), ctx.max_smem_optin);
+                "n + m = %d (padded %d) needs %zu B of shared memory per QP, the device allows %d B (a B200 takes "
+                "padded n + m <= 224 when m <= n): too large for the shared-memory-resident kernels", N, l.N8, l.bytes(),
+                ctx.max_smem_optin);
   return FCCQP_OK;
 }
 

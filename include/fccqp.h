@@ -37,6 +37,10 @@ typedef enum fccqp_error {
   FCCQP_E_CUDA = -2,        /* CUDA runtime failure (message has the CUDA error string)      */
   FCCQP_E_UNSUPPORTED = -3  /* problem too large for the device kernels, unknown precision   */
 } fccqp_error;
+/* Largest problem: the padded KKT matrix of one QP (n and m each rounded up to a multiple of 8) lives in the opt-in
+ * shared memory of one thread block.  On a B200 (227 KB per block) that allows padded n + m <= 224 for every problem
+ * with m <= n (e.g. n = 140, m = 76); fccqp_create and the batch calls return FCCQP_E_UNSUPPORTED for a problem with
+ * m <= n whose padded n + m is 232 or more.  (Only problems with more equality rows than variables, n <= 16, fit at 232.) */
 
 /* Per-QP solve status.  0/1 are the reference's FCCQPSolveStatus
  * (src/fcc_qp.hpp:14-17; derived at src/fcc_qp.cpp:203-204).  2 is an

@@ -9,11 +9,14 @@ import numpy as np
 import pytest
 
 import oracle
+from kernel_layout import layout_bytes
 from test_gpu_random_shapes import random_qps, rel
 
 pytestmark = pytest.mark.gpu
 OPTS = dict(max_iter=200, rho=1e-3, eps_fcone=1e-7, eps_bound=1e-7)
-SMALL = [(5, 2, 3, 1), (12, 6, 6, 3), (18, 14, 6, 10), (24, 8, 9, 0), (32, 0, 12, 20), (3, 0, 3, 0), (20, 12, 0, 0)]
+# n + m = 32 is the largest shape of the warp kernel, 33 the smallest of the CTA-per-QP kernels
+SMALL = [(5, 2, 3, 1), (12, 6, 6, 3), (18, 14, 6, 10), (24, 8, 9, 0), (32, 0, 12, 20), (3, 0, 3, 0), (20, 12, 0, 0),
+         (27, 6, 9, 12)]
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -34,7 +37,8 @@ def test_small_shapes_cold_and_warm_match_the_restatement(n, m, nc, lcs):
     s = solver(n, m, nc, lcs)
     s.Solve(qp.Q, qp.b, qp.A_eq, qp.b_eq, qp.friction_coeffs, qp.lb, qp.ub)
     sol = s.GetSolution()
-    assert nat.last_launch_info()["block"] == 128 and nat.last_launch_info()["smem_bytes"] == 4 * (n + m) * ((n + m) | 1) * 8
+    smem = 4 * (n + m) * ((n + m) | 1) * 8 if n + m <= 32 else layout_bytes(n, m, nc)   # else the general kernel
+    assert nat.last_launch_info()["block"] == 128 and nat.last_launch_info()["smem_bytes"] == smem
     same = sol.details.n_iter == ref["n_iter"]
     assert rel(sol.z[same], ref["z"][same]) <= 1e-6
     assert (~same).mean() <= 0.01, (~same).sum()
