@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # FCCQP_LIB: developer override (e.g. an instrumented -DFCCQP_DEV build of the same sources)
 LIB_PATH = os.environ.get("FCCQP_LIB") or os.path.join(_HERE, "libfccqp_b200.so")
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 STRUCTURE_AUTO, STRUCTURE_DENSE, STRUCTURE_CAPS = 0, 1, 2
 STRUCTURE_REFINE = 256   # flag: iterative refinement of the reduced cold pre-solve
 SCHEDULE_LPT = 512       # flag: n_iter holds an earlier solve's counts; lanes that ran long are processed first
@@ -65,6 +65,7 @@ class BatchDesc(C.Structure):
         ("stream", C.c_void_p),
         ("device_seconds", _dp),
         ("structure", C.c_int32), ("struct_caps", C.c_int32 * 3),
+        ("warm_lanes", C.c_void_p),
     ]
 
 

@@ -101,6 +101,7 @@ class FCCQPBatch:
         self.schedule_from_previous = False
         self._caps = None
         self.warm_start = False
+        self.warm_lanes = None  # per-lane mask of set_warm_start (None: warm_start holds for every lane)
         self.time_kernel = True
         self._state = None     # (x, mu_x, mu_c) arrays / tensors
         self._host_out = None  # page-locked output buffers of the numpy path
@@ -124,8 +125,42 @@ class FCCQPBatch:
         self.options = FCCQPOptionsB(int(opt.max_iter), float(opt.rho), float(opt.eps_fcone), float(opt.eps_bound),
                                      float(getattr(opt, "relaxation", 1.0)), int(getattr(opt, "adapt_rho_interval", 0)))
 
-    def set_warm_start(self, warm_start: bool):
-        self.warm_start = bool(warm_start)
+    def set_warm_start(self, warm_start):
+        """``True`` / ``False`` for every lane, as on the reference object; or a per-lane ``[B]`` mask: lane i is solved
+        as a reference object after ``set_warm_start(mask[i] != 0)`` -- warm from its carried state, or cold (pre-solve,
+        zero duals).  A numpy bool / uint8 array for numpy batches (staged with the batch), a torch CUDA bool / uint8
+        tensor for device batches: passed by pointer, read by the kernels when they run, so a mask updated in place
+        between replays of a captured CUDA graph takes effect at every replay.  The mask is kept, not copied."""
+        if _is_torch(warm_start):
+            import torch
+            if warm_start.dtype not in (torch.bool, torch.uint8) or warm_start.dim() != 1:
+                raise ValueError("a warm-start mask must be a 1-D bool or uint8 tensor")
+            if warm_start.device.type != "cuda":
+                raise ValueError("a torch warm-start mask must be a CUDA tensor (numpy masks go with numpy batches)")
+            if warm_start.numel() > 1 and warm_start.stride(0) != 1:
+                raise ValueError("a warm-start mask must be contiguous (it is read in place)")
+            self.warm_start, self.warm_lanes = True, warm_start
+        elif isinstance(warm_start, np.ndarray) and warm_start.ndim > 0:
+            if warm_start.dtype not in (np.bool_, np.uint8) or warm_start.ndim != 1:
+                raise ValueError("a warm-start mask must be a 1-D bool or uint8 array")
+            self.warm_start, self.warm_lanes = True, np.ascontiguousarray(warm_start)
+        else:
+            self.warm_start, self.warm_lanes = bool(warm_start), None
+
+    def _mask_ptr(self, B: int, dev) -> int:
+        """Pointer of the per-lane mask for a batch of B lanes (0: none); refuses a mask that does not fit the call."""
+        w = self.warm_lanes
+        if w is None:
+            return 0
+        if w.shape[0] != B:
+            raise ValueError(f"warm-start mask has {w.shape[0]} lanes, the batch {B}")
+        if dev is None:
+            if _is_torch(w):
+                raise ValueError("numpy batch with a torch warm-start mask: pass a numpy mask")
+            return w.ctypes.data
+        if not _is_torch(w) or w.device != dev:
+            raise ValueError(f"device batch on {dev} needs a CUDA warm-start mask on the same device")
+        return w.data_ptr()
 
     def contact_vars_start(self) -> int:
         return self.lcs
@@ -241,6 +276,7 @@ class FCCQPBatch:
         self._check_shapes([a.shape for a in (Q, b, A_eq, b_eq, mu, lb, ub)], B)
         n, m, nc = self.n, self.m, self.nc
         warm = self.warm_start
+        mask = self._mask_ptr(B, None)
         st = self._state
         # Outputs live in solver-owned page-locked buffers (true asynchronous D2H), reused from
         # call to call; x doubles as the carried warm-start state, exactly like the reference's x_.
@@ -262,6 +298,7 @@ class FCCQPBatch:
         n_iter, status, res = ob["n_iter"], ob["status"], ob["res"]
         d = self._desc(B, nat.MEM_HOST)
         d.warm_start = int(warm)
+        d.warm_lanes = mask or None
         p = lambda a: a.ctypes.data
         d.Q, d.q_batch_stride, d.q_row_stride, d.q_col_stride = p(Q), (0 if shared else n * n), n, 1
         d.b, d.b_batch_stride = p(b), n
@@ -310,6 +347,7 @@ class FCCQPBatch:
         cont = lambda a: a if a.stride(-1) == 1 or a.shape[-1] <= 1 else a.contiguous()
         b, b_eq, mu, lb, ub = map(cont, (b, b_eq, mu, lb, ub))
         warm = self.warm_start
+        mask = self._mask_ptr(B, dev)
         st = self._state
         # Outputs and carried state live in solver-owned device tensors, allocated once per (B, device) and reused
         # from call to call (nothing is allocated inside a steady-state Solve).  A cold solve ignores the state
@@ -340,6 +378,7 @@ class FCCQPBatch:
         d = self._desc(B, nat.MEM_DEVICE)
         probed = (d.structure & ~(nat.STRUCTURE_REFINE | nat.SCHEDULE_LPT)) == nat.STRUCTURE_AUTO
         d.warm_start = int(warm)
+        d.warm_lanes = mask or None
         if self.schedule_from_previous and not fresh:
             d.structure |= nat.SCHEDULE_LPT
         bs = lambda a, full_ndim: int(a.stride(0)) if a.dim() == full_ndim and B > 1 else (
@@ -366,6 +405,7 @@ class FCCQPBatch:
         self._after_device_call(B, probed)
         # keep the inputs alive until the (possibly asynchronous) launch has consumed them
         self._keepalive = (Q, b, A_eq, b_eq, mu, lb, ub)
+        self._mask_keepalive = self.warm_lanes
         self._state = (x, mux, muc)
         # zero_copy_outputs: z and the details are the solver-owned tensors themselves, valid until the next Solve();
         # default: independent copies, like FCCQP::GetSolution
@@ -461,11 +501,22 @@ class FCCQPBatchCpp:
             else mod.FCCQPBatch(self.n, self.m, self.nc, self.lcs, int(device))
         self._out = None
         self._sol = None
+        self._mask = None      # torch per-lane mask of the device path (SolveDLPack's warm_lanes)
         self.time_kernel = False
 
     def set_rho(self, rho): self._s.set_rho(float(rho))
     def set_max_iter(self, n): self._s.set_max_iter(int(n))
-    def set_warm_start(self, warm_start): self._s.set_warm_start(bool(warm_start))
+
+    def set_warm_start(self, warm_start):
+        """A bool, or a per-lane [B] mask: numpy / sequence for host stacks, a CUDA bool / uint8 tensor for device ones."""
+        self._mask = None
+        if _is_torch(warm_start):
+            self._mask = warm_start
+            self._s.set_warm_start(True)
+        elif isinstance(warm_start, (list, tuple)) or (isinstance(warm_start, np.ndarray) and warm_start.ndim > 0):
+            self._s.set_warm_start(np.asarray(warm_start, dtype=np.uint8))
+        else:
+            self._s.set_warm_start(bool(warm_start))
     def contact_vars_start(self): return self.lcs
 
     def set_options(self, opt):
@@ -494,8 +545,9 @@ class FCCQPBatchCpp:
             else torch.as_tensor(np.asarray(friction_coeffs, dtype=np.float64), device=dev)
         with torch.cuda.device(dev):
             secs = self._s.SolveDLPack(Q, b, A_eq, b_eq, mu, lb, ub, *o,
-                                       stream=torch.cuda.current_stream(dev).cuda_stream, time_kernel=self.time_kernel)
-        self._keepalive = (Q, b, A_eq, b_eq, mu, lb, ub)
+                                       stream=torch.cuda.current_stream(dev).cuda_stream, time_kernel=self.time_kernel,
+                                       warm_lanes=self._mask)
+        self._keepalive = (Q, b, A_eq, b_eq, mu, lb, ub, self._mask)
         x, _, _, n_iter, status, det = o
         self._sol = BatchSolution(BatchDetails(n_iter, det[0], det[1], det[2], det[3], status, secs, secs), x)
 

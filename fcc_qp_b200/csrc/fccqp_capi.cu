@@ -31,7 +31,7 @@ std::atomic<long long> g_launches{0};
 struct LaunchInfo { int grid = 0, block = 0, smem = 0, ctas_per_sm = 0; };
 LaunchInfo g_last_launch;
 // what the last batch launch did about problem structure (fccqp_last_struct_info)
-struct StructInfo { int used = 0, nr = 0, ndp = 0, nd0 = 0, rows = 0, rows_dense = 0, device = 0; };
+struct StructInfo { int used = 0, nr = 0, ndp = 0, nd0 = 0, rows = 0, rows_dense = 0, device = 0, deferred_words = 1; };
 StructInfo g_last_struct;
 std::mutex g_info_mu;
 
@@ -80,7 +80,8 @@ struct DeviceCtx {
   char* hstage = nullptr;
   size_t hstage_bytes = 0;
   cudaEvent_t chunk_ev[16] = {};
-  unsigned int* h_deferred = nullptr;   // pinned: QPs the structure-exploiting kernel handed to the general one (last launch)
+  unsigned int* h_deferred = nullptr;   // pinned [2]: QPs the structure-exploiting kernel handed to the general one (last
+                                        // launch; [1]: its warm QPs when it had a per-lane mask)
   int* h_probe = nullptr;               // pinned [4]: result of the structure probe
   std::mutex mu;       // guards counters / gscratch / occupancy cache
   std::mutex host_mu;  // serialises FCCQP_MEM_HOST calls (they share the staging buffer)
@@ -118,8 +119,8 @@ int get_ctx(int device, DeviceCtx** out) {
   }
   for (auto& s : ctx->streams) CUDA_TRY(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
   for (auto& e : ctx->chunk_ev) CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  CUDA_TRY(cudaMallocHost(&ctx->h_deferred, sizeof(unsigned int)));
-  *ctx->h_deferred = 0;
+  CUDA_TRY(cudaMallocHost(&ctx->h_deferred, 2 * sizeof(unsigned int)));
+  ctx->h_deferred[0] = ctx->h_deferred[1] = 0;
   CUDA_TRY(cudaMallocHost(&ctx->h_probe, 4 * sizeof(int)));
   *out = ctx.get();
   g_ctx[device] = std::move(ctx);
@@ -252,24 +253,63 @@ struct Scratch {
   static constexpr size_t kWork = 0;       // work counter of the first launch
   static constexpr size_t kWork2 = 1;      // work counter of the second launch
   static constexpr size_t kListCount = 2;  // length of the hand-over list
+  static constexpr size_t kWarmListCount = 3;  // per-lane mask: length of the warm QPs' hand-over list (next to kListCount)
   static constexpr size_t kProbe = 4;      // [4, 8): structure probe (atomicMax)
   static constexpr size_t kLpt = 8;        // [8, 10): counters of lpt_order_kernel
   static constexpr size_t kWork3 = 10;     // work counter of the resume launch of a two-stage structure solve
   static constexpr size_t kResumeCount = 11;  // length of its list
-  static constexpr size_t kHeader = 16;    // then [B] the hand-over list, [B] the resume list, [B] the LPT order
+  static constexpr size_t kColdCount = 12;    // per-lane mask: lengths of the cold and the warm list (warm_split_kernel)
+  static constexpr size_t kWarmCount = 13;
+  static constexpr size_t kWork4 = 14;     // per-lane mask: work counters of the launches over the warm QPs
+  static constexpr size_t kWork5 = 15;
+  static constexpr size_t kHeader = 16;    // then [B] the hand-over list, [B] the resume list, [B] the LPT order; with a
+                                           // per-lane mask also [B] the cold list, [B] the warm list, [B] the warm hand-over
   unsigned int* w = nullptr;
   size_t B = 0;
+  bool mask = false;                       // a per-lane mask: the call runs as a cold call over the cold list and a warm one
+                                           // over the warm list
   int* list() const { return reinterpret_cast<int*>(w + kHeader); }
   int* resume_list() const { return reinterpret_cast<int*>(w + kHeader + B); }
   int* order() const { return reinterpret_cast<int*>(w + kHeader + 2 * B); }
+  int* cold_list() const { return reinterpret_cast<int*>(w + kHeader + 3 * B); }
+  int* warm_list() const { return reinterpret_cast<int*>(w + kHeader + 4 * B); }
+  int* warm_handover() const { return reinterpret_cast<int*>(w + kHeader + 5 * B); }
 };
+
+// Per-lane warm start (fccqp_batch_desc::warm_lanes): the processing order (`order`, or 0..B-1) split into the cold and the
+// warm QPs, in that order within every warp of 32 slots; counts[0] / counts[1] = the lengths (zeroed by the caller).  The
+// lists are pre-filled with kNoQP (>= B) bytes: the warp and structure-exploiting kernels stop at an index >= B and need no
+// count; the general and shared-structure kernels take the count (SolveParams::count_dev).
+constexpr unsigned char kNoQPByte = 0x7f;
+__global__ void __launch_bounds__(256) warm_split_kernel(const uint8_t* __restrict__ warm_lanes, const int* __restrict__ order,
+                                                         const int B, int* __restrict__ cold_list, int* __restrict__ warm_list,
+                                                         unsigned int* __restrict__ counts) {
+  const int slot = blockIdx.x * blockDim.x + threadIdx.x, lane = threadIdx.x & 31;
+  const int qp = slot < B ? (order ? order[slot] : slot) : -1;
+  const bool warm = qp >= 0 && warm_lanes[qp] != 0, cold = qp >= 0 && !warm;
+  const unsigned int bw = __ballot_sync(0xffffffffu, warm), bc = __ballot_sync(0xffffffffu, cold);
+  unsigned int base_c = 0, base_w = 0;
+  if (lane == 0) {
+    if (bc) base_c = atomicAdd(counts, (unsigned int)__popc(bc));
+    if (bw) base_w = atomicAdd(counts + 1, (unsigned int)__popc(bw));
+  }
+  base_c = __shfl_sync(0xffffffffu, base_c, 0);
+  base_w = __shfl_sync(0xffffffffu, base_w, 0);
+  const unsigned int below = (1u << lane) - 1u;
+  if (cold) cold_list[base_c + __popc(bc & below)] = qp;
+  if (warm) warm_list[base_w + __popc(bw & below)] = qp;
+}
 
 // Allocates the scratch of a call.  FCCQP_SCHEDULE_LPT, when the batch holds at least two QPs for each of the `slots`
 // that run at once: QPs whose previous solve ran long go to the front of the processing order (p.index_list).
-int begin_call(fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long long slots, Scratch* s) {
+// warm_lanes (device memory): the processing order is split into the cold and the warm list (Scratch::cold_list / warm_list).
+int begin_call(fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long long slots, Scratch* s,
+               const uint8_t* warm_lanes) {
   const bool lpt = lpt_hint && p.n_iter != nullptr && p.B >= 2 * slots;
   s->B = (size_t)p.B;
-  CUDA_TRY(cudaMallocAsync(&s->w, (Scratch::kHeader + (lpt ? 3 : 2) * s->B) * sizeof(unsigned int), stream));
+  s->mask = warm_lanes != nullptr;
+  const size_t arrays = s->mask ? 6 : (lpt ? 3 : 2);
+  CUDA_TRY(cudaMallocAsync(&s->w, (Scratch::kHeader + arrays * s->B) * sizeof(unsigned int), stream));
   CUDA_TRY(cudaMemsetAsync(s->w, 0, Scratch::kHeader * sizeof(unsigned int), stream));
   p.work_counter = s->w + Scratch::kWork;
   if (lpt) {
@@ -278,7 +318,24 @@ int begin_call(fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long l
     CUDA_TRY(cudaGetLastError());
     p.index_list = s->order();
   }
+  if (s->mask) {
+    CUDA_TRY(cudaMemsetAsync(s->cold_list(), kNoQPByte, 2 * s->B * sizeof(int), stream));
+    warm_split_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(warm_lanes, p.index_list, p.B, s->cold_list(), s->warm_list(),
+                                                             s->w + Scratch::kColdCount);
+    CUDA_TRY(cudaGetLastError());
+  }
   return FCCQP_OK;
+}
+
+// The cold or the warm QPs of a call with a per-lane mask as a uniform call of their own: the list of begin_call as the
+// processing order, counted (count_dev) for the kernels that need the count, and a work counter of their own.
+fccqp::SolveParams mask_lanes(const fccqp::SolveParams& p, const Scratch& s, bool warm, bool counted) {
+  fccqp::SolveParams q = p;
+  q.warm = warm;
+  q.index_list = warm ? s.warm_list() : s.cold_list();
+  q.count_dev = counted ? s.w + (warm ? Scratch::kWarmCount : Scratch::kColdCount) : nullptr;
+  q.work_counter = s.w + (warm ? Scratch::kWork4 : Scratch::kWork);
+  return q;
 }
 
 // Frees the scratch (stream-ordered) and records the call for fccqp_kernel_launch_count, fccqp_last_launch_info and
@@ -341,7 +398,7 @@ const char* const kGeneralPhases[16] = {"stage-in", "assemble", "sigma/rhs0", "l
 // Small problems (n + m <= 32): one QP per warp (fccqp_warp.cuh), four warps per CTA, each pulling QPs from the work
 // counter on its own; shared memory per CTA = 4 private (n + m) x ((n + m) | 1) slabs.
 // f32: the FP32 arithmetic instance (FCCQP_PRECISION_FP32: float32 problem data, float slabs).
-int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool f32, bool lpt_hint) {
+int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool f32, bool lpt_hint, const uint8_t* warm_lanes) {
   constexpr int kW = 4;
   const int N = p.n + p.m;
   const size_t smem = (size_t)kW * N * (N | 1) * (f32 ? sizeof(float) : sizeof(double));
@@ -351,8 +408,15 @@ int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool 
   LaunchInfo li;
   Scratch s;
   int rc = geometry(ctx, fn, 32 * kW, smem, p.B, kW, &li);
-  if (!rc) rc = begin_call(p, stream, lpt_hint, (long long)kW * li.ctas_per_sm * ctx.num_sms, &s);
+  if (!rc) rc = begin_call(p, stream, lpt_hint, (long long)kW * li.ctas_per_sm * ctx.num_sms, &s, warm_lanes);
   if (rc) return rc;
+  if (s.mask) {   // the cold QPs, then the warm ones (each list ends at its kNoQP padding)
+    fn<<<li.grid, li.block, smem, stream>>>(mask_lanes(p, s, false, false));
+    CUDA_TRY(cudaGetLastError());
+    fn<<<li.grid, li.block, smem, stream>>>(mask_lanes(p, s, true, false));
+    CUDA_TRY(cudaGetLastError());
+    return end_call(s, stream, 2, li, dense_info(ctx, N));
+  }
   fn<<<li.grid, li.block, smem, stream>>>(p);
   CUDA_TRY(cudaGetLastError());
   return end_call(s, stream, 1, li, dense_info(ctx, N));
@@ -361,6 +425,7 @@ int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool 
 // Shared-structure batch (one Q and one A_eq for the whole batch): every CTA caches its KKT factorization
 // (SolveParams::shared_mode).  Cold: a pre-solve launch hands the QPs that need ADMM iterations to an ADMM launch.
 // Warm (an MPC loop re-solving around one linearisation with carried duals): no pre-solve, the ADMM launch alone.
+// Per-lane mask: the cold sequence over the cold QPs, then the warm ADMM launch over the warm ones.
 int launch_shared(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s) {
   const int threads = p.lay.N8 <= 128 ? 128 : 256;
   KernelFn fn = pick_kernel(threads, true, false, false);
@@ -368,6 +433,24 @@ int launch_shared(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, con
   int rc = geometry(ctx, fn, threads, p.lay.bytes(), p.B, 1, &li);
   if (rc) return rc;
   p.shared_mode = 2;
+  if (s.mask) {
+    fccqp::SolveParams a = mask_lanes(p, s, false, true);
+    a.shared_mode = 1;
+    a.pending_count = s.w + Scratch::kListCount;
+    a.pending_list = s.list();
+    fn<<<li.grid, li.block, li.smem, stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    fccqp::SolveParams c = p;
+    c.warm = 0;
+    c.count_dev = a.pending_count;
+    c.index_list = s.list();
+    c.work_counter = s.w + Scratch::kWork2;
+    fn<<<li.grid, li.block, li.smem, stream>>>(c);
+    CUDA_TRY(cudaGetLastError());
+    fn<<<li.grid, li.block, li.smem, stream>>>(mask_lanes(p, s, true, true));
+    CUDA_TRY(cudaGetLastError());
+    return end_call(s, stream, 3, li, dense_info(ctx, p.lay.N8));
+  }
   if (!p.warm) {
     fccqp::SolveParams a = p;
     a.shared_mode = 1;
@@ -430,15 +513,16 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   if (rc) return rc;
   // Cold batches of at least 8 QPs per resident CTA run in two stages: the first-stage kernel takes every QP through the
   // exit test of iteration 0 (where nearly all whole-body-control QPs stop) and lists the others, which the full kernel
-  // resumes from there.  Smaller batches and warm solves keep the single launch.
-  const bool split = !p.warm && p.B >= 8LL * fli.ctas_per_sm * ctx.num_sms;
+  // resumes from there.  Smaller batches and warm solves keep the single launch.  A per-lane mask: the cold QPs as a cold
+  // call of the whole batch (split by the same rule), the warm ones as the single launch of a warm call.
+  const bool split = (!p.warm || s.mask) && p.B >= 8LL * fli.ctas_per_sm * ctx.num_sms;
   KernelFn fn;
   if (threads == 64) fn = struct_instance<64, 8>(adapt);
   else if (threads == 96) fn = struct_instance<96, 5>(adapt);
   else if (threads == 128) fn = struct_instance<128, 4>(adapt);
   else fn = struct_instance<256, 2>(adapt);
   if ((rc = geometry(ctx, fn, threads, sl.bytes(), p.B, 1, &li))) return rc;
-  fccqp::SolveParams a = p;
+  fccqp::SolveParams a = s.mask ? mask_lanes(p, s, false, false) : p;
   a.slay = sl;
   a.pending_count = s.w + Scratch::kListCount;
   a.pending_list = s.list();
@@ -470,20 +554,45 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
 #endif
   fn<<<li.grid, li.block, li.smem, stream>>>(a);
   CUDA_TRY(cudaGetLastError());
+  if (s.mask) {
+    fccqp::SolveParams w = mask_lanes(p, s, true, false);
+    w.slay = sl;
+    w.pending_count = s.w + Scratch::kWarmListCount;
+    w.pending_list = s.warm_handover();
+    w.op_stride = a.op_stride;
+    w.op_scratch = a.op_scratch;
+    fn<<<li.grid, li.block, li.smem, stream>>>(w);
+    CUDA_TRY(cudaGetLastError());
+  }
   CUDA_TRY(cudaFreeAsync(a.op_scratch, stream));
 #ifdef FCCQP_DEV
   if ((rc = prof.report(stream, split ? "struct resume" : "struct", kStructPhases, p.B, li.grid))) return rc;
 #endif
   fccqp::SolveParams b = p;
+  if (s.mask) b.warm = 0;
   b.count_dev = a.pending_count;
   b.index_list = s.list();
   b.work_counter = s.w + Scratch::kWork2;
   general<<<gli.grid, gli.block, gli.smem, stream>>>(b);
   CUDA_TRY(cudaGetLastError());
-  CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, a.pending_count, sizeof(unsigned int), cudaMemcpyDeviceToHost, stream));
+  int launches = split ? 3 : 2;
+  if (s.mask) {   // the warm QPs the full kernel handed over
+    fccqp::SolveParams bw = p;
+    bw.warm = 1;
+    bw.count_dev = s.w + Scratch::kWarmListCount;
+    bw.index_list = s.warm_handover();
+    bw.work_counter = s.w + Scratch::kWork5;
+    general<<<gli.grid, gli.block, gli.smem, stream>>>(bw);
+    CUDA_TRY(cudaGetLastError());
+    launches += 2;
+  }
+  // (the warm hand-over count sits right after the cold one)
+  const int words = s.mask ? 2 : 1;
+  CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, a.pending_count, words * sizeof(unsigned int), cudaMemcpyDeviceToHost, stream));
   StructInfo si;
   si.used = 1; si.nr = caps[0]; si.ndp = caps[1]; si.nd0 = caps[2]; si.rows = sl.N8c; si.rows_dense = p.lay.N8; si.device = ctx.device;
-  return end_call(s, stream, split ? 3 : 2, split ? fli : li, si);
+  si.deferred_words = words;
+  return end_call(s, stream, launches, split ? fli : li, si);
 }
 
 int launch_general(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s, KernelFn fn, const LaunchInfo& li) {
@@ -492,18 +601,26 @@ int launch_general(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, co
   int rc = prof.start(stream, &p);
   if (rc) return rc;
 #endif
-  fn<<<li.grid, li.block, li.smem, stream>>>(p);
+  if (s.mask) {   // the cold QPs, then the warm ones
+    fn<<<li.grid, li.block, li.smem, stream>>>(mask_lanes(p, s, false, true));
+    CUDA_TRY(cudaGetLastError());
+    fn<<<li.grid, li.block, li.smem, stream>>>(mask_lanes(p, s, true, true));
+  } else {
+    fn<<<li.grid, li.block, li.smem, stream>>>(p);
+  }
   CUDA_TRY(cudaGetLastError());
 #ifdef FCCQP_DEV
   if ((rc = prof.report(stream, "general", kGeneralPhases, p.B, li.grid))) return rc;
 #endif
-  return end_call(s, stream, 1, li, dense_info(ctx, p.lay.N8));
+  return end_call(s, stream, s.mask ? 2 : 1, li, dense_info(ctx, p.lay.N8));
 }
 
 // Launches the solve on `stream` for device-resident data described by p (scratch allocated here, stream-ordered).
 // precision: fccqp_precision of the call (FP32_DATA and FP32: float32 problem data behind the pointers of p; FP32: FP32
 // arithmetic too where a kernel for it exists -- the warp kernel -- and FP32_DATA's FP64 arithmetic otherwise)
-int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int precision, const StructHint& hint) {
+// warm_lanes: optional per-lane mask in device memory (fccqp_batch_desc::warm_lanes); p.warm is then ignored.
+int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int precision, const StructHint& hint,
+                 const uint8_t* warm_lanes = nullptr) {
   if (p.B == 0) return FCCQP_OK;
   int rc = check_shape(ctx, p.n, p.m, p.nc);
   if (rc) return rc;
@@ -514,7 +631,7 @@ int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int 
   p.full_inverse_at = sw.full_inverse_at ? sw.full_inverse_at : (small ? 8 : 6);
   p.struct_refine = hint.refine;
   if (small && (precision == FCCQP_PRECISION_FP32 || (!f32 && !sw.no_warp)))
-    return launch_warp(ctx, p, stream, precision == FCCQP_PRECISION_FP32, hint.lpt);
+    return launch_warp(ctx, p, stream, precision == FCCQP_PRECISION_FP32, hint.lpt, warm_lanes);
 
   // one CTA per QP; float32 problem data take the general kernel's widening instance, same geometry
   const int threads = p.lay.N8 <= 128 ? 128 : 256;
@@ -522,7 +639,7 @@ int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int 
   LaunchInfo li;
   Scratch s;
   if ((rc = geometry(ctx, general, threads, p.lay.bytes(), p.B, 1, &li)) ||
-      (rc = begin_call(p, stream, hint.lpt, (long long)li.ctas_per_sm * ctx.num_sms, &s)))
+      (rc = begin_call(p, stream, hint.lpt, (long long)li.ctas_per_sm * ctx.num_sms, &s, warm_lanes)))
     return rc;
   // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs.  Not with
   // adaptive rho: a lane that moves its rho needs its own rho-KKT factorization, so those batches take the
@@ -655,7 +772,8 @@ int fccqp_last_struct_info(int* used, int* caps, int* rows, int* rows_dense, int
     if (si.used) {
       std::lock_guard<std::mutex> lk(g_ctx_mu);
       auto it = g_ctx.find(si.device);
-      if (it != g_ctx.end() && it->second->h_deferred) *deferred = (int)*it->second->h_deferred;
+      if (it != g_ctx.end() && it->second->h_deferred)
+        for (int k = 0; k < si.deferred_words; ++k) *deferred += (int)it->second->h_deferred[k];
     }
   }
   return FCCQP_OK;
@@ -910,6 +1028,8 @@ static int validate_desc(const fccqp_batch_desc* d) {
   if (d->nc > 0 && !d->friction_coeffs) return fail(FCCQP_E_INVALID, "null friction_coeffs with nc > 0");
   if (d->warm_start && (!d->mu_x || (d->nc > 0 && !d->mu_lambda_c)))
     return fail(FCCQP_E_INVALID, "warm_start needs mu_x and mu_lambda_c");
+  if (d->warm_lanes && (!d->mu_x || (d->nc > 0 && !d->mu_lambda_c)))
+    return fail(FCCQP_E_INVALID, "warm_lanes needs mu_x and mu_lambda_c");
   return FCCQP_OK;
 }
 
@@ -947,7 +1067,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
       CUDA_TRY(cudaEventCreate(&ev1));
       CUDA_TRY(cudaEventRecord(ev0, st));
     }
-    rc = launch_solve(*ctx, p, st, d.precision, hint);
+    rc = launch_solve(*ctx, p, st, d.precision, hint, d.warm_lanes);
     if (rc) { if (ev0) { cudaEventDestroy(ev0); cudaEventDestroy(ev1); } return rc; }
     if (d.device_seconds) {
       float ms = 0.f;
@@ -990,6 +1110,8 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
   Seg sx = seg(cur, n, false), smx = seg(cur, n, false), smc = seg(cur, nc, false);
   Seg sres = seg(cur, 4, false);
   Seg sint = seg(cur, 1, false);  // 2 ints per QP packed in one double slot
+  const Seg smask{cur, 1, false};  // per-lane warm mask: one byte per QP
+  if (d.warm_lanes) cur += align_up((size_t)B, 256);
   if (cur > ctx->stage_bytes) {
     if (ctx->stage) CUDA_TRY(cudaFree(ctx->stage));
     ctx->stage = nullptr; ctx->stage_bytes = 0;
@@ -1066,9 +1188,10 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
     if ((rc = h2d(sQ, d.Q, es)) || (rc = h2d(sA, d.A_eq, es)) || (rc = h2d(sb, d.b, es)) || (rc = h2d(sbeq, d.b_eq, es)) ||
         (rc = h2d(smu, d.friction_coeffs, es)) || (rc = h2d(slb, d.lb, es)) || (rc = h2d(sub, d.ub, es)))
       return rc;
-    if (d.warm_start) {
+    if (d.warm_start || d.warm_lanes) {
       if ((rc = h2d(sx, d.x, 8)) || (rc = h2d(smx, d.mu_x, 8)) || (rc = h2d(smc, d.mu_lambda_c, 8))) return rc;
     }
+    if (d.warm_lanes && (rc = h2d(smask, d.warm_lanes, 1))) return rc;
     fccqp::SolveParams p = solve_params((int)cnt, n, m, nc, d.lambda_c_start, d.options, d.warm_start != 0);
     auto off = [&](const Seg& s) { return s.shared ? dp(s) : dp(s) + lo * s.per_qp; };
     auto offi = [&](const Seg& s) {   // problem data: element size es
@@ -1085,7 +1208,8 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
     p.n_iter = d_niter + lo; p.status = d_status + lo;
     double* res = dp(sres);
     p.res_b = res + lo; p.res_f = res + (size_t)B + lo; p.bviol = res + 2 * (size_t)B + lo; p.fviol = res + 3 * (size_t)B + lo;
-    rc = launch_solve(*ctx, p, st, d.precision, hint);
+    rc = launch_solve(*ctx, p, st, d.precision, hint,
+                      d.warm_lanes ? reinterpret_cast<const uint8_t*>(base + smask.off) + lo : nullptr);
     if (rc) return rc;
     // D2H: straight into the caller's buffer when it is page-locked (a true asynchronous DMA);
     // otherwise into the pinned bounce buffer, copied out below once the chunk's event has fired
@@ -1185,6 +1309,7 @@ int fccqp_batch_solve_multi(const fccqp_batch_desc* desc, const int32_t* devices
     if (d.x) s.x = d.x + lo * d.n;
     if (d.mu_x) s.mu_x = d.mu_x + lo * d.n;
     if (d.mu_lambda_c) s.mu_lambda_c = d.mu_lambda_c + lo * d.nc;
+    if (d.warm_lanes) s.warm_lanes = d.warm_lanes + lo;
     if (d.n_iter) s.n_iter = d.n_iter + lo;
     if (d.status) s.status = d.status + lo;
     if (d.res_bounds) s.res_bounds = d.res_bounds + lo;

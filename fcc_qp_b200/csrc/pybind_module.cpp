@@ -52,7 +52,7 @@ struct DLDevice_ { int32_t device_type; int32_t device_id; };
 struct DLDataType_ { uint8_t code; uint8_t bits; uint16_t lanes; };
 struct DLTensor_ { void* data; DLDevice_ device; int32_t ndim; DLDataType_ dtype; int64_t* shape; int64_t* strides; uint64_t byte_offset; };
 struct DLManagedTensor_ { DLTensor_ dl_tensor; void* manager_ctx; void (*deleter)(DLManagedTensor_*); };
-constexpr int kDLCUDA = 2, kDLInt = 0, kDLFloat = 2;
+constexpr int kDLCUDA = 2, kDLInt = 0, kDLUInt = 1, kDLFloat = 2, kDLBool = 6;
 
 struct DevView {
   void* data = nullptr;
@@ -61,6 +61,7 @@ struct DevView {
 };
 
 // Consumes the capsule at once (pointer, shape and strides are copied out; the caller keeps the tensor object alive).
+// code kDLUInt with bits 8 also takes kDLBool (one byte per element): the per-lane warm-start mask.
 DevView dev_view(const py::object& obj, const char* name, int code, int bits, int max_ndim) {
   if (!py::hasattr(obj, "__dlpack__")) throw py::type_error(std::string(name) + ": expected an object with __dlpack__ (device tensor)");
   py::capsule cap = obj.attr("__dlpack__")();
@@ -70,7 +71,8 @@ DevView dev_view(const py::object& obj, const char* name, int code, int bits, in
   DevView v;
   std::string err;
   if (t.device.device_type != kDLCUDA) err = ": must live in CUDA device memory (no CPU solve path; pass numpy arrays to Solve for host data)";
-  else if (t.dtype.code != code || t.dtype.bits != bits || t.dtype.lanes != 1) err = std::string(": must be ") + (code == kDLFloat ? "float64" : "int32");
+  else if (!(t.dtype.code == code || (code == kDLUInt && t.dtype.code == kDLBool)) || t.dtype.bits != bits || t.dtype.lanes != 1)
+    err = std::string(": must be ") + (code == kDLFloat ? "float64" : code == kDLInt ? "int32" : "bool or uint8");
   else if (t.ndim < 1 || t.ndim > max_ndim) err = ": wrong number of dimensions";
   if (err.empty()) {
     v.data = static_cast<char*>(t.data) + t.byte_offset;
@@ -196,7 +198,15 @@ PYBIND11_MODULE(fcc_qp_solver, m) {
            py::arg("nc"), py::arg("lambda_c_start"), py::arg("devices"))
       .def("set_rho", &FCCQPBatch::set_rho)
       .def("set_max_iter", &FCCQPBatch::set_max_iter)
-      .def("set_warm_start", &FCCQPBatch::set_warm_start)
+      // a bool for every lane, or a per-lane sequence (list, numpy bool / uint8 array) for the host Solve
+      .def("set_warm_start",
+           [](FCCQPBatch& self, const py::object& w) {
+             if (!py::isinstance<py::sequence>(w)) { self.set_warm_start(w.cast<bool>()); return; }
+             const auto a = py::array_t<uint8_t, py::array::c_style | py::array::forcecast>::ensure(w);
+             if (!a || a.ndim() != 1) throw py::value_error("a warm-start mask must be a 1-D sequence");
+             self.set_warm_start(std::vector<uint8_t>(a.data(), a.data() + a.size()));
+           },
+           py::arg("warm_start"))
       .def("set_options", &FCCQPBatch::set_options)
       .def("set_structure", &FCCQPBatch::set_structure)
       .def("contact_vars_start", &FCCQPBatch::contact_vars_start)
@@ -240,7 +250,7 @@ PYBIND11_MODULE(fcc_qp_solver, m) {
           [](FCCQPBatch& self, const py::object& Q, const py::object& b, const py::object& A_eq, const py::object& b_eq,
              const py::object& mu, const py::object& lb, const py::object& ub, const py::object& x, const py::object& mu_x,
              const py::object& mu_lambda_c, const py::object& n_iter, const py::object& solve_status, const py::object& details,
-             std::uintptr_t stream, bool time_kernel) {
+             std::uintptr_t stream, bool time_kernel, const py::object& warm_lanes) {
             const int n = self.num_vars(), mm = self.num_equality_constraints(), nc = self.num_contact_vars();
             const DevView vb = dev_view(b, "b", kDLFloat, 64, 2);
             if (vb.ndim != 2 || vb.shape[1] != n) throw py::value_error("b must be [B,n]");
@@ -269,14 +279,21 @@ PYBIND11_MODULE(fcc_qp_solver, m) {
             io.admm_residual_bounds = det; io.admm_residual_friction_cone = det + B; io.bounds_viol = det + 2 * (size_t)B;
             io.friction_cone_viol = det + 3 * (size_t)B;
             io.stream = reinterpret_cast<void*>(stream);
+            const uint8_t* mask = nullptr;   // per-lane warm start of this call, [B] bool / uint8 on the same device
+            if (!warm_lanes.is_none()) {
+              const DevView vm = dev_view(warm_lanes, "warm_lanes", kDLUInt, 8, 1);
+              if (vm.shape[0] != B || (B > 1 && vm.stride[0] != 1) || vm.device != io.device)
+                throw py::value_error("warm_lanes must be a contiguous [B] tensor on the device of the batch");
+              mask = static_cast<const uint8_t*>(vm.data);
+            }
             double secs = 0.0;
             {
               py::gil_scoped_release release;
-              self.SolveDevice(B, io, time_kernel ? &secs : nullptr);
+              self.SolveDevice(B, io, time_kernel ? &secs : nullptr, mask);
             }
             return secs;
           },
           py::arg("Q"), py::arg("b"), py::arg("A_eq"), py::arg("b_eq"), py::arg("friction_coeffs"), py::arg("lb"), py::arg("ub"),
           py::arg("x"), py::arg("mu_x"), py::arg("mu_lambda_c"), py::arg("n_iter"), py::arg("solve_status"), py::arg("details"),
-          py::arg("stream") = 0, py::arg("time_kernel") = false);
+          py::arg("stream") = 0, py::arg("time_kernel") = false, py::arg("warm_lanes") = py::none());
 }

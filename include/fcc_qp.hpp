@@ -14,6 +14,7 @@
 #pragma once
 
 #include <cstddef>
+#include <cstdint>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -245,11 +246,21 @@ class FCCQPBatch {
     opt_.max_iter = o.max_iter; opt_.rho = o.rho; opt_.eps_fcone = o.eps_fcone; opt_.eps_bound = o.eps_bound;
     opt_.relaxation = o.relaxation; opt_.adapt_rho_interval = o.adapt_rho_interval;
   }
-  void set_warm_start(bool warm_start) { warm_ = warm_start; }
+  void set_warm_start(bool warm_start) { warm_ = warm_start; warm_lanes_.clear(); }
+  // Per lane (fccqp_batch_desc::warm_lanes): lane i of the next host Solve is solved as an FCCQP after
+  // set_warm_start(warm_lanes[i] != 0).  The vector must hold one entry per lane of that Solve.
+  void set_warm_start(const std::vector<uint8_t>& warm_lanes) {
+    if (warm_lanes.empty()) throw std::invalid_argument("warm_lanes is empty");
+    warm_ = true;
+    warm_lanes_ = warm_lanes;
+  }
 
   // Host pointers; blocks until the results are back.
   void Solve(int batch, const FCCQPBatchProblem& p) {
     const size_t B = (size_t)batch, n = (size_t)n_, m = (size_t)m_, nc = (size_t)nc_;
+    if (!warm_lanes_.empty() && warm_lanes_.size() != B)
+      throw std::invalid_argument("warm_lanes has " + std::to_string(warm_lanes_.size()) + " entries, the batch " +
+                                  std::to_string(batch));
     const bool carry = warm_ && sol_.batch == batch;    // like a never-solved FCCQP, a fresh lane starts from zero
     if (!carry) { sol_.z.assign(B * n, 0.0); mu_x_.assign(B * n, 0.0); mu_c_.assign(B * nc, 0.0); }
     sol_.batch = batch;
@@ -274,6 +285,7 @@ class FCCQPBatch {
     double secs = 0.0;
     d.device_seconds = &secs;
     d.structure = structure_;
+    d.warm_lanes = warm_lanes_.empty() ? nullptr : warm_lanes_.data();
     const int rc = devices_.size() > 1 ? fccqp_batch_solve_multi(&d, devices_.data(), (int32_t)devices_.size())
                                        : fccqp_batch_solve(&d);
     if (rc == FCCQP_E_INVALID) throw std::invalid_argument(fccqp_last_error());
@@ -284,8 +296,10 @@ class FCCQPBatch {
 
   // Device pointers; enqueued on io.stream and NOT waited for unless device_seconds is given (then the call
   // returns after the kernels and *device_seconds holds their time).  io.x / mu_x / mu_lambda_c are the carried
-  // state when set_warm_start(true).
-  void SolveDevice(int batch, const FCCQPBatchDeviceIO& io, double* device_seconds = nullptr) {
+  // state when set_warm_start(true).  warm_lanes: optional DEVICE [batch] mask, one byte per lane, that replaces
+  // set_warm_start for this call (lane i warm where warm_lanes[i] != 0; read by the kernels when they run).
+  void SolveDevice(int batch, const FCCQPBatchDeviceIO& io, double* device_seconds = nullptr,
+                   const uint8_t* warm_lanes = nullptr) {
     fccqp_batch_desc d{};
     d.abi_version = FCCQP_ABI_VERSION; d.batch = batch; d.n = n_; d.m = m_; d.nc = nc_; d.lambda_c_start = lcs_;
     d.device = io.device; d.memory_space = FCCQP_MEM_DEVICE; d.precision = FCCQP_PRECISION_FP64; d.warm_start = warm_ ? 1 : 0;
@@ -304,6 +318,7 @@ class FCCQPBatch {
     d.stream = io.stream;
     d.device_seconds = device_seconds;
     d.structure = structure_;
+    d.warm_lanes = warm_lanes;
     const int rc = fccqp_batch_solve(&d);
     if (rc == FCCQP_E_INVALID) throw std::invalid_argument(fccqp_last_error());
     if (rc != FCCQP_OK) throw std::runtime_error(fccqp_last_error());
@@ -317,6 +332,7 @@ class FCCQPBatch {
   const int n_, m_, nc_, lcs_, device_;
   fccqp_options opt_{};
   bool warm_ = false;
+  std::vector<uint8_t> warm_lanes_;   // per-lane warm start of the host Solve (empty: warm_ for every lane)
   int structure_ = FCCQP_STRUCTURE_AUTO;
   std::vector<int32_t> devices_;
   FCCQPBatchSolution sol_;

@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define FCCQP_ABI_VERSION 4
+#define FCCQP_ABI_VERSION 5
 
 typedef enum fccqp_error {
   FCCQP_OK = 0,
@@ -222,7 +222,8 @@ typedef struct fccqp_batch_desc {
   int32_t memory_space;    /* fccqp_memory_space: where EVERY pointer below lives */
   int32_t precision;       /* fccqp_precision */
   int32_t warm_start;      /* 0: cold (pre-solve, duals zeroed; fcc_qp.cpp:136-139,159-178)
-                              1: warm: x/mu_x/mu_lambda_c are read as the carried state      */
+                              1: warm: x/mu_x/mu_lambda_c are read as the carried state
+                              (ignored when warm_lanes is set)                                */
   fccqp_options options;
 
   /* inputs (float32 arrays behind the same pointer types when precision = FCCQP_PRECISION_FP32_DATA);
@@ -238,7 +239,7 @@ typedef struct fccqp_batch_desc {
   const double* ub;       int64_t ub_batch_stride;
 
   /* in/out state, dense [B,n] / [B,n] / [B,nc].  x is also the solution z.
-   * mu_x / mu_lambda_c may be NULL for cold solves whose duals are not needed. */
+   * mu_x / mu_lambda_c may be NULL for cold solves (warm_start = 0, no warm_lanes) whose duals are not needed. */
   double* x;
   double* mu_x;
   double* mu_lambda_c;
@@ -256,6 +257,19 @@ typedef struct fccqp_batch_desc {
   double* device_seconds;  /* optional HOST pointer: kernel time by CUDA events (forces a sync) */
   int32_t structure;       /* enum fccqp_structure, optionally | FCCQP_STRUCTURE_REFINE; 0 = AUTO */
   int32_t struct_caps[3];  /* FCCQP_STRUCTURE_CAPS only */
+
+  /* Per-lane cold or warm start (ABI version 5): NULL = warm_start decides for every lane.  Otherwise a dense [B]
+   * array, one byte per lane in the call's memory_space, and it alone decides: lane i is solved exactly as a reference
+   * object after set_warm_start(warm_lanes[i] != 0) -- a warm lane from its carried x / mu_x / mu_lambda_c (pre-solve only
+   * when equality-constrained, fcc_qp.cpp:159), a cold lane with the pre-solve and zero duals, its state ignored on
+   * input -- and no lane's result depends on the other lanes.  x, mu_x and mu_lambda_c (nc > 0) must then be non-NULL.
+   * FCCQP_MEM_DEVICE: read on the device when the call runs (no synchronisation), so a captured CUDA graph sees the
+   * values written into it before each replay (environments of a vectorised simulation that reset at different
+   * steps).  FCCQP_MEM_HOST: staged with every chunk of the batch.  One small kernel splits the lanes into a cold and
+   * a warm list; the call then runs the launches of a cold call of the whole batch over the cold list and those of a
+   * warm call over the warm list, with the same kernels, so every lane returns the bits of a uniform call (on the
+   * shared-structure path up to the last bits that already depend there on which QPs a thread block solves first). */
+  const uint8_t* warm_lanes;
 } fccqp_batch_desc;
 
 int fccqp_batch_solve(const fccqp_batch_desc* desc);
