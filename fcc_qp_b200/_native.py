@@ -120,7 +120,7 @@ EXPORTS = [
     "fccqp_release_workspaces", "fccqp_kernel_launch_count", "fccqp_last_launch_info",
     "fccqp_alloc_pinned", "fccqp_free_pinned", "fccqp_wbc_assemble",
     "fccqp_last_struct_info", "fccqp_set_structure", "fccqp_batch_solve_multi", "fccqp_measure_fp64_peak",
-    "fccqp_polish_prepare", "fccqp_polish_finish",
+    "fccqp_polish_prepare", "fccqp_polish_finish", "fccqp_batch_solve_rho", "fccqp_batch_solve_multi_rho",
 ]
 
 _lib = None
@@ -153,6 +153,8 @@ def lib() -> C.CDLL:
     L.fccqp_set_warm_state.argtypes = [C.c_void_p, _dp, _dp, _dp]
     L.fccqp_batch_solve.argtypes = [C.POINTER(BatchDesc)]
     L.fccqp_batch_solve_multi.argtypes = [C.POINTER(BatchDesc), C.POINTER(C.c_int32), C.c_int32]
+    L.fccqp_batch_solve_rho.argtypes = [C.POINTER(BatchDesc), C.c_void_p]
+    L.fccqp_batch_solve_multi_rho.argtypes = [C.POINTER(BatchDesc), C.c_void_p, C.POINTER(C.c_int32), C.c_int32]
     L.fccqp_kernel_launch_count.restype = C.c_int64
     L.fccqp_measure_fp64_peak.argtypes = [C.c_int, C.POINTER(C.c_double)]
     L.fccqp_last_launch_info.argtypes = [_ip, _ip, _ip, _ip]

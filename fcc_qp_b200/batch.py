@@ -102,6 +102,7 @@ class FCCQPBatch:
         self._caps = None
         self.warm_start = False
         self.warm_lanes = None  # per-lane mask of set_warm_start (None: warm_start holds for every lane)
+        self.rho_lanes = None   # per-lane rho of set_rho, read and written by every Solve (None: options.rho for every lane)
         self.time_kernel = True
         self._state = None     # (x, mu_x, mu_c) arrays / tensors
         self._host_out = None  # page-locked output buffers of the numpy path
@@ -111,10 +112,56 @@ class FCCQPBatch:
         nat.lib()              # fail loudly if the CUDA library is not built
 
     # --- same setters as the reference object (src/fcc_qp.hpp:75-91)
-    def set_rho(self, rho: float):
-        if not rho > 0:
-            raise ValueError("rho must be > 0")
-        self.options.rho = float(rho)
+    def set_rho(self, rho):
+        """A float: one rho for every lane, as on the reference object (clears a per-lane array).  Or a per-lane ``[B]``
+        float64 array: lane i is solved as a reference object after ``set_rho(rho[i])``, and every ``Solve`` overwrites
+        rho[i] with the rho lane i ended with -- under adaptive rho the next warm ``Solve`` continues from it, with the
+        carried duals scaled for it (fccqp_batch_solve_rho in include/fccqp.h).  A numpy array for numpy batches, a
+        contiguous CUDA tensor on the batch's device for device batches: kept, not copied, and read and written in place,
+        so a captured CUDA graph carries it from replay to replay.  Entries of a device tensor that are not finite or
+        not > 0 end their lane with status NUMERICAL_ISSUE and n_iter 0."""
+        if _is_torch(rho):
+            import torch
+            if rho.dtype != torch.float64 or rho.dim() != 1:
+                raise ValueError("a per-lane rho must be a 1-D float64 tensor")
+            if rho.device.type != "cuda":
+                raise ValueError("a torch per-lane rho must be a CUDA tensor (numpy arrays go with numpy batches)")
+            if rho.numel() > 1 and rho.stride(0) != 1:
+                raise ValueError("a per-lane rho must be contiguous (it is read and written in place)")
+            self.rho_lanes = rho
+        elif isinstance(rho, np.ndarray) and rho.ndim > 0:
+            if rho.dtype != np.float64 or rho.ndim != 1:
+                raise ValueError("a per-lane rho must be a 1-D float64 array")
+            if not rho.flags.c_contiguous or not rho.flags.writeable:
+                raise ValueError("a per-lane rho must be a contiguous, writeable array (it is written in place)")
+            self._check_rho_values(rho)
+            self.rho_lanes = rho
+        else:
+            if not rho > 0:
+                raise ValueError("rho must be > 0")
+            self.options.rho = float(rho)
+            self.rho_lanes = None
+
+    @staticmethod
+    def _check_rho_values(rho: np.ndarray):
+        if not np.all(np.isfinite(rho) & (rho > 0)):
+            raise ValueError("every per-lane rho must be finite and > 0")
+
+    def _rho_ptr(self, B: int, dev) -> int:
+        """Pointer of the per-lane rho for a batch of B lanes (0: none); refuses an array that does not fit the call."""
+        r = self.rho_lanes
+        if r is None:
+            return 0
+        if r.shape[0] != B:
+            raise ValueError(f"per-lane rho has {r.shape[0]} lanes, the batch {B}")
+        if dev is None:
+            if _is_torch(r):
+                raise ValueError("numpy batch with a torch per-lane rho: pass a numpy array")
+            self._check_rho_values(r)
+            return r.ctypes.data
+        if not _is_torch(r) or r.device != dev:
+            raise ValueError(f"device batch on {dev} needs a CUDA per-lane rho on the same device")
+        return r.data_ptr()
 
     def set_max_iter(self, n: int):
         if not n > 0:
@@ -277,6 +324,7 @@ class FCCQPBatch:
         n, m, nc = self.n, self.m, self.nc
         warm = self.warm_start
         mask = self._mask_ptr(B, None)
+        rho = self._rho_ptr(B, None)
         st = self._state
         # Outputs live in solver-owned page-locked buffers (true asynchronous D2H), reused from
         # call to call; x doubles as the carried warm-start state, exactly like the reference's x_.
@@ -315,9 +363,9 @@ class FCCQPBatch:
         t0 = time.perf_counter()
         if self.devices is not None:
             devs = (C.c_int32 * len(self.devices))(*self.devices)
-            nat.check(nat.lib().fccqp_batch_solve_multi(C.byref(d), devs, len(self.devices)))
+            nat.check(nat.lib().fccqp_batch_solve_multi_rho(C.byref(d), rho or None, devs, len(self.devices)))
         else:
-            nat.check(nat.lib().fccqp_batch_solve(C.byref(d)))
+            nat.check(nat.lib().fccqp_batch_solve_rho(C.byref(d), rho or None))
         wall = time.perf_counter() - t0
         self._state = (x, mux, muc)
         # zero_copy_outputs: z and the details are views of the solver-owned page-locked buffers,
@@ -348,6 +396,7 @@ class FCCQPBatch:
         b, b_eq, mu, lb, ub = map(cont, (b, b_eq, mu, lb, ub))
         warm = self.warm_start
         mask = self._mask_ptr(B, dev)
+        rho = self._rho_ptr(B, dev)
         st = self._state
         # Outputs and carried state live in solver-owned device tensors, allocated once per (B, device) and reused
         # from call to call (nothing is allocated inside a steady-state Solve).  A cold solve ignores the state
@@ -400,12 +449,12 @@ class FCCQPBatch:
             d.device_seconds = C.pointer(secs)
         t0 = time.perf_counter()
         with torch.cuda.device(dev):
-            nat.check(nat.lib().fccqp_batch_solve(C.byref(d)))
+            nat.check(nat.lib().fccqp_batch_solve_rho(C.byref(d), rho or None))
         wall = time.perf_counter() - t0
         self._after_device_call(B, probed)
         # keep the inputs alive until the (possibly asynchronous) launch has consumed them
         self._keepalive = (Q, b, A_eq, b_eq, mu, lb, ub)
-        self._mask_keepalive = self.warm_lanes
+        self._mask_keepalive = (self.warm_lanes, self.rho_lanes)
         self._state = (x, mux, muc)
         # zero_copy_outputs: z and the details are the solver-owned tensors themselves, valid until the next Solve();
         # default: independent copies, like FCCQP::GetSolution
@@ -502,9 +551,23 @@ class FCCQPBatchCpp:
         self._out = None
         self._sol = None
         self._mask = None      # torch per-lane mask of the device path (SolveDLPack's warm_lanes)
+        self._rho = None       # torch per-lane rho of the device path (SolveDLPack's rho)
         self.time_kernel = False
 
-    def set_rho(self, rho): self._s.set_rho(float(rho))
+    def set_rho(self, rho):
+        """A float, or a per-lane [B] rho: numpy / sequence for host stacks (the C++ object keeps a copy and writes the
+        final rho into it: ``rho_lanes``), a contiguous CUDA float64 tensor for device ones (read and written in place)."""
+        self._rho = None
+        if _is_torch(rho):
+            self._rho = rho
+        elif isinstance(rho, (list, tuple)) or (isinstance(rho, np.ndarray) and rho.ndim > 0):
+            self._s.set_rho(np.asarray(rho, dtype=np.float64))
+        else:
+            self._s.set_rho(float(rho))
+
+    @property
+    def rho_lanes(self):
+        return self._rho if self._rho is not None else self._s.rho_lanes
     def set_max_iter(self, n): self._s.set_max_iter(int(n))
 
     def set_warm_start(self, warm_start):
@@ -546,8 +609,8 @@ class FCCQPBatchCpp:
         with torch.cuda.device(dev):
             secs = self._s.SolveDLPack(Q, b, A_eq, b_eq, mu, lb, ub, *o,
                                        stream=torch.cuda.current_stream(dev).cuda_stream, time_kernel=self.time_kernel,
-                                       warm_lanes=self._mask)
-        self._keepalive = (Q, b, A_eq, b_eq, mu, lb, ub, self._mask)
+                                       warm_lanes=self._mask, rho=self._rho)
+        self._keepalive = (Q, b, A_eq, b_eq, mu, lb, ub, self._mask, self._rho)
         x, _, _, n_iter, status, det = o
         self._sol = BatchSolution(BatchDetails(n_iter, det[0], det[1], det[2], det[3], status, secs, secs), x)
 

@@ -300,6 +300,17 @@ __global__ void __launch_bounds__(256) warm_split_kernel(const uint8_t* __restri
   if (warm) warm_list[base_w + __popc(bw & below)] = qp;
 }
 
+// Per-lane rho (SolveParams::rho_lanes) and a two-stage structure solve: the first stage never reads rho, so a cold lane
+// whose entry the solve cannot take may finish there.  Its n_iter and status are set here, after the launches, to what
+// every other kernel path reports for it.
+__global__ void __launch_bounds__(256) rho_invalid_kernel(const double* __restrict__ rho_lanes, const int B,
+                                                          int* __restrict__ n_iter, int* __restrict__ status) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= B || fccqp::rho_valid(rho_lanes[i])) return;
+  if (n_iter) n_iter[i] = 0;
+  if (status) status[i] = FCCQP_STATUS_NUMERICAL_ISSUE;
+}
+
 // Allocates the scratch of a call.  FCCQP_SCHEDULE_LPT, when the batch holds at least two QPs for each of the `slots`
 // that run at once: QPs whose previous solve ran long go to the front of the processing order (p.index_list).
 // warm_lanes (device memory): the processing order is split into the cold and the warm list (Scratch::cold_list / warm_list).
@@ -402,7 +413,9 @@ int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool 
   constexpr int kW = 4;
   const int N = p.n + p.m;
   const size_t smem = (size_t)kW * N * (N | 1) * (f32 ? sizeof(float) : sizeof(double));
-  KernelFn fn = f32 ? (KernelFn)fccqp::fccqp_warp_kernel<kW, 6, float> : (KernelFn)fccqp::fccqp_warp_kernel<kW, 6, double>;
+  using fccqp::fccqp_warp_kernel;
+  KernelFn fn = p.rho_lanes ? (f32 ? (KernelFn)fccqp_warp_kernel<kW, 6, float, true> : (KernelFn)fccqp_warp_kernel<kW, 6, double, true>)
+                            : (f32 ? (KernelFn)fccqp_warp_kernel<kW, 6, float> : (KernelFn)fccqp_warp_kernel<kW, 6, double>);
   // (measured, tools/bench_small.py: 6 CTAs x 4 warps at 80 registers beats 8 x 4 at 64 and 4 x 4 at 128 on every shape but n = 6;
   //  float instance, tools/fp32_occ.py: 6 / 8 / 10 / 12 CTAs -> 82.7 / 78.5 / 71.4 / 70.5 M QP/s at n = 6, 22.4 / 23.1 / 21.1 / 21.7 at n = 24)
   LaunchInfo li;
@@ -501,7 +514,7 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   if (sl.N8c + 8 > p.lay.N8 || sl.bytes() > (size_t)ctx.max_smem_optin) return kNotApplicable;
   // threads >= max(n, padded reduced KKT size), at most 256 since the reduced size is below p.lay.N8
   const int need = p.n > sl.N8c ? p.n : sl.N8c;
-  const bool adapt = p.adapt_k > 0, refine = p.struct_refine != 0;
+  const bool adapt = p.adapt_k > 0 || p.rho_lanes, refine = p.struct_refine != 0;
   int threads;
   KernelFn first;
   if (need <= 64) { threads = 64; first = struct_first_instance<64, 8>(refine); }
@@ -568,6 +581,10 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
 #ifdef FCCQP_DEV
   if ((rc = prof.report(stream, split ? "struct resume" : "struct", kStructPhases, p.B, li.grid))) return rc;
 #endif
+  if (split && p.rho_lanes) {
+    rho_invalid_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.rho_lanes, p.B, p.n_iter, p.status);
+    CUDA_TRY(cudaGetLastError());
+  }
   fccqp::SolveParams b = p;
   if (s.mask) b.warm = 0;
   b.count_dev = a.pending_count;
@@ -575,7 +592,7 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   b.work_counter = s.w + Scratch::kWork2;
   general<<<gli.grid, gli.block, gli.smem, stream>>>(b);
   CUDA_TRY(cudaGetLastError());
-  int launches = split ? 3 : 2;
+  int launches = (split ? 3 : 2) + (split && p.rho_lanes ? 1 : 0);
   if (s.mask) {   // the warm QPs the full kernel handed over
     fccqp::SolveParams bw = p;
     bw.warm = 1;
@@ -619,6 +636,8 @@ int launch_general(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, co
 // precision: fccqp_precision of the call (FP32_DATA and FP32: float32 problem data behind the pointers of p; FP32: FP32
 // arithmetic too where a kernel for it exists -- the warp kernel -- and FP32_DATA's FP64 arithmetic otherwise)
 // warm_lanes: optional per-lane mask in device memory (fccqp_batch_desc::warm_lanes); p.warm is then ignored.
+// p.rho_lanes: optional per-lane rho in device memory (fccqp_batch_solve_rho); such calls run the instances that keep rho
+// per QP (kAdapt, and kRhoLanes of the warp kernel), never the shared-structure path (its cached factorization has one rho).
 int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int precision, const StructHint& hint,
                  const uint8_t* warm_lanes = nullptr) {
   if (p.B == 0) return FCCQP_OK;
@@ -635,16 +654,16 @@ int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int 
 
   // one CTA per QP; float32 problem data take the general kernel's widening instance, same geometry
   const int threads = p.lay.N8 <= 128 ? 128 : 256;
-  KernelFn general = pick_kernel(threads, false, f32, p.adapt_k > 0);
+  KernelFn general = pick_kernel(threads, false, f32, p.adapt_k > 0 || p.rho_lanes);
   LaunchInfo li;
   Scratch s;
   if ((rc = geometry(ctx, general, threads, p.lay.bytes(), p.B, 1, &li)) ||
       (rc = begin_call(p, stream, hint.lpt, (long long)li.ctas_per_sm * ctx.num_sms, &s, warm_lanes)))
     return rc;
   // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs.  Not with
-  // adaptive rho: a lane that moves its rho needs its own rho-KKT factorization, so those batches take the
+  // adaptive or per-lane rho: a lane with its own rho needs its own rho-KKT factorization, so those batches take the
   // structure-exploiting or general kernel (both read Q and A_eq through the batch stride).
-  if (!sw.no_shared && !f32 && p.adapt_k == 0 && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) &&
+  if (!sw.no_shared && !f32 && p.adapt_k == 0 && !p.rho_lanes && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) &&
       p.B >= 4 * li.ctas_per_sm * ctx.num_sms)
     return launch_shared(ctx, p, stream, s);
   if (!f32 && hint.mode != FCCQP_STRUCTURE_DENSE && p.m > 0 &&
@@ -1033,8 +1052,20 @@ static int validate_desc(const fccqp_batch_desc* d) {
   return FCCQP_OK;
 }
 
-int fccqp_batch_solve(const fccqp_batch_desc* desc) {
+// A host-memory per-lane rho array is checked before anything runs (a device one lane by lane in the kernels).
+static int validate_rho(const fccqp_batch_desc* d, const double* rho) {
+  if (!rho || d->memory_space != FCCQP_MEM_HOST) return FCCQP_OK;
+  for (int i = 0; i < d->batch; ++i)
+    if (!(rho[i] > 0.0 && std::isfinite(rho[i])))
+      return fail(FCCQP_E_INVALID, "rho[%d] = %g: every per-lane rho must be finite and > 0", i, rho[i]);
+  return FCCQP_OK;
+}
+
+int fccqp_batch_solve(const fccqp_batch_desc* desc) { return fccqp_batch_solve_rho(desc, nullptr); }
+
+int fccqp_batch_solve_rho(const fccqp_batch_desc* desc, double* rho) {
   int rc = validate_desc(desc);
+  if (!rc) rc = validate_rho(desc, rho);
   if (rc) return rc;
   const fccqp_batch_desc& d = *desc;
   DeviceCtx* ctx = nullptr;
@@ -1056,6 +1087,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
     p.x = d.x; p.mu_x = d.mu_x; p.mu_c = d.mu_lambda_c;
     p.n_iter = d.n_iter; p.status = d.status;
     p.res_b = d.res_bounds; p.res_f = d.res_fcone; p.bviol = d.bounds_viol; p.fviol = d.fcone_viol;
+    p.rho_lanes = rho;
     cudaStream_t st = (cudaStream_t)d.stream;
     StructHint hint;
     hint.set(d.structure);
@@ -1112,6 +1144,8 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
   Seg sint = seg(cur, 1, false);  // 2 ints per QP packed in one double slot
   const Seg smask{cur, 1, false};  // per-lane warm mask: one byte per QP
   if (d.warm_lanes) cur += align_up((size_t)B, 256);
+  const Seg srho{cur, 1, false};   // per-lane rho: in and out
+  if (rho) cur += align_up((size_t)B * sizeof(double), 256);
   if (cur > ctx->stage_bytes) {
     if (ctx->stage) CUDA_TRY(cudaFree(ctx->stage));
     ctx->stage = nullptr; ctx->stage_bytes = 0;
@@ -1141,12 +1175,13 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
   CUDA_TRY(cudaStreamSynchronize(s0));
 
   // where do the outputs go?  (page-locked destination: direct DMA; pageable: pinned bounce buffer)
-  void* outs[9] = {d.x, d.mu_x, d.mu_lambda_c, d.n_iter, d.status, d.res_bounds, d.res_fcone, d.bounds_viol, d.fcone_viol};
-  const size_t out_elem[9] = {n * sizeof(double), n * sizeof(double), nc * sizeof(double), sizeof(int), sizeof(int),
-                              sizeof(double), sizeof(double), sizeof(double), sizeof(double)};
-  bool out_pinned[9];
-  size_t out_off[9], hneed = 0;
-  for (int i = 0; i < 9; ++i) {
+  void* outs[10] = {d.x, d.mu_x, d.mu_lambda_c, d.n_iter, d.status, d.res_bounds, d.res_fcone, d.bounds_viol, d.fcone_viol,
+                    rho};
+  const size_t out_elem[10] = {n * sizeof(double), n * sizeof(double), nc * sizeof(double), sizeof(int), sizeof(int),
+                               sizeof(double), sizeof(double), sizeof(double), sizeof(double), sizeof(double)};
+  bool out_pinned[10];
+  size_t out_off[10], hneed = 0;
+  for (int i = 0; i < 10; ++i) {
     out_pinned[i] = true;
     out_off[i] = 0;
     if (!outs[i] || !out_elem[i]) continue;
@@ -1192,6 +1227,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
       if ((rc = h2d(sx, d.x, 8)) || (rc = h2d(smx, d.mu_x, 8)) || (rc = h2d(smc, d.mu_lambda_c, 8))) return rc;
     }
     if (d.warm_lanes && (rc = h2d(smask, d.warm_lanes, 1))) return rc;
+    if (rho && (rc = h2d(srho, rho, sizeof(double)))) return rc;
     fccqp::SolveParams p = solve_params((int)cnt, n, m, nc, d.lambda_c_start, d.options, d.warm_start != 0);
     auto off = [&](const Seg& s) { return s.shared ? dp(s) : dp(s) + lo * s.per_qp; };
     auto offi = [&](const Seg& s) {   // problem data: element size es
@@ -1208,6 +1244,7 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
     p.n_iter = d_niter + lo; p.status = d_status + lo;
     double* res = dp(sres);
     p.res_b = res + lo; p.res_f = res + (size_t)B + lo; p.bviol = res + 2 * (size_t)B + lo; p.fviol = res + 3 * (size_t)B + lo;
+    p.rho_lanes = rho ? dp(srho) + lo : nullptr;
     rc = launch_solve(*ctx, p, st, d.precision, hint,
                       d.warm_lanes ? reinterpret_cast<const uint8_t*>(base + smask.off) + lo : nullptr);
     if (rc) return rc;
@@ -1233,7 +1270,8 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
         (rc = d2h(5, d.res_bounds, p.res_b, sizeof(double))) ||
         (rc = d2h(6, d.res_fcone, p.res_f, sizeof(double))) ||
         (rc = d2h(7, d.bounds_viol, p.bviol, sizeof(double))) ||
-        (rc = d2h(8, d.fcone_viol, p.fviol, sizeof(double))))
+        (rc = d2h(8, d.fcone_viol, p.fviol, sizeof(double))) ||
+        (rc = d2h(9, rho, p.rho_lanes, sizeof(double))))
       return rc;
     CUDA_TRY(cudaEventRecord(ctx->chunk_ev[c], st));
   }
@@ -1257,7 +1295,12 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc) {
 // and runs the single-device host path on its own host thread: staging buffers, streams, H2D / solve / D2H
 // pipeline and structure classification are per device.
 int fccqp_batch_solve_multi(const fccqp_batch_desc* desc, const int32_t* devices, int32_t n_devices) {
+  return fccqp_batch_solve_multi_rho(desc, nullptr, devices, n_devices);
+}
+
+int fccqp_batch_solve_multi_rho(const fccqp_batch_desc* desc, double* rho, const int32_t* devices, int32_t n_devices) {
   int rc = validate_desc(desc);
+  if (!rc) rc = validate_rho(desc, rho);
   if (rc) return rc;
   if (!devices || n_devices < 1) return fail(FCCQP_E_INVALID, "devices / n_devices");
   if (desc->memory_space != FCCQP_MEM_HOST)
@@ -1316,7 +1359,7 @@ int fccqp_batch_solve_multi(const fccqp_batch_desc* desc, const int32_t* devices
     if (d.res_fcone) s.res_fcone = d.res_fcone + lo;
     if (d.bounds_viol) s.bounds_viol = d.bounds_viol + lo;
     if (d.fcone_viol) s.fcone_viol = d.fcone_viol + lo;
-    return fccqp_batch_solve(&s);
+    return fccqp_batch_solve_rho(&s, rho ? rho + lo : nullptr);
   };
   auto shard = [&](int r) {
     for (;;) {

@@ -203,9 +203,19 @@ struct SolveParams {
   int struct_refine;           // that kernel: one step of iterative refinement on the cold pre-solve
   double* op_scratch;          // that kernel: per-CTA global scratch of the full-space operator of long-running QPs
   long long op_stride;         //   doubles per CTA
-  int* resume_list;            // its first stage (kStructFirst): QPs that keep iterating
-  unsigned int* resume_count;  //   their count
+  // One slot, read by disjoint instances: resume_list only by the first stage of a structure solve, rho_lanes only by the
+  // instances that keep rho per QP (kAdapt, kRhoLanes), which never run as a first stage.  Sharing it keeps the size of
+  // SolveParams, so kernels with parameters after it (the structure probe) keep their code.
+  union {
+    int* resume_list;          // its first stage (kStructFirst): QPs that keep iterating
+    double* rho_lanes;         // optional [B] per-lane rho (fccqp_batch_solve_rho): the lane's starting rho, overwritten
+                               // with the rho it ended with
+  };
+  unsigned int* resume_count;  //   first stage: the count of resume_list
 };
+
+// A per-lane rho entry the solve accepts (the single-problem object's set_rho refuses the others).
+__device__ __forceinline__ bool rho_valid(const double rho) { return rho > 0.0 && isfinite(rho); }
 
 __device__ __forceinline__ double warp_max(double v) {
 #pragma unroll
@@ -1180,6 +1190,18 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
     const int qslot = *s_work;
     if (qslot >= Btot) break;
     const int qp = p.index_list ? p.index_list[qslot] : qslot;
+    // per-lane rho (kAdapt instances only): the lane's starting rho, and at exit the one it ended with.  An entry the
+    // solve cannot take ends the lane here with NUMERICAL_ISSUE, its state and the entry untouched.
+    double rho_qp = p.rho;
+    if constexpr (kAdapt) {
+      if (p.rho_lanes) {
+        rho_qp = p.rho_lanes[qp];
+        if (!rho_valid(rho_qp)) {
+          if (tid == 0) store_details(p, qp, 0, true, 0.0, 0.0, 0.0, 0.0, 0ull, clock64());
+          continue;
+        }
+      }
+    }
 
     const double* Qg = p.Q + (size_t)qp * p.q_bs;
     const double* Ag = p.A + (size_t)qp * p.a_bs;
@@ -1248,6 +1270,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
       double v_xbase = 0.0;        // its x_base entry of row t
       double rhs0 = 0.0;   // pass-0 right-hand side of row t
       double rho_cur = p.rho;      // (changes only with the adaptive-rho extension, SolveParams::adapt_k)
+      if constexpr (kAdapt) rho_cur = rho_qp;
 
 #pragma unroll 1
       for (int iter = 0; iter < iters; ++iter) {
@@ -1586,6 +1609,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
           const double rho_new = cta_rebalance_rho(rx, rc, dz, rho_cur, v_mux, muc + 3 * t, t < nc / 3, red, parity);
           if (rho_new != rho_cur) {
             rho_cur = rho_new;
+            rho_qp = rho_new;
             factored = false;
             full_inverse = false;
           }
@@ -1620,6 +1644,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_solve_kernel(const
     }
     if (p.mu_c && t < nc) p.mu_c[(size_t)qp * nc + t] = muc[t];
     if (tid == 0) store_details(p, qp, n_iter, bad, res_x, res_c, bv, fv, fact_cycles, t_start);
+    if constexpr (kAdapt) {
+      if (p.rho_lanes && tid == 0) p.rho_lanes[qp] = rho_qp;
+    }
     FCCQP_PROF(10);
     FCCQP_PROF_COUNT(14);
   }

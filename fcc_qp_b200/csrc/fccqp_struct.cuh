@@ -942,6 +942,17 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
     const int qp = s_work[0];
     if (qp >= p.B) break;
     const bool resume = !kFirst && p.count_dev != nullptr;
+    // per-lane rho (kAdapt instances only; the first stage never reaches the rho-KKT system): as in fccqp_solve_kernel
+    double rho_qp = p.rho;
+    if constexpr (kAdapt) {
+      if (p.rho_lanes) {
+        rho_qp = p.rho_lanes[qp];
+        if (!rho_valid(rho_qp)) {
+          if (tid == 0) store_details(p, qp, 0, true, 0.0, 0.0, 0.0, 0.0, 0ull, clock64());
+          continue;
+        }
+      }
+    }
     const double* Qg = p.Q + (size_t)qp * p.q_bs;
     const double* Ag = p.A + (size_t)qp * p.a_bs;
     FCCQP_PROF(0);
@@ -1004,6 +1015,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
       }
       const int iters = pass == 0 ? 1 : p.max_iter;
       double shift = pass == 0 ? 0.0 : p.rho;   // (rho of pass 1 changes only with the adaptive-rho extension)
+      if constexpr (kAdapt) shift = pass == 0 ? 0.0 : rho_qp;
       // In the ADMM pass the zero-cost variables have h = rho > 0 like everybody else: they are eliminated too
       // (keeping them as a trailing block with a rho-sized pivot costs three digits; tools/proto), so the
       // reduced system of pass 1 is [R, constraints] only.
@@ -1294,6 +1306,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
           const double rho_new = cta_rebalance_rho(rx, rc, dz, shift, v_mux, muc + 3 * t, t < nc / 3, red, parity);
           if (rho_new != shift) {
             shift = rho_new;
+            rho_qp = rho_new;
             hi = (ve.type == VT_DP || ve.type == VT_D1) ? 1.0 / (ve.qd + shift) : 0.0;
             factored = false; full_inverse = false; full_op = false;
           }
@@ -1323,6 +1336,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) fccqp_struct_kernel(cons
     }
     if (p.mu_c && t < nc) p.mu_c[(size_t)qp * nc + t] = muc[t];
     if (tid == 0) store_details(p, qp, n_iter, bad, res_x, res_c, bv, fv, fact_cycles, t_start);
+    if constexpr (kAdapt) {
+      if (p.rho_lanes && tid == 0) p.rho_lanes[qp] = rho_qp;
+    }
     FCCQP_PROF(9);
     FCCQP_PROF_COUNT(14);
   }

@@ -98,7 +98,8 @@ __device__ __noinline__ T warp_solve(const T* __restrict__ K, const int N, const
   return y;
 }
 
-template <int kWarps, int kMinBlocks, typename T>
+// kRhoLanes: the per-lane rho of SolveParams::rho_lanes compiled in (a separate instance: the default path carries none of it)
+template <int kWarps, int kMinBlocks, typename T, bool kRhoLanes = false>
 __global__ void __launch_bounds__(32 * kWarps, kMinBlocks) fccqp_warp_kernel(const SolveParams p) {
   extern __shared__ __align__(16) double smem_d[];
   T* const smem = reinterpret_cast<T*>(smem_d);
@@ -130,6 +131,14 @@ __global__ void __launch_bounds__(32 * kWarps, kMinBlocks) fccqp_warp_kernel(con
     const T* const lbg = reinterpret_cast<const T*>(p.lb), *const ubg = reinterpret_cast<const T*>(p.ub);
     const T* const mug = reinterpret_cast<const T*>(p.mu);
     const T rho0 = (T)p.rho, alpha = (T)p.alpha, eps_fcone = (T)p.eps_fcone, eps_bound = (T)p.eps_bound;
+    // per-lane rho: an entry the solve cannot take ends the lane here with NUMERICAL_ISSUE, its state and the entry
+    // untouched (fccqp_solve_kernel); the others start pass 1 below, converted to T at the boundary
+    if constexpr (kRhoLanes) {
+      if (!rho_valid(p.rho_lanes[qp])) {
+        if (lane == 0) store_details(p, qp, 0, true, T(0), T(0), T(0), T(0), 0ull, t_start);
+        continue;
+      }
+    }
 
     // ---------------- vectors: one register per row and vector ----------------
     T v_b = 0, v_lb = 0, v_ub = 0, v_mux = 0, v_xbar = 0, v_x = 0;
@@ -169,6 +178,7 @@ __global__ void __launch_bounds__(32 * kWarps, kMinBlocks) fccqp_warp_kernel(con
       bool factored = false, have_g = false;
       T dinv = 0, rhs0 = 0, v_xbase = 0;
       T rho_cur = rho0;   // (changes only with the adaptive-rho extension)
+      if constexpr (kRhoLanes) rho_cur = (T)p.rho_lanes[qp];
 
 #pragma unroll 1
       for (int iter = 0; iter < iters; ++iter) {
@@ -324,6 +334,9 @@ __global__ void __launch_bounds__(32 * kWarps, kMinBlocks) fccqp_warp_kernel(con
             const T sc = rho_cur / rho_new;
             v_mux *= sc; v_muc *= sc;
             rho_cur = rho_new;
+            // (the lane's entry follows each move, so it ends with the final rho; an entry that never moves is not
+            // written, which T = float would round)
+            if constexpr (kRhoLanes) { if (lane == 0) p.rho_lanes[qp] = (double)rho_new; }
             factored = false;
             have_g = false;
           }

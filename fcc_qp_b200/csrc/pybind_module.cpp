@@ -196,7 +196,18 @@ PYBIND11_MODULE(fcc_qp_solver, m) {
            py::arg("nc"), py::arg("lambda_c_start"), py::arg("device") = 0)
       .def(py::init<int, int, int, int, std::vector<int>>(), py::arg("num_vars"), py::arg("num_equality_constraints"),
            py::arg("nc"), py::arg("lambda_c_start"), py::arg("devices"))
-      .def("set_rho", &FCCQPBatch::set_rho)
+      // a float for every lane, or a per-lane sequence for the host Solve (written back: rho_lanes)
+      .def("set_rho",
+           [](FCCQPBatch& self, const py::object& r) {
+             if (!py::isinstance<py::sequence>(r) && !py::isinstance<py::array>(r)) { self.set_rho(r.cast<double>()); return; }
+             const auto a = py::array_t<double, py::array::c_style | py::array::forcecast>::ensure(r);
+             if (!a || a.ndim() != 1) throw py::value_error("a per-lane rho must be a 1-D sequence");
+             self.set_rho(std::vector<double>(a.data(), a.data() + a.size()));
+           },
+           py::arg("rho"))
+      .def_property_readonly("rho_lanes", [](const FCCQPBatch& self) {
+        return py::array_t<double>((py::ssize_t)self.rho_lanes().size(), self.rho_lanes().data());
+      })
       .def("set_max_iter", &FCCQPBatch::set_max_iter)
       // a bool for every lane, or a per-lane sequence (list, numpy bool / uint8 array) for the host Solve
       .def("set_warm_start",
@@ -250,7 +261,7 @@ PYBIND11_MODULE(fcc_qp_solver, m) {
           [](FCCQPBatch& self, const py::object& Q, const py::object& b, const py::object& A_eq, const py::object& b_eq,
              const py::object& mu, const py::object& lb, const py::object& ub, const py::object& x, const py::object& mu_x,
              const py::object& mu_lambda_c, const py::object& n_iter, const py::object& solve_status, const py::object& details,
-             std::uintptr_t stream, bool time_kernel, const py::object& warm_lanes) {
+             std::uintptr_t stream, bool time_kernel, const py::object& warm_lanes, const py::object& rho) {
             const int n = self.num_vars(), mm = self.num_equality_constraints(), nc = self.num_contact_vars();
             const DevView vb = dev_view(b, "b", kDLFloat, 64, 2);
             if (vb.ndim != 2 || vb.shape[1] != n) throw py::value_error("b must be [B,n]");
@@ -286,14 +297,21 @@ PYBIND11_MODULE(fcc_qp_solver, m) {
                 throw py::value_error("warm_lanes must be a contiguous [B] tensor on the device of the batch");
               mask = static_cast<const uint8_t*>(vm.data);
             }
+            double* rho_lanes = nullptr;   // per-lane rho of this call, [B] float64 on the same device, written back
+            if (!rho.is_none()) {
+              const DevView vr = dev_view(rho, "rho", kDLFloat, 64, 1);
+              if (vr.ndim != 1 || vr.shape[0] != B || (B > 1 && vr.stride[0] != 1) || vr.device != io.device)
+                throw py::value_error("rho must be a contiguous [B] float64 tensor on the device of the batch");
+              rho_lanes = static_cast<double*>(vr.data);
+            }
             double secs = 0.0;
             {
               py::gil_scoped_release release;
-              self.SolveDevice(B, io, time_kernel ? &secs : nullptr, mask);
+              self.SolveDevice(B, io, time_kernel ? &secs : nullptr, mask, rho_lanes);
             }
             return secs;
           },
           py::arg("Q"), py::arg("b"), py::arg("A_eq"), py::arg("b_eq"), py::arg("friction_coeffs"), py::arg("lb"), py::arg("ub"),
           py::arg("x"), py::arg("mu_x"), py::arg("mu_lambda_c"), py::arg("n_iter"), py::arg("solve_status"), py::arg("details"),
-          py::arg("stream") = 0, py::arg("time_kernel") = false, py::arg("warm_lanes") = py::none());
+          py::arg("stream") = 0, py::arg("time_kernel") = false, py::arg("warm_lanes") = py::none(), py::arg("rho") = py::none());
 }

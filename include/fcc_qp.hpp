@@ -13,6 +13,7 @@
 // below (plain pointers + strides) and z is a std::vector<double>.
 #pragma once
 
+#include <cmath>
 #include <cstddef>
 #include <cstdint>
 #include <stdexcept>
@@ -240,7 +241,22 @@ class FCCQPBatch {
   }
   // fccqp_structure (| FCCQP_STRUCTURE_REFINE) of the batched calls; default FCCQP_STRUCTURE_AUTO
   void set_structure(int structure) { structure_ = structure; }
-  void set_rho(double rho) { if (!(rho > 0)) throw std::invalid_argument("rho must be > 0"); opt_.rho = rho; }
+  // One rho for every lane (clears a per-lane rho), as on FCCQP.
+  void set_rho(double rho) {
+    if (!(rho > 0)) throw std::invalid_argument("rho must be > 0");
+    opt_.rho = rho;
+    rho_lanes_.clear();
+  }
+  // Per lane (fccqp_batch_solve_rho): lane i of the next host Solve is solved as an FCCQP after set_rho(rho_lanes[i]),
+  // and the vector, owned by this object, then holds the rho each lane ended with (rho_lanes()): with adaptive rho the
+  // next warm Solve continues from it.  One entry per lane of that Solve, each finite and > 0.
+  void set_rho(const std::vector<double>& rho_lanes) {
+    if (rho_lanes.empty()) throw std::invalid_argument("rho_lanes is empty");
+    for (double r : rho_lanes)
+      if (!(r > 0 && std::isfinite(r))) throw std::invalid_argument("every per-lane rho must be finite and > 0");
+    rho_lanes_ = rho_lanes;
+  }
+  const std::vector<double>& rho_lanes() const { return rho_lanes_; }
   void set_max_iter(int n) { if (n <= 0) throw std::invalid_argument("max_iter must be > 0"); opt_.max_iter = n; }
   void set_options(FCCQPOptions o) {
     opt_.max_iter = o.max_iter; opt_.rho = o.rho; opt_.eps_fcone = o.eps_fcone; opt_.eps_bound = o.eps_bound;
@@ -260,6 +276,9 @@ class FCCQPBatch {
     const size_t B = (size_t)batch, n = (size_t)n_, m = (size_t)m_, nc = (size_t)nc_;
     if (!warm_lanes_.empty() && warm_lanes_.size() != B)
       throw std::invalid_argument("warm_lanes has " + std::to_string(warm_lanes_.size()) + " entries, the batch " +
+                                  std::to_string(batch));
+    if (!rho_lanes_.empty() && rho_lanes_.size() != B)
+      throw std::invalid_argument("rho_lanes has " + std::to_string(rho_lanes_.size()) + " entries, the batch " +
                                   std::to_string(batch));
     const bool carry = warm_ && sol_.batch == batch;    // like a never-solved FCCQP, a fresh lane starts from zero
     if (!carry) { sol_.z.assign(B * n, 0.0); mu_x_.assign(B * n, 0.0); mu_c_.assign(B * nc, 0.0); }
@@ -286,8 +305,9 @@ class FCCQPBatch {
     d.device_seconds = &secs;
     d.structure = structure_;
     d.warm_lanes = warm_lanes_.empty() ? nullptr : warm_lanes_.data();
-    const int rc = devices_.size() > 1 ? fccqp_batch_solve_multi(&d, devices_.data(), (int32_t)devices_.size())
-                                       : fccqp_batch_solve(&d);
+    double* rho = rho_lanes_.empty() ? nullptr : rho_lanes_.data();
+    const int rc = devices_.size() > 1 ? fccqp_batch_solve_multi_rho(&d, rho, devices_.data(), (int32_t)devices_.size())
+                                       : fccqp_batch_solve_rho(&d, rho);
     if (rc == FCCQP_E_INVALID) throw std::invalid_argument(fccqp_last_error());
     if (rc != FCCQP_OK) throw std::runtime_error(fccqp_last_error());
     sol_.solve_time = secs;
@@ -297,9 +317,15 @@ class FCCQPBatch {
   // Device pointers; enqueued on io.stream and NOT waited for unless device_seconds is given (then the call
   // returns after the kernels and *device_seconds holds their time).  io.x / mu_x / mu_lambda_c are the carried
   // state when set_warm_start(true).  warm_lanes: optional DEVICE [batch] mask, one byte per lane, that replaces
-  // set_warm_start for this call (lane i warm where warm_lanes[i] != 0; read by the kernels when they run).
+  // set_warm_start for this call (lane i warm where warm_lanes[i] != 0; read by the kernels when they run).  rho:
+  // optional DEVICE [batch] per-lane rho that replaces the options' rho for this call, read and overwritten in place
+  // with the rho each lane ended with (fccqp_batch_solve_rho).
   void SolveDevice(int batch, const FCCQPBatchDeviceIO& io, double* device_seconds = nullptr,
                    const uint8_t* warm_lanes = nullptr) {
+    SolveDevice(batch, io, device_seconds, warm_lanes, nullptr);
+  }
+  void SolveDevice(int batch, const FCCQPBatchDeviceIO& io, double* device_seconds, const uint8_t* warm_lanes,
+                   double* rho) {
     fccqp_batch_desc d{};
     d.abi_version = FCCQP_ABI_VERSION; d.batch = batch; d.n = n_; d.m = m_; d.nc = nc_; d.lambda_c_start = lcs_;
     d.device = io.device; d.memory_space = FCCQP_MEM_DEVICE; d.precision = FCCQP_PRECISION_FP64; d.warm_start = warm_ ? 1 : 0;
@@ -319,7 +345,7 @@ class FCCQPBatch {
     d.device_seconds = device_seconds;
     d.structure = structure_;
     d.warm_lanes = warm_lanes;
-    const int rc = fccqp_batch_solve(&d);
+    const int rc = fccqp_batch_solve_rho(&d, rho);
     if (rc == FCCQP_E_INVALID) throw std::invalid_argument(fccqp_last_error());
     if (rc != FCCQP_OK) throw std::runtime_error(fccqp_last_error());
   }
@@ -333,6 +359,7 @@ class FCCQPBatch {
   fccqp_options opt_{};
   bool warm_ = false;
   std::vector<uint8_t> warm_lanes_;   // per-lane warm start of the host Solve (empty: warm_ for every lane)
+  std::vector<double> rho_lanes_;     // per-lane rho of the host Solve, written back by it (empty: opt_.rho for every lane)
   int structure_ = FCCQP_STRUCTURE_AUTO;
   std::vector<int32_t> devices_;
   FCCQPBatchSolution sol_;

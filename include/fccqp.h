@@ -281,6 +281,27 @@ int fccqp_batch_solve(const fccqp_batch_desc* desc);
  * wall time of the whole call.
  * (Device-resident data lives on ONE device: shard it yourself and call fccqp_batch_solve per device.) */
 int fccqp_batch_solve_multi(const fccqp_batch_desc* desc, const int32_t* devices, int32_t n_devices);
+
+/* Per-lane rho (next to warm_lanes; the descriptor and FCCQP_ABI_VERSION are unchanged): fccqp_batch_solve and
+ * fccqp_batch_solve_multi are these calls with rho = NULL, which is today's behaviour bit for bit.  Otherwise rho is a
+ * dense [B] FP64 array in the call's memory_space that the call both reads and writes:
+ *   - lane i is solved exactly as a reference object on which set_rho(rho[i]) was called before Solve, cold or warm,
+ *     with or without warm_lanes (both index the same lanes); options.rho is not used;
+ *   - on return rho[i] holds the rho lane i ended with.  With options.adapt_rho_interval = 0 that is rho[i] unchanged.
+ *     With adaptive rho the returned mu_x / mu_lambda_c are scaled for that rho (y = rho mu), so feeding x, mu_x,
+ *     mu_lambda_c AND rho back into the next warm call continues every lane's ADMM from a consistent state.  (Without
+ *     the array each warm call restarts at options.rho and reads the duals as if they were scaled for it: y is off by
+ *     the factor rho_end / options.rho, and rho has to adapt again from scratch.)
+ *   - FCCQP_MEM_DEVICE: read and written in place by the kernels (no synchronisation), so CUDA-graph replays carry rho
+ *     from step to step.  An entry that is not finite or not > 0 ends its lane with FCCQP_STATUS_NUMERICAL_ISSUE and
+ *     n_iter = 0; the entry is left as it was, the lane's other outputs are unspecified, no other lane is affected.
+ *   - FCCQP_MEM_HOST: staged with every chunk (in and out); an array with such an entry is refused with FCCQP_E_INVALID
+ *     before anything runs.
+ * Calls with the array run the kernel instances that keep rho per QP (those of adaptive rho), and a shared-structure
+ * batch (Q and A_eq with batch stride 0) runs on the per-QP kernels, as it does under adaptive rho: a cached
+ * factorization has one rho. */
+int fccqp_batch_solve_rho(const fccqp_batch_desc* desc, double* rho);
+int fccqp_batch_solve_multi_rho(const fccqp_batch_desc* desc, double* rho, const int32_t* devices, int32_t n_devices);
 /* Page-locked host memory for FCCQP_MEM_HOST callers: inputs and outputs that live in
  * memory from here (or from cudaHostAlloc / torch pin_memory) move by asynchronous DMA that
  * overlaps the solve; pageable outputs go through an internal pinned bounce buffer. */
