@@ -31,7 +31,7 @@ std::atomic<long long> g_launches{0};
 struct LaunchInfo { int grid = 0, block = 0, smem = 0, ctas_per_sm = 0; };
 LaunchInfo g_last_launch;
 // what the last batch launch did about problem structure (fccqp_last_struct_info)
-struct StructInfo { int used = 0, nr = 0, ndp = 0, nd0 = 0, rows = 0, rows_dense = 0, device = 0, deferred_words = 1; };
+struct StructInfo { int used = 0, nr = 0, ndp = 0, nd0 = 0, rows = 0, rows_dense = 0, device = 0; };
 StructInfo g_last_struct;
 std::mutex g_info_mu;
 
@@ -80,8 +80,8 @@ struct DeviceCtx {
   char* hstage = nullptr;
   size_t hstage_bytes = 0;
   cudaEvent_t chunk_ev[16] = {};
-  unsigned int* h_deferred = nullptr;   // pinned [2]: QPs the structure-exploiting kernel handed to the general one (last
-                                        // launch; [1]: its warm QPs when it had a per-lane mask)
+  unsigned int* h_deferred = nullptr;   // pinned [2]: QPs the structure-exploiting kernel handed to the general one in
+                                        // the last structure call, per lane set
   int* h_probe = nullptr;               // pinned [4]: result of the structure probe
   std::mutex mu;       // guards counters / gscratch / occupancy cache
   std::mutex host_mu;  // serialises FCCQP_MEM_HOST calls (they share the staging buffer)
@@ -247,33 +247,40 @@ int geometry(DeviceCtx& ctx, KernelFn fn, int threads, size_t smem, int B, int q
   return FCCQP_OK;
 }
 
+// One uniform set of QPs, run by a path launcher with exactly the launches a uniform call of its kind runs: the whole
+// batch, or the cold or the warm QPs of a call with a per-lane mask.  Its counters and lists are its own.
+struct LaneSet {
+  int warm = 0;
+  const int* order = nullptr;            // processing order: nullptr (0..B-1), the LPT order, or a kNoQP-padded list
+  const unsigned int* count = nullptr;   // device-side length of a list; nullptr: the order ends at B or at its padding
+  unsigned int* work = nullptr;          // [3] work counters: first or single launch, general kernel, resume launch
+  unsigned int* handover_count = nullptr;  // QPs handed to a later launch: structure -> general kernel, shared-structure
+  int* handover = nullptr;                 //   pre-solve -> ADMM launch
+  unsigned int* resume_count = nullptr;    // QPs the first stage of a two-stage structure solve leaves to the resume
+  int* resume = nullptr;                   //   launch
+};
+
 // Stream-ordered scratch of one launch_solve call: one allocation and one memset of its header, so that any number of
 // calls may be in flight on any number of streams.  Offsets in 32-bit words.
 struct Scratch {
-  static constexpr size_t kWork = 0;       // work counter of the first launch
-  static constexpr size_t kWork2 = 1;      // work counter of the second launch
-  static constexpr size_t kListCount = 2;  // length of the hand-over list
-  static constexpr size_t kWarmListCount = 3;  // per-lane mask: length of the warm QPs' hand-over list (next to kListCount)
-  static constexpr size_t kProbe = 4;      // [4, 8): structure probe (atomicMax)
-  static constexpr size_t kLpt = 8;        // [8, 10): counters of lpt_order_kernel
-  static constexpr size_t kWork3 = 10;     // work counter of the resume launch of a two-stage structure solve
-  static constexpr size_t kResumeCount = 11;  // length of its list
-  static constexpr size_t kColdCount = 12;    // per-lane mask: lengths of the cold and the warm list (warm_split_kernel)
-  static constexpr size_t kWarmCount = 13;
-  static constexpr size_t kWork4 = 14;     // per-lane mask: work counters of the launches over the warm QPs
-  static constexpr size_t kWork5 = 15;
-  static constexpr size_t kHeader = 16;    // then [B] the hand-over list, [B] the resume list, [B] the LPT order; with a
-                                           // per-lane mask also [B] the cold list, [B] the warm list, [B] the warm hand-over
+  static constexpr size_t kProbe = 0;          // [0, 4): structure probe (atomicMax)
+  static constexpr size_t kLpt = 4;            // [4, 6): counters of lpt_order_kernel
+  static constexpr size_t kListCount = 6;      // [6, 8): lengths of the cold and the warm list (warm_split_kernel)
+  static constexpr size_t kHandoverCount = 8;  // [8, 10): hand-over count of lane set 0 and of lane set 1, adjacent
+  static constexpr size_t kResumeCount = 10;   // [10, 12): resume count of each lane set
+  static constexpr size_t kWork = 12;          // [12, 18): three work counters of each lane set
+  static constexpr size_t kHeader = 18;        // then [B] arrays: the hand-over and the resume list of set 0, the LPT
+                                               // order; with a per-lane mask also the cold list, the warm list and the
+                                               // hand-over and the resume list of set 1
   unsigned int* w = nullptr;
   size_t B = 0;
-  bool mask = false;                       // a per-lane mask: the call runs as a cold call over the cold list and a warm one
-                                           // over the warm list
-  int* list() const { return reinterpret_cast<int*>(w + kHeader); }
-  int* resume_list() const { return reinterpret_cast<int*>(w + kHeader + B); }
-  int* order() const { return reinterpret_cast<int*>(w + kHeader + 2 * B); }
-  int* cold_list() const { return reinterpret_cast<int*>(w + kHeader + 3 * B); }
-  int* warm_list() const { return reinterpret_cast<int*>(w + kHeader + 4 * B); }
-  int* warm_handover() const { return reinterpret_cast<int*>(w + kHeader + 5 * B); }
+  int sets = 1;                                // 2 with a per-lane mask: set[0] its cold QPs, set[1] its warm ones
+  LaneSet set[2];
+  int* array(int i) const { return reinterpret_cast<int*>(w + kHeader + i * B); }
+  LaneSet lanes(int k, int warm, const int* order, const unsigned int* count) const {
+    return {warm, order, count, w + kWork + 3 * k, w + kHandoverCount + k, array(k ? 5 : 0), w + kResumeCount + k,
+            array(k ? 6 : 1)};
+  }
 };
 
 // Per-lane warm start (fccqp_batch_desc::warm_lanes): the processing order (`order`, or 0..B-1) split into the cold and the
@@ -311,49 +318,57 @@ __global__ void __launch_bounds__(256) rho_invalid_kernel(const double* __restri
   if (status) status[i] = FCCQP_STATUS_NUMERICAL_ISSUE;
 }
 
-// Allocates the scratch of a call.  FCCQP_SCHEDULE_LPT, when the batch holds at least two QPs for each of the `slots`
-// that run at once: QPs whose previous solve ran long go to the front of the processing order (p.index_list).
-// warm_lanes (device memory): the processing order is split into the cold and the warm list (Scratch::cold_list / warm_list).
-int begin_call(fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long long slots, Scratch* s,
-               const uint8_t* warm_lanes) {
+// Allocates the scratch of a call and sets out its lane sets.  FCCQP_SCHEDULE_LPT, when the batch holds at least two QPs
+// for each of the `slots` that run at once: QPs whose previous solve ran long go to the front of the processing order.
+// warm_lanes (device memory): the processing order is split into a cold and a warm list, one lane set each.
+int begin_call(const fccqp::SolveParams& p, cudaStream_t stream, bool lpt_hint, long long slots, const uint8_t* warm_lanes,
+               Scratch* s) {
   const bool lpt = lpt_hint && p.n_iter != nullptr && p.B >= 2 * slots;
   s->B = (size_t)p.B;
-  s->mask = warm_lanes != nullptr;
-  const size_t arrays = s->mask ? 6 : (lpt ? 3 : 2);
+  const size_t arrays = warm_lanes ? 7 : (lpt ? 3 : 2);
   CUDA_TRY(cudaMallocAsync(&s->w, (Scratch::kHeader + arrays * s->B) * sizeof(unsigned int), stream));
   CUDA_TRY(cudaMemsetAsync(s->w, 0, Scratch::kHeader * sizeof(unsigned int), stream));
-  p.work_counter = s->w + Scratch::kWork;
+  int* order = nullptr;
   if (lpt) {
-    fccqp::lpt_order_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.n_iter, p.B, p.full_inverse_at, s->order(),
+    order = s->array(2);
+    fccqp::lpt_order_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.n_iter, p.B, p.full_inverse_at, order,
                                                                    s->w + Scratch::kLpt, s->w + Scratch::kLpt + 1);
     CUDA_TRY(cudaGetLastError());
-    p.index_list = s->order();
   }
-  if (s->mask) {
-    CUDA_TRY(cudaMemsetAsync(s->cold_list(), kNoQPByte, 2 * s->B * sizeof(int), stream));
-    warm_split_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(warm_lanes, p.index_list, p.B, s->cold_list(), s->warm_list(),
-                                                             s->w + Scratch::kColdCount);
-    CUDA_TRY(cudaGetLastError());
+  if (!warm_lanes) {
+    s->set[0] = s->lanes(0, p.warm, order, nullptr);
+    return FCCQP_OK;
   }
+  int *cold = s->array(3), *warm = s->array(4);
+  CUDA_TRY(cudaMemsetAsync(cold, kNoQPByte, 2 * s->B * sizeof(int), stream));
+  warm_split_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(warm_lanes, order, p.B, cold, warm, s->w + Scratch::kListCount);
+  CUDA_TRY(cudaGetLastError());
+  s->sets = 2;
+  s->set[0] = s->lanes(0, 0, cold, s->w + Scratch::kListCount);
+  s->set[1] = s->lanes(1, 1, warm, s->w + Scratch::kListCount + 1);
   return FCCQP_OK;
 }
 
-// The cold or the warm QPs of a call with a per-lane mask as a uniform call of their own: the list of begin_call as the
-// processing order, counted (count_dev) for the kernels that need the count, and a work counter of their own.
-fccqp::SolveParams mask_lanes(const fccqp::SolveParams& p, const Scratch& s, bool warm, bool counted) {
-  fccqp::SolveParams q = p;
-  q.warm = warm;
-  q.index_list = warm ? s.warm_list() : s.cold_list();
-  q.count_dev = counted ? s.w + (warm ? Scratch::kWarmCount : Scratch::kColdCount) : nullptr;
-  q.work_counter = s.w + (warm ? Scratch::kWork4 : Scratch::kWork);
-  return q;
+// p over a lane set: its warm flag, processing order and count, and its first work counter.
+fccqp::SolveParams over(fccqp::SolveParams p, const LaneSet& l) {
+  p.warm = l.warm;
+  p.index_list = l.order;
+  p.count_dev = l.count;
+  p.work_counter = l.work;
+  return p;
 }
 
-// Frees the scratch (stream-ordered) and records the call for fccqp_kernel_launch_count, fccqp_last_launch_info and
-// fccqp_last_struct_info.
-int end_call(const Scratch& s, cudaStream_t stream, int launches, const LaunchInfo& li, const StructInfo& si) {
+// Every solve launch: launched, checked and counted (fccqp_kernel_launch_count).
+int launch(KernelFn fn, const LaunchInfo& li, const fccqp::SolveParams& p, cudaStream_t stream) {
+  fn<<<li.grid, li.block, li.smem, stream>>>(p);
+  CUDA_TRY(cudaGetLastError());
+  g_launches.fetch_add(1);
+  return FCCQP_OK;
+}
+
+// Frees the scratch (stream-ordered) and records the call for fccqp_last_launch_info and fccqp_last_struct_info.
+int end_call(const Scratch& s, cudaStream_t stream, const LaunchInfo& li, const StructInfo& si) {
   CUDA_TRY(cudaFreeAsync(s.w, stream));
-  g_launches.fetch_add(launches);
   std::lock_guard<std::mutex> lk(g_info_mu);
   g_last_launch = li;
   g_last_struct = si;
@@ -406,89 +421,44 @@ const char* const kGeneralPhases[16] = {"stage-in", "assemble", "sigma/rhs0", "l
                                         "B-work-w0w2", "B-work-w1w3", "B-barrier-w0", nullptr, nullptr};
 #endif
 
-// Small problems (n + m <= 32): one QP per warp (fccqp_warp.cuh), four warps per CTA, each pulling QPs from the work
-// counter on its own; shared memory per CTA = 4 private (n + m) x ((n + m) | 1) slabs.
-// f32: the FP32 arithmetic instance (FCCQP_PRECISION_FP32: float32 problem data, float slabs).
-int launch_warp(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, bool f32, bool lpt_hint, const uint8_t* warm_lanes) {
-  constexpr int kW = 4;
-  const int N = p.n + p.m;
-  const size_t smem = (size_t)kW * N * (N | 1) * (f32 ? sizeof(float) : sizeof(double));
-  using fccqp::fccqp_warp_kernel;
-  KernelFn fn = p.rho_lanes ? (f32 ? (KernelFn)fccqp_warp_kernel<kW, 6, float, true> : (KernelFn)fccqp_warp_kernel<kW, 6, double, true>)
-                            : (f32 ? (KernelFn)fccqp_warp_kernel<kW, 6, float> : (KernelFn)fccqp_warp_kernel<kW, 6, double>);
-  // (measured, tools/bench_small.py: 6 CTAs x 4 warps at 80 registers beats 8 x 4 at 64 and 4 x 4 at 128 on every shape but n = 6;
-  //  float instance, tools/fp32_occ.py: 6 / 8 / 10 / 12 CTAs -> 82.7 / 78.5 / 71.4 / 70.5 M QP/s at n = 6, 22.4 / 23.1 / 21.1 / 21.7 at n = 24)
-  LaunchInfo li;
-  Scratch s;
-  int rc = geometry(ctx, fn, 32 * kW, smem, p.B, kW, &li);
-  if (!rc) rc = begin_call(p, stream, lpt_hint, (long long)kW * li.ctas_per_sm * ctx.num_sms, &s, warm_lanes);
-  if (rc) return rc;
-  if (s.mask) {   // the cold QPs, then the warm ones (each list ends at its kNoQP padding)
-    fn<<<li.grid, li.block, smem, stream>>>(mask_lanes(p, s, false, false));
-    CUDA_TRY(cudaGetLastError());
-    fn<<<li.grid, li.block, smem, stream>>>(mask_lanes(p, s, true, false));
-    CUDA_TRY(cudaGetLastError());
-    return end_call(s, stream, 2, li, dense_info(ctx, N));
-  }
-  fn<<<li.grid, li.block, smem, stream>>>(p);
-  CUDA_TRY(cudaGetLastError());
-  return end_call(s, stream, 1, li, dense_info(ctx, N));
-}
-
 // Shared-structure batch (one Q and one A_eq for the whole batch): every CTA caches its KKT factorization
 // (SolveParams::shared_mode).  Cold: a pre-solve launch hands the QPs that need ADMM iterations to an ADMM launch.
 // Warm (an MPC loop re-solving around one linearisation with carried duals): no pre-solve, the ADMM launch alone.
-// Per-lane mask: the cold sequence over the cold QPs, then the warm ADMM launch over the warm ones.
-int launch_shared(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s) {
-  const int threads = p.lay.N8 <= 128 ? 128 : 256;
-  KernelFn fn = pick_kernel(threads, true, false, false);
-  LaunchInfo li;
-  int rc = geometry(ctx, fn, threads, p.lay.bytes(), p.B, 1, &li);
-  if (rc) return rc;
-  p.shared_mode = 2;
-  if (s.mask) {
-    fccqp::SolveParams a = mask_lanes(p, s, false, true);
-    a.shared_mode = 1;
-    a.pending_count = s.w + Scratch::kListCount;
-    a.pending_list = s.list();
-    fn<<<li.grid, li.block, li.smem, stream>>>(a);
-    CUDA_TRY(cudaGetLastError());
-    fccqp::SolveParams c = p;
-    c.warm = 0;
-    c.count_dev = a.pending_count;
-    c.index_list = s.list();
-    c.work_counter = s.w + Scratch::kWork2;
-    fn<<<li.grid, li.block, li.smem, stream>>>(c);
-    CUDA_TRY(cudaGetLastError());
-    fn<<<li.grid, li.block, li.smem, stream>>>(mask_lanes(p, s, true, true));
-    CUDA_TRY(cudaGetLastError());
-    return end_call(s, stream, 3, li, dense_info(ctx, p.lay.N8));
+int launch_shared(KernelFn fn, const LaunchInfo& li, const fccqp::SolveParams& p, const LaneSet& l, cudaStream_t stream) {
+  fccqp::SolveParams a = over(p, l);
+  if (!l.warm) {
+    fccqp::SolveParams pre = a;
+    pre.shared_mode = 1;
+    pre.pending_count = l.handover_count;
+    pre.pending_list = l.handover;
+    if (int rc = launch(fn, li, pre, stream)) return rc;
+    a.count_dev = l.handover_count;
+    a.index_list = l.handover;
+    a.work_counter = l.work + 1;
   }
-  if (!p.warm) {
-    fccqp::SolveParams a = p;
-    a.shared_mode = 1;
-    a.pending_count = s.w + Scratch::kListCount;
-    a.pending_list = s.list();
-    fn<<<li.grid, li.block, li.smem, stream>>>(a);
-    CUDA_TRY(cudaGetLastError());
-    p.count_dev = a.pending_count;
-    p.index_list = s.list();
-    p.work_counter = s.w + Scratch::kWork2;
-  }
-  fn<<<li.grid, li.block, li.smem, stream>>>(p);
-  CUDA_TRY(cudaGetLastError());
-  return end_call(s, stream, p.warm ? 1 : 2, li, dense_info(ctx, p.lay.N8));
+  a.shared_mode = 2;
+  return launch(fn, li, a, stream);
 }
 
 constexpr int kNotApplicable = 1;
 
 // Structure-exploiting kernel (fccqp_struct.cuh): QPs whose separable variables can be eliminated analytically run on
-// a reduced KKT system; the others (if any) are appended to a device-side list that the general kernel (geometry gli)
-// takes in a last launch.  Large cold batches run the structure-exploiting solve in two stages (kStructFirst, then
-// the full kernel over the QPs the first stage listed).  Returns kNotApplicable, with nothing launched but the probe, when the
-// reduction does not pay.
-int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stream, const Scratch& s, const StructHint& hint,
-                  KernelFn general, const LaunchInfo& gli) {
+// a reduced KKT system; the others (if any) are appended to a device-side list that the general kernel takes in a last
+// launch.  plan_struct decides once per call what launch_struct runs for each lane set.
+struct StructPlan {
+  StructInfo info;
+  fccqp::StructLayout sl;
+  KernelFn first = nullptr, full = nullptr;   // the first stage; the single or the resume launch
+  LaunchInfo fli, li;                          // their geometry
+  bool two_stage = false;                      // a cold lane set runs in two stages
+  double* op_scratch = nullptr;                // per-CTA global scratch of the full-space operator of long-running QPs
+  long long op_stride = 0;                     //   (build_full_op), doubles per CTA
+};
+
+// The caps (probed on the device, or given), the reduced layout, the instances and their geometry, and op_scratch.
+// Returns kNotApplicable, with nothing launched but the probe, when the reduction does not pay.
+int plan_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stream, const Scratch& s, const StructHint& hint,
+                StructPlan* sp) {
   int caps[3] = {hint.caps[0], hint.caps[1], hint.caps[2]};
   if (hint.mode != FCCQP_STRUCTURE_CAPS) {
     // probe: classify up to 128 QPs spread over the batch, take the largest structure seen
@@ -516,126 +486,94 @@ int launch_struct(DeviceCtx& ctx, const fccqp::SolveParams& p, cudaStream_t stre
   const int need = p.n > sl.N8c ? p.n : sl.N8c;
   const bool adapt = p.adapt_k > 0 || p.rho_lanes, refine = p.struct_refine != 0;
   int threads;
-  KernelFn first;
-  if (need <= 64) { threads = 64; first = struct_first_instance<64, 8>(refine); }
-  else if (need <= 96) { threads = 96; first = struct_first_instance<96, 5>(refine); }
-  else if (need <= 128) { threads = 128; first = struct_first_instance<128, 4>(refine); }
-  else { threads = 256; first = struct_first_instance<256, 2>(refine); }
-  LaunchInfo li, fli;
-  int rc = geometry(ctx, first, threads, sl.bytes(), p.B, 1, &fli);
-  if (rc) return rc;
+  if (need <= 64) { threads = 64; sp->first = struct_first_instance<64, 8>(refine); sp->full = struct_instance<64, 8>(adapt); }
+  else if (need <= 96) { threads = 96; sp->first = struct_first_instance<96, 5>(refine); sp->full = struct_instance<96, 5>(adapt); }
+  else if (need <= 128) { threads = 128; sp->first = struct_first_instance<128, 4>(refine); sp->full = struct_instance<128, 4>(adapt); }
+  else { threads = 256; sp->first = struct_first_instance<256, 2>(refine); sp->full = struct_instance<256, 2>(adapt); }
+  int rc;
+  if ((rc = geometry(ctx, sp->first, threads, sl.bytes(), p.B, 1, &sp->fli)) ||
+      (rc = geometry(ctx, sp->full, threads, sl.bytes(), p.B, 1, &sp->li)))
+    return rc;
   // Cold batches of at least 8 QPs per resident CTA run in two stages: the first-stage kernel takes every QP through the
   // exit test of iteration 0 (where nearly all whole-body-control QPs stop) and lists the others, which the full kernel
-  // resumes from there.  Smaller batches and warm solves keep the single launch.  A per-lane mask: the cold QPs as a cold
-  // call of the whole batch (split by the same rule), the warm ones as the single launch of a warm call.
-  const bool split = (!p.warm || s.mask) && p.B >= 8LL * fli.ctas_per_sm * ctx.num_sms;
-  KernelFn fn;
-  if (threads == 64) fn = struct_instance<64, 8>(adapt);
-  else if (threads == 96) fn = struct_instance<96, 5>(adapt);
-  else if (threads == 128) fn = struct_instance<128, 4>(adapt);
-  else fn = struct_instance<256, 2>(adapt);
-  if ((rc = geometry(ctx, fn, threads, sl.bytes(), p.B, 1, &li))) return rc;
-  fccqp::SolveParams a = s.mask ? mask_lanes(p, s, false, false) : p;
-  a.slay = sl;
-  a.pending_count = s.w + Scratch::kListCount;
-  a.pending_list = s.list();
+  // resumes from there.  Smaller batches and warm solves keep the single launch.  The rule looks at the whole batch,
+  // also when a per-lane mask leaves only some of its QPs cold.
+  sp->two_stage = p.B >= 8LL * sp->fli.ctas_per_sm * ctx.num_sms;
+  sp->sl = sl;
+  // B, Z, X, Y tiles and 1/h sized for every variable eliminated
+  const long long neT = sl.n8 >> 3, NBr = sl.nr8c >> 3, mt = sl.mt;
+  sp->op_stride = (2 * mt * neT + neT * NBr + neT * (neT + 1) / 2) * 64 + 8 * neT;
+  CUDA_TRY(cudaMallocAsync(&sp->op_scratch, (size_t)sp->li.grid * sp->op_stride * sizeof(double), stream));
+  StructInfo& si = sp->info;
+  si.used = 1; si.nr = caps[0]; si.ndp = caps[1]; si.nd0 = caps[2]; si.rows = sl.N8c; si.rows_dense = p.lay.N8; si.device = ctx.device;
+  return FCCQP_OK;
+}
+
+// One lane set on the structure path: the single launch, or a cold set in two stages; then the general kernel (geometry
+// gli) over the QPs handed over.
+int launch_struct(const StructPlan& sp, KernelFn general, const LaunchInfo& gli, const fccqp::SolveParams& p, const LaneSet& l,
+                  cudaStream_t stream) {
+  const bool split = !l.warm && sp.two_stage;
+  fccqp::SolveParams a = over(p, l);
+  a.count_dev = nullptr;   // to the structure kernel a count marks the resume launch; a list's padding ends this one
+  a.slay = sp.sl;
+  a.pending_count = l.handover_count;
+  a.pending_list = l.handover;
+  int rc;
   if (split) {
     fccqp::SolveParams f = a;
-    f.resume_list = s.resume_list();
-    f.resume_count = s.w + Scratch::kResumeCount;
+    f.resume_list = l.resume;
+    f.resume_count = l.resume_count;
 #ifdef FCCQP_DEV
     PhaseProfile prof;
     if ((rc = prof.start(stream, &f))) return rc;
 #endif
-    first<<<fli.grid, fli.block, fli.smem, stream>>>(f);
-    CUDA_TRY(cudaGetLastError());
+    if ((rc = launch(sp.first, sp.fli, f, stream))) return rc;
 #ifdef FCCQP_DEV
-    if ((rc = prof.report(stream, "struct first stage", kStructPhases, p.B, fli.grid))) return rc;
+    if ((rc = prof.report(stream, "struct first stage", kStructPhases, p.B, sp.fli.grid))) return rc;
 #endif
-    a.count_dev = f.resume_count;
-    a.index_list = f.resume_list;
-    a.work_counter = s.w + Scratch::kWork3;
+    a.count_dev = l.resume_count;
+    a.index_list = l.resume;
+    a.work_counter = l.work + 2;
   }
-  // per-CTA global scratch of the full-space operator of long-running QPs (build_full_op): B, Z, X, Y tiles and 1/h
-  // sized for every variable eliminated
-  const long long neT = sl.n8 >> 3, NBr = sl.nr8c >> 3, mt = sl.mt;
-  a.op_stride = (2 * mt * neT + neT * NBr + neT * (neT + 1) / 2) * 64 + 8 * neT;
-  CUDA_TRY(cudaMallocAsync(&a.op_scratch, (size_t)li.grid * a.op_stride * sizeof(double), stream));
+  a.op_scratch = sp.op_scratch;
+  a.op_stride = sp.op_stride;
 #ifdef FCCQP_DEV
   PhaseProfile prof;
   if ((rc = prof.start(stream, &a))) return rc;
 #endif
-  fn<<<li.grid, li.block, li.smem, stream>>>(a);
-  CUDA_TRY(cudaGetLastError());
-  if (s.mask) {
-    fccqp::SolveParams w = mask_lanes(p, s, true, false);
-    w.slay = sl;
-    w.pending_count = s.w + Scratch::kWarmListCount;
-    w.pending_list = s.warm_handover();
-    w.op_stride = a.op_stride;
-    w.op_scratch = a.op_scratch;
-    fn<<<li.grid, li.block, li.smem, stream>>>(w);
-    CUDA_TRY(cudaGetLastError());
-  }
-  CUDA_TRY(cudaFreeAsync(a.op_scratch, stream));
+  if ((rc = launch(sp.full, sp.li, a, stream))) return rc;
 #ifdef FCCQP_DEV
-  if ((rc = prof.report(stream, split ? "struct resume" : "struct", kStructPhases, p.B, li.grid))) return rc;
+  if ((rc = prof.report(stream, split ? "struct resume" : "struct", kStructPhases, p.B, sp.li.grid))) return rc;
 #endif
   if (split && p.rho_lanes) {
     rho_invalid_kernel<<<(p.B + 255) / 256, 256, 0, stream>>>(p.rho_lanes, p.B, p.n_iter, p.status);
     CUDA_TRY(cudaGetLastError());
+    g_launches.fetch_add(1);
   }
-  fccqp::SolveParams b = p;
-  if (s.mask) b.warm = 0;
-  b.count_dev = a.pending_count;
-  b.index_list = s.list();
-  b.work_counter = s.w + Scratch::kWork2;
-  general<<<gli.grid, gli.block, gli.smem, stream>>>(b);
-  CUDA_TRY(cudaGetLastError());
-  int launches = (split ? 3 : 2) + (split && p.rho_lanes ? 1 : 0);
-  if (s.mask) {   // the warm QPs the full kernel handed over
-    fccqp::SolveParams bw = p;
-    bw.warm = 1;
-    bw.count_dev = s.w + Scratch::kWarmListCount;
-    bw.index_list = s.warm_handover();
-    bw.work_counter = s.w + Scratch::kWork5;
-    general<<<gli.grid, gli.block, gli.smem, stream>>>(bw);
-    CUDA_TRY(cudaGetLastError());
-    launches += 2;
-  }
-  // (the warm hand-over count sits right after the cold one)
-  const int words = s.mask ? 2 : 1;
-  CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, a.pending_count, words * sizeof(unsigned int), cudaMemcpyDeviceToHost, stream));
-  StructInfo si;
-  si.used = 1; si.nr = caps[0]; si.ndp = caps[1]; si.nd0 = caps[2]; si.rows = sl.N8c; si.rows_dense = p.lay.N8; si.device = ctx.device;
-  si.deferred_words = words;
-  return end_call(s, stream, launches, split ? fli : li, si);
+  fccqp::SolveParams b = over(p, l);
+  b.count_dev = l.handover_count;
+  b.index_list = l.handover;
+  b.work_counter = l.work + 1;
+  return launch(general, gli, b, stream);
 }
 
-int launch_general(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, const Scratch& s, KernelFn fn, const LaunchInfo& li) {
+int launch_general(KernelFn fn, const LaunchInfo& li, fccqp::SolveParams p, cudaStream_t stream) {
 #ifdef FCCQP_DEV
   PhaseProfile prof;
   int rc = prof.start(stream, &p);
-  if (rc) return rc;
+  if (!rc) rc = launch(fn, li, p, stream);
+  return rc ? rc : prof.report(stream, "general", kGeneralPhases, p.B, li.grid);
+#else
+  return launch(fn, li, p, stream);
 #endif
-  if (s.mask) {   // the cold QPs, then the warm ones
-    fn<<<li.grid, li.block, li.smem, stream>>>(mask_lanes(p, s, false, true));
-    CUDA_TRY(cudaGetLastError());
-    fn<<<li.grid, li.block, li.smem, stream>>>(mask_lanes(p, s, true, true));
-  } else {
-    fn<<<li.grid, li.block, li.smem, stream>>>(p);
-  }
-  CUDA_TRY(cudaGetLastError());
-#ifdef FCCQP_DEV
-  if ((rc = prof.report(stream, "general", kGeneralPhases, p.B, li.grid))) return rc;
-#endif
-  return end_call(s, stream, s.mask ? 2 : 1, li, dense_info(ctx, p.lay.N8));
 }
 
 // Launches the solve on `stream` for device-resident data described by p (scratch allocated here, stream-ordered).
 // precision: fccqp_precision of the call (FP32_DATA and FP32: float32 problem data behind the pointers of p; FP32: FP32
 // arithmetic too where a kernel for it exists -- the warp kernel -- and FP32_DATA's FP64 arithmetic otherwise)
-// warm_lanes: optional per-lane mask in device memory (fccqp_batch_desc::warm_lanes); p.warm is then ignored.
+// warm_lanes: optional per-lane mask in device memory (fccqp_batch_desc::warm_lanes); p.warm is then ignored, and the
+// path runs twice: as a uniform cold call over the cold QPs, then as a uniform warm call over the warm ones.
 // p.rho_lanes: optional per-lane rho in device memory (fccqp_batch_solve_rho); such calls run the instances that keep rho
 // per QP (kAdapt, and kRhoLanes of the warp kernel), never the shared-structure path (its cached factorization has one rho).
 int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int precision, const StructHint& hint,
@@ -649,27 +587,69 @@ int launch_solve(DeviceCtx& ctx, fccqp::SolveParams p, cudaStream_t stream, int 
   p.lay = fccqp::Layout(p.n, p.m, p.nc);
   p.full_inverse_at = sw.full_inverse_at ? sw.full_inverse_at : (small ? 8 : 6);
   p.struct_refine = hint.refine;
-  if (small && (precision == FCCQP_PRECISION_FP32 || (!f32 && !sw.no_warp)))
-    return launch_warp(ctx, p, stream, precision == FCCQP_PRECISION_FP32, hint.lpt, warm_lanes);
-
-  // one CTA per QP; float32 problem data take the general kernel's widening instance, same geometry
-  const int threads = p.lay.N8 <= 128 ? 128 : 256;
-  KernelFn general = pick_kernel(threads, false, f32, p.adapt_k > 0 || p.rho_lanes);
-  LaunchInfo li;
+  enum { kWarp, kShared, kStruct, kGeneral } path;
+  KernelFn fn, general = nullptr;
+  LaunchInfo li, gli;   // geometry of fn, and of the general kernel
+  long long slots;      // QPs that run at once
+  int rows = p.lay.N8;
+  if (small && (precision == FCCQP_PRECISION_FP32 || (!f32 && !sw.no_warp))) {
+    // Small problems (n + m <= 32): one QP per warp (fccqp_warp.cuh), four warps per CTA, each pulling QPs from the work
+    // counter on its own; shared memory per CTA = 4 private (n + m) x ((n + m) | 1) slabs.  FCCQP_PRECISION_FP32: the FP32
+    // arithmetic instance (float32 problem data, float slabs).
+    constexpr int kW = 4;
+    const bool f32a = precision == FCCQP_PRECISION_FP32;
+    rows = p.n + p.m;
+    const size_t smem = (size_t)kW * rows * (rows | 1) * (f32a ? sizeof(float) : sizeof(double));
+    using fccqp::fccqp_warp_kernel;
+    fn = p.rho_lanes ? (f32a ? (KernelFn)fccqp_warp_kernel<kW, 6, float, true> : (KernelFn)fccqp_warp_kernel<kW, 6, double, true>)
+                     : (f32a ? (KernelFn)fccqp_warp_kernel<kW, 6, float> : (KernelFn)fccqp_warp_kernel<kW, 6, double>);
+    // (measured, tools/bench_small.py: 6 CTAs x 4 warps at 80 registers beats 8 x 4 at 64 and 4 x 4 at 128 on every shape but n = 6;
+    //  float instance, tools/fp32_occ.py: 6 / 8 / 10 / 12 CTAs -> 82.7 / 78.5 / 71.4 / 70.5 M QP/s at n = 6, 22.4 / 23.1 / 21.1 / 21.7 at n = 24)
+    path = kWarp;
+    rc = geometry(ctx, fn, 32 * kW, smem, p.B, kW, &li);
+    slots = (long long)kW * li.ctas_per_sm * ctx.num_sms;
+  } else {
+    // one CTA per QP; float32 problem data take the general kernel's widening instance, same geometry
+    const int threads = p.lay.N8 <= 128 ? 128 : 256;
+    general = pick_kernel(threads, false, f32, p.adapt_k > 0 || p.rho_lanes);
+    if ((rc = geometry(ctx, general, threads, p.lay.bytes(), p.B, 1, &gli))) return rc;
+    slots = (long long)gli.ctas_per_sm * ctx.num_sms;
+    // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs.  Not with
+    // adaptive or per-lane rho: a lane with its own rho needs its own rho-KKT factorization, so those batches take the
+    // structure-exploiting or general kernel (both read Q and A_eq through the batch stride).
+    if (!sw.no_shared && !f32 && p.adapt_k == 0 && !p.rho_lanes && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) &&
+        p.B >= 4 * gli.ctas_per_sm * ctx.num_sms) {
+      path = kShared;
+      fn = pick_kernel(threads, true, false, false);
+      rc = geometry(ctx, fn, threads, p.lay.bytes(), p.B, 1, &li);
+    } else {
+      path = !f32 && hint.mode != FCCQP_STRUCTURE_DENSE && p.m > 0 ? kStruct : kGeneral;
+      fn = general;
+      li = gli;
+    }
+  }
   Scratch s;
-  if ((rc = geometry(ctx, general, threads, p.lay.bytes(), p.B, 1, &li)) ||
-      (rc = begin_call(p, stream, hint.lpt, (long long)li.ctas_per_sm * ctx.num_sms, &s, warm_lanes)))
-    return rc;
-  // one Q and one A_eq for the whole batch: caching the factorization pays once every CTA sees several QPs.  Not with
-  // adaptive or per-lane rho: a lane with its own rho needs its own rho-KKT factorization, so those batches take the
-  // structure-exploiting or general kernel (both read Q and A_eq through the batch stride).
-  if (!sw.no_shared && !f32 && p.adapt_k == 0 && !p.rho_lanes && p.q_bs == 0 && (p.m == 0 || p.a_bs == 0) &&
-      p.B >= 4 * li.ctas_per_sm * ctx.num_sms)
-    return launch_shared(ctx, p, stream, s);
-  if (!f32 && hint.mode != FCCQP_STRUCTURE_DENSE && p.m > 0 &&
-      (rc = launch_struct(ctx, p, stream, s, hint, general, li)) != kNotApplicable)
-    return rc;
-  return launch_general(ctx, p, stream, s, general, li);
+  if (rc || (rc = begin_call(p, stream, hint.lpt, slots, warm_lanes, &s))) return rc;
+  StructPlan sp;
+  if (path == kStruct && (rc = plan_struct(ctx, p, stream, s, hint, &sp))) {
+    if (rc != kNotApplicable) return rc;
+    path = kGeneral;
+    rc = FCCQP_OK;
+  }
+  for (int k = 0; k < s.sets && !rc; ++k) {
+    const LaneSet& l = s.set[k];
+    if (path == kWarp) rc = launch(fn, li, over(p, l), stream);
+    else if (path == kShared) rc = launch_shared(fn, li, p, l, stream);
+    else if (path == kStruct) rc = launch_struct(sp, general, gli, p, l, stream);
+    else rc = launch_general(fn, li, over(p, l), stream);
+  }
+  if (rc) return rc;
+  if (path != kStruct) return end_call(s, stream, li, dense_info(ctx, rows));
+  CUDA_TRY(cudaFreeAsync(sp.op_scratch, stream));
+  CUDA_TRY(cudaMemcpyAsync(ctx.h_deferred, s.w + Scratch::kHandoverCount, 2 * sizeof(unsigned int), cudaMemcpyDeviceToHost,
+                           stream));
+  // the geometry of the cold sequence: its first stage when it ran in two stages
+  return end_call(s, stream, sp.two_stage && !s.set[0].warm ? sp.fli : sp.li, sp.info);
 }
 
 int check_dims(int n, int m, int nc, int lcs) {
@@ -792,7 +772,7 @@ int fccqp_last_struct_info(int* used, int* caps, int* rows, int* rows_dense, int
       std::lock_guard<std::mutex> lk(g_ctx_mu);
       auto it = g_ctx.find(si.device);
       if (it != g_ctx.end() && it->second->h_deferred)
-        for (int k = 0; k < si.deferred_words; ++k) *deferred += (int)it->second->h_deferred[k];
+        *deferred = (int)it->second->h_deferred[0] + (int)it->second->h_deferred[1];
     }
   }
   return FCCQP_OK;

@@ -9,7 +9,8 @@
    with set_rho(last_rho) before every step, under the bar of test_adaptive_rho.py; the returned rho is the restatement's.
 4. A warm_lanes mask with per-lane rho: every lane equals the uniform call of its kind at its rho.
 5. CUDA graph: replays carry rho from step to step, and an entry changed in place between replays takes effect.
-6. Entries that are not finite or not > 0 end their lane with NUMERICAL_ISSUE and n_iter 0 and stay as they were.
+6. Entries that are not finite or not > 0 end their lane with NUMERICAL_ISSUE and n_iter 0 and stay as they were, in
+   cold, warm and mixed calls.
 7. FCCQP_SCHEDULE_LPT with an array changes the processing order only.
 """
 import numpy as np
@@ -350,7 +351,9 @@ def test_invalid_entries(walking_log, log512, log16k, path):
     bad = np.array([0, 1, 2, B // 2, B - 1])
     r_bad = r.copy()
     r_bad[bad] = [0.0, -1.0, np.nan, np.inf, -0.0]
-    for warm in (False, True):
+    # a mask puts bad entries on cold and on warm lanes; its cold launches (on struct-split two-stage, rho_invalid_kernel
+    # included) run before its warm ones
+    for warm in (False, True, scattered_mask(B, 49)):
         got = solve_step(make, qp0, qp1, warm, rho=r_bad, **kw)
         want = solve_step(make, qp0, qp1, warm, rho=r, **kw)
         assert np.array_equal(got["status"][bad], np.full(bad.size, 2)) and not got["n_iter"][bad].any(), path
